@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- the driver's contract benchmark.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload cX]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload cX] [--dump-outputs DIR]
 
 Metric (BASELINE.json): GStencil/s and achieved HBM GB/s (% of roofline) per stencil.
 A "step" is one run of the reference's emitted host loop (codegen_2d.hpp:610-613) over one
@@ -28,6 +28,12 @@ synthetic grid: `for (t = 0; t < iterations; t += 2*step) { sweep(A,B); sweep(B,
 `cpu_baseline`  the CPU oracle (a port: the reference has no CPU loop) on ALL host cores (whatever
             OMP_NUM_THREADS says -- torchrun sets it to 1), on a bounded sample of the same workload.
 `--impl reference`  the same oracle port, timed as the reference arm (rank 0 only).
+`--dump-outputs DIR`  after the timed steps, the buffers the timed call hands back (A, where the result lands, and B)
+            as DIR/<name>.npy in their own dtype: whole up to 2^21 / N elements, else the same seeded sample of
+            2^21 / N flat positions on every run (N ranks: 32 MiB in all at most).  The inputs depend only on the
+            arguments, so two builds can be compared output for output.
+
+The tree is only read: kernels compiled at run time go to a temporary cache seeded with the cubins build() left.
 """
 import argparse
 import json
@@ -168,6 +174,40 @@ def time_steps(plan, A, B, timesteps, steps, warmup):
     return e0.elapsed_time(e1) * 1e-3, plan.launch_count - l0
 
 
+DUMP_POINTS = 1 << 21
+
+
+def dump_outputs(out_dir, arrays, points=DUMP_POINTS):
+    """{name: tensor} -> out_dir/<name>.npy: the whole array up to `points` elements, else the values at one fixed,
+    seeded set of `points` flat positions (sorted), the same on every run."""
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        n = t.numel()
+        if n <= points:
+            host = t.cpu().numpy()
+        else:
+            idx = np.unique(np.random.default_rng(20251020).integers(0, n, points))
+            host = t.reshape(-1)[torch.from_numpy(idx).to(t.device)].cpu().numpy()
+        np.save(os.path.join(out_dir, name + ".npy"), host)
+
+
+def private_jit_cache():
+    """Points the engine's kernel cache at a new temporary directory that links the cubins build() left in
+    drstencil_b200/_jitcache/, so that kernels compiled during the run are written there and not into the tree."""
+    import tempfile
+    import drstencil_b200 as drs
+    tmp = tempfile.mkdtemp(prefix="drs_bench_jitcache_")
+    src = os.path.join(ROOT, "drstencil_b200", "_jitcache")
+    if os.path.isdir(src):
+        for f in os.listdir(src):
+            if f.endswith(".cubin"):
+                os.symlink(os.path.join(src, f), os.path.join(tmp, f))
+    drs.lib().drs_set_cache_dir(tmp.encode())
+    return tmp
+
+
 # ---------------------------------------------------------------------------------------------
 # CPU legs (the only code in this file that touches oracle/)
 # ---------------------------------------------------------------------------------------------
@@ -243,7 +283,7 @@ def run_reference(args, rank):
     for _ in range(args.warmup):
         cs.run(3.0)
     vals, secs, sweeps = [], 0.0, 0
-    for _ in range(max(1, args.steps)):
+    for _ in range(args.steps):
         v, t, n = cs.run(3.0)
         vals.append(v)
         secs += t
@@ -465,6 +505,9 @@ def run_single(args, rank, world):
     sampler.start()
     secs, launches = time_steps(plan, A, B, timesteps, args.steps, args.warmup)
     clocks = sampler.stop()
+    if args.dump_outputs:
+        suffix = "_rank%d" % rank if world > 1 else ""
+        dump_outputs(args.dump_outputs, {"A" + suffix: A, "B" + suffix: B}, DUMP_POINTS // world)
     data_finite = bool(torch.isfinite(A).all()) and float(A.abs().max()) > 0
     info = plan.info
     if world > 1:
@@ -616,6 +659,9 @@ def run_slab(args, rank, world):
     e1.record()
     slab.plan.sync_check()
     clocks = sampler.stop()
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"A_rank%d" % rank: slab.owned(0), "B_rank%d" % rank: slab.owned(1)},
+                     DUMP_POINTS // world)
     secs = e0.elapsed_time(e1) * 1e-3
     t = torch.tensor([secs], device="cuda", dtype=torch.float64)
     dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -817,6 +863,7 @@ def per_config(args):
 
 
 def main():
+    sys.dont_write_bytecode = True       # the tree may be read-only; nothing is cached in it
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
     ap.add_argument("--steps", type=int, default=10)
@@ -829,7 +876,12 @@ def main():
     ap.add_argument("--halo", default="p2p", choices=["p2p", "p2p-flags", "nccl"], help="N > 1: halo exchange path")
     ap.add_argument("--depth", type=int, default=1, help="c5 only: in-kernel temporal depth (extra evidence; "
                     "the contract line is depth 1, bit-exact)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the buffers of the last timed step to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs: the reference arm sweeps for a fixed time, so its outputs differ from run to run")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -850,6 +902,9 @@ def main():
     if not torch.cuda.is_available():
         sys.exit("bench.py: no CUDA device -- the engine has no CPU path (use --impl reference for the CPU oracle)")
     torch.cuda.set_device(local)
+    import atexit
+    import shutil
+    atexit.register(shutil.rmtree, private_jit_cache(), True)
     if world > 1:
         import torch.distributed as dist
         dist.init_process_group("nccl", device_id=torch.device("cuda", local))

@@ -1,6 +1,7 @@
-"""The `drstencil` command line against the reference binary (oracle/_ref/drstencil_ref, built from
-/root/reference/main.cpp): same exit codes and messages for the same argv (CPU), and the emitted
+"""The `drstencil` command line against the original generator's answers (tests/golden/ref_cli.json, made by
+tests/golden/make_cli_golden.py): same exit codes and messages for the same argv (CPU), and the emitted
 program compiled with nvcc and run on the GPU (gpu)."""
+import json
 import os
 import re
 import shutil
@@ -11,7 +12,8 @@ import pytest
 from helpers import ROOT, SHIPPED
 
 CLI = os.path.join(ROOT, "drstencil_b200", "bin", "drstencil")
-REF = os.path.join(ROOT, "oracle", "_ref", "drstencil_ref")
+with open(os.path.join(ROOT, "tests", "golden", "ref_cli.json")) as _f:
+    GOLDEN = json.load(_f)
 
 ARGVS = [
     [],
@@ -47,28 +49,24 @@ def _run(binary, argv, cwd, timeout=60):
     return r.returncode, r.stdout
 
 
-@pytest.mark.skipif(not os.path.exists(REF), reason="oracle/_ref/drstencil_ref not built")
 def test_exit_codes_and_messages_match_the_reference_binary(built, tmp_path):
-    for d in ("ours", "ref"):
-        os.makedirs(tmp_path / d)
-        for name in SHIPPED:
-            shutil.copy(os.path.join(ROOT, "stc", name + ".stc"), tmp_path / d)
-    for argv in ARGVS:
-        rc_o, out_o = _run(CLI, argv, tmp_path / "ours")
-        rc_r, out_r = _run(REF, argv, tmp_path / "ref")
-        assert rc_o == rc_r, (argv, rc_o, rc_r, out_o, out_r)
+    assert [r["argv"] for r in GOLDEN["fixed"]] == ARGVS
+    for name in SHIPPED:
+        shutil.copy(os.path.join(ROOT, "stc", name + ".stc"), tmp_path)
+    for ref in GOLDEN["fixed"]:
+        argv = ref["argv"]
+        rc_o, out_o = _run(CLI, argv, tmp_path)
+        assert rc_o == ref["rc"], (argv, rc_o, ref, out_o)
         if argv and argv[0] in ("--help", "-h"):
-            for opt in re.findall(r"^(--?[a-z0-9-]+)", out_r, re.M):     # every reference option is documented
+            for opt in ref["options"]:                                    # every reference option is documented
                 assert opt in out_o, opt
             continue
-        assert out_o.strip().splitlines()[:1] == out_r.strip().splitlines()[:1], (argv, out_o, out_r)
+        assert out_o.strip().splitlines()[:1] == ([ref["first"]] if ref["first"] else []), (argv, out_o, ref)
         # both write (or do not write) an output file
-        made_o = {f for f in os.listdir(tmp_path / "ours") if f.endswith(".cu")}
-        made_r = {f for f in os.listdir(tmp_path / "ref") if f.endswith(".cu")}
-        assert made_o == made_r, (argv, made_o, made_r)
+        made_o = sorted(f for f in os.listdir(tmp_path) if f.endswith(".cu"))
+        assert made_o == [f for f in ref["made"] if f.endswith(".cu")], (argv, made_o, ref)
         for f in made_o:
-            os.remove(tmp_path / "ours" / f)
-            os.remove(tmp_path / "ref" / f)
+            os.remove(tmp_path / f)
 
 
 def test_emitted_program_is_self_contained_text(built, tmp_path):
@@ -173,34 +171,29 @@ def _random_argv(rng):
     return argv
 
 
-@pytest.mark.skipif(not os.path.exists(REF), reason="oracle/_ref/drstencil_ref not built")
 def test_random_command_lines_against_the_reference_binary(built, tmp_path):
     """Differential test: 250 seeded random command lines give the same exit code, the same first line
     of output and the same set of emitted files as the reference binary."""
     import random
-    for d in ("ours", "ref"):
-        os.makedirs(tmp_path / d)
-        for name in SHIPPED:
-            shutil.copy(os.path.join(ROOT, "stc", name + ".stc"), tmp_path / d)
+    for name in SHIPPED:
+        shutil.copy(os.path.join(ROOT, "stc", name + ".stc"), tmp_path)
     rng = random.Random(20240)
     first = lambda s: (s.strip().splitlines() or [""])[0]
     hung_or_crashed = []
-    for _ in range(250):
+    assert len(GOLDEN["random"]) == 250
+    for ref in GOLDEN["random"]:
         argv = _random_argv(rng)
-        rc_o, out_o = _run(CLI, argv, tmp_path / "ours", timeout=20)
-        rc_r, out_r = _run(REF, argv, tmp_path / "ref", timeout=5)
-        made_o = {f for f in os.listdir(tmp_path / "ours") if not f.endswith(".stc")}     # `-o --3d` names a file "--3d"
-        made_r = {f for f in os.listdir(tmp_path / "ref") if not f.endswith(".stc")}
+        assert argv == ref["argv"]
+        rc_o, out_o = _run(CLI, argv, tmp_path, timeout=20)
+        made_o = sorted(f for f in os.listdir(tmp_path) if not f.endswith(".stc"))     # `-o --3d` names a file "--3d"
         for f in made_o:
-            os.remove(tmp_path / "ours" / f)
-        for f in made_r:
-            os.remove(tmp_path / "ref" / f)
+            os.remove(tmp_path / f)
         assert rc_o != "timeout", argv
-        if rc_r == "timeout" or (isinstance(rc_r, int) and rc_r < 0):
+        if ref["rc"] is None or ref["rc"] < 0:
             hung_or_crashed.append(argv)         # the reference spins or dies on this input: nothing to compare
             continue
-        assert rc_o == rc_r, (argv, rc_o, rc_r, out_o, out_r)
-        assert made_o == made_r, (argv, made_o, made_r)
+        assert rc_o == ref["rc"], (argv, rc_o, ref, out_o)
+        assert made_o == ref["made"], (argv, made_o, ref)
         if not (argv and argv[0] in ("--help", "-h")):
-            assert first(out_o) == first(out_r), (argv, out_o, out_r)
+            assert first(out_o) == ref["first"], (argv, out_o, ref)
     assert len(hung_or_crashed) <= 10, hung_or_crashed

@@ -235,25 +235,27 @@ def test_unaligned_row_pitch_temporal_kernels(built, name, shape, kn, mode, monk
 ])
 def test_unaligned_row_pitch_is_no_performance_cliff(built, name, odd, even, kn, bar):
     """VERDICT r01 item 8: an odd N must stay close to the aligned size next to it (round 1: the naive kernel, ~10x
-    slower; the cp.async form: 1.3x - 1.6x; per-row TMA: 0.97x / 1.14x / 1.21x, profiles/r02_unaligned_pitch.md)."""
+    slower; the cp.async form: 1.3x - 1.6x; per-row TMA: 0.97x / 1.14x / 1.21x, profiles/r02_unaligned_pitch.md).
+    The bursts of the two sizes alternate, so that both are timed under the same clocks and the same neighbours."""
     import torch
-    per_point = []
+    runs = []
     for shape in (odd, even):
         plan = _plan(name, shape, **kn)
         A = torch.rand(shape, dtype=torch.float64, device="cuda")
         B = torch.zeros_like(A)
         _sweeps(plan, A, B, 4)
-        e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-        best = None
-        for _ in range(3):
+        runs.append((plan, A, B, float(np.prod(shape))))
+    e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    per_point = [None, None]
+    for _ in range(5):
+        for q, (plan, A, B, points) in enumerate(runs):
             e0.record()
             _sweeps(plan, A, B, 20)
             e1.record()
             torch.cuda.synchronize()
-            t = e0.elapsed_time(e1)
-            best = t if best is None else min(best, t)
-        per_point.append(best / float(np.prod(shape)))
-        del A, B
+            t = e0.elapsed_time(e1) / points
+            per_point[q] = t if per_point[q] is None else min(per_point[q], t)
+    del runs
     print("unaligned / aligned time per point: %.3f" % (per_point[0] / per_point[1]))
     assert per_point[0] <= bar * per_point[1], per_point
 

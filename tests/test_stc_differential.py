@@ -1,20 +1,25 @@
-"""Randomised differential test of the .stc front end against the reference generator
-(oracle/_ref/drstencil_ref, built from /root/reference/main.cpp): random descriptions (keys in any
+"""Randomised differential test of the .stc front end against the reference generator's answers
+(tests/golden/ref_cli.json, made by tests/golden/make_cli_golden.py): random descriptions (keys in any
 order, unknown tokens such as the shipped "iteratioins" typo, duplicate keys and points, radius 1-3,
 2D and 3D, assorted coefficient spellings) run through both command lines with random --step/--dist;
 exit code, first output line and the L/M/N/Iterations/Halo macros of the emitted programs must agree
-(/root/reference/drstencil_2d.hpp:48-97, drstencil.hpp:52-103)."""
+(drstencil_2d.hpp:48-97, drstencil.hpp:52-103 of the original)."""
+import json
 import os
 import random
 import re
 import subprocess
+import sys
 
 import pytest
 
 from helpers import ROOT
 
+sys.path.insert(0, os.path.join(ROOT, "tests", "golden"))
+
 CLI = os.path.join(ROOT, "drstencil_b200", "bin", "drstencil")
-REF = os.path.join(ROOT, "oracle", "_ref", "drstencil_ref")
+with open(os.path.join(ROOT, "tests", "golden", "ref_cli.json")) as _f:
+    GOLDEN = json.load(_f)
 
 
 def random_stc(rng, is3d):
@@ -54,72 +59,53 @@ def _defines(path):
     return {m.group(1): int(m.group(2)) for m in re.finditer(r"^#define\s+(\w+)\s+(-?\d+)", open(path).read(), re.M)}
 
 
-@pytest.mark.skipif(not os.path.exists(REF), reason="oracle/_ref/drstencil_ref not built")
 def test_random_descriptions_parse_and_analyse_like_the_reference(built, tmp_path):
+    from make_cli_golden import parse_argv
     compared = emitted = 0
-    for seed in range(160):
-        rng = random.Random(seed)
-        is3d = rng.random() < 0.4
-        text, has_iterations = random_stc(rng, is3d)
+    assert [r["seed"] for r in GOLDEN["parse"]] == list(range(160))
+    for ref in GOLDEN["parse"]:
+        seed = ref["seed"]
+        text, has_iterations, is3d, argv = parse_argv(random.Random(seed))
         (tmp_path / "t.stc").write_text(text)
-        step, dist = rng.choice([1, 1, 2, 3]), rng.choice([0, 0, 1, 2])
-        argv = (["--3d"] if is3d else []) + ["--step", str(step)] + (["--dist", str(dist)] if dist else []) + \
-            ["--bx", "64", "--by", "16"]
-        for f in ("o.cu", "r.cu"):
-            if os.path.exists(tmp_path / f):
-                os.remove(tmp_path / f)
+        if os.path.exists(tmp_path / "o.cu"):
+            os.remove(tmp_path / "o.cu")
         ours = subprocess.run([CLI] + argv + ["-o", "o.cu", "t.stc"], cwd=tmp_path, stdout=subprocess.PIPE,
                               stderr=subprocess.STDOUT, text=True, timeout=60)
-        try:
-            ref = subprocess.run([REF] + argv + ["-o", "r.cu", "t.stc"], cwd=tmp_path, stdout=subprocess.PIPE,
-                                 stderr=subprocess.STDOUT, text=True, timeout=5)
-        except subprocess.TimeoutExpired:
+        if ref["rc"] is None:                # the reference timed out on this input
             continue
         compared += 1
-        assert ours.returncode == ref.returncode, (seed, argv, text, ours.stdout, ref.stdout)
-        assert ours.stdout.strip().splitlines()[:1] == ref.stdout.strip().splitlines()[:1], (seed, argv, text)
-        if ref.returncode != 0:
+        assert ours.returncode == ref["rc"], (seed, argv, text, ours.stdout, ref)
+        assert ours.stdout.strip().splitlines()[:1] == ([ref["first"]] if ref["first"] else []), (seed, argv, text)
+        if ref["rc"] != 0:
             continue
         emitted += 1
-        mine, theirs = _defines(tmp_path / "o.cu"), _defines(tmp_path / "r.cu")
+        mine = _defines(tmp_path / "o.cu")
         pairs = {"M": "GridM", "N": "GridN", "Halo": "Halo"}
         if is3d:
             pairs["L"] = "GridL"
         if has_iterations:                 # without the key the reference prints an uninitialised int
             pairs["Iterations"] = "Iterations"
         for r, o in pairs.items():
-            assert theirs.get(r) == mine.get(o), (seed, argv, r, theirs.get(r), mine.get(o), text)
+            assert ref["macros"][r] == mine.get(o), (seed, argv, r, ref["macros"][r], mine.get(o), text)
     assert compared >= 150 and emitted >= 60, (compared, emitted)
 
 
-@pytest.mark.skipif(not os.path.exists(REF), reason="oracle/_ref/drstencil_ref not built")
 def test_random_descriptions_compose_like_the_reference(built, tmp_path):
     """The gold expression the reference emits (`--check`) for random descriptions and steps: term order,
     offsets and the 6-significant-digit coefficient literals, plus the Halo / Dist / Range macros -- against
     BOTH the oracle's restatement (oracle/oracle.py) and the product's C ABI (drs_stencil_compose / _terms /
     _term_text / _analyze).  Many-digit coefficients (0.3333333 composed three times) exercise the literal
-    round trip (/root/reference/drstencil_2d.hpp:174,231-251)."""
-    import sys
-    sys.path.insert(0, os.path.join(ROOT, "tests", "golden"))
-    from make_golden import parse_emitted
+    round trip (drstencil_2d.hpp:174,231-251 of the original)."""
+    from make_cli_golden import compose_argv, terms_digest
     import drstencil_b200 as drs
     from oracle import oracle
     checked = 0
-    for seed in range(1000, 1120):
-        rng = random.Random(seed)
-        is3d = rng.random() < 0.4
-        text, _ = random_stc(rng, is3d)
+    assert [r["seed"] for r in GOLDEN["compose"]] == list(range(1000, 1120))
+    for ref in GOLDEN["compose"]:
+        seed = ref["seed"]
+        text, is3d, step, dist, mf, _ = compose_argv(random.Random(seed))
         (tmp_path / "t.stc").write_text(text)
-        step = rng.choice([1, 2, 2, 3])
-        dist = rng.choice([0, 0, 1, 2])
-        mf = rng.choice([5, 5, 1, 9])
-        argv = (["--3d"] if is3d else []) + ["--step", str(step), "--merge-forward", str(mf)] + \
-            (["--dist", str(dist)] if dist else []) + ["--streaming", "--bx", "256", "--sn", "64", "--check", "-o", "r.cu", "t.stc"]
-        if os.path.exists(tmp_path / "r.cu"):
-            os.remove(tmp_path / "r.cu")
-        try:
-            ref = subprocess.run([REF] + argv, cwd=tmp_path, stdout=subprocess.PIPE, stderr=subprocess.STDOUT, text=True, timeout=5)
-        except subprocess.TimeoutExpired:
+        if ref["rc"] is None:
             continue
         # oracle restatement
         s = oracle.parse_stc(str(tmp_path / "t.stc"), is3d)
@@ -128,22 +114,22 @@ def test_random_descriptions_compose_like_the_reference(built, tmp_path):
         part = oracle.partition(pts, s.dim, d, mf)
         # product
         st = drs.Stencil.from_file(str(tmp_path / "t.stc"), is3d).compose(step)
-        if ref.returncode == 1:
-            assert "No data to reuse" in ref.stdout and part is None, (seed, text)
+        if ref["rc"] == 1:
+            assert "No data to reuse" in ref["first"] and part is None, (seed, text)
             with pytest.raises(drs.DrsError):
                 st.analyze(dist, mf)
             continue
-        if ref.returncode != 0:
+        if ref["rc"] != 0:
             continue                        # "Invalid configuration!" depends on the tile, not on the operator
-        macros, terms = parse_emitted(open(tmp_path / "r.cu").read(), is3d)
+        macros = ref["macros"]
         keys = sorted(pts)
-        assert [list(k) for k in keys] == [t[:3] for t in terms], (seed, text)
-        assert [oracle.literal_text(pts[k]) for k in keys] == [t[3] for t in terms], (seed, text)
+        assert len(keys) == ref["nterms"], (seed, text)
+        assert terms_digest([list(k) + [oracle.literal_text(pts[k])] for k in keys]) == ref["terms_sha256"], (seed, text)
         assert macros["Halo"] == halo and macros["Dist"] == d and macros["Range"] == part["high"] - part["low"] + 1, (seed, text)
         mine = st.terms()
-        assert [list(t[:3]) for t in mine] == [t[:3] for t in terms], (seed, text)
-        assert st.term_texts() == [t[3] for t in terms], (seed, text)
-        assert [t[3] for t in mine] == [float(t[3]) for t in terms], (seed, text)
+        texts = st.term_texts()
+        assert terms_digest([list(t[:3]) + [x] for t, x in zip(mine, texts)]) == ref["terms_sha256"], (seed, text)
+        assert [t[3] for t in mine] == [float(x) for x in texts], (seed, text)
         a = st.analyze(dist, mf)
         assert (a["halo"], a["dist"], a["range"]) == (macros["Halo"], macros["Dist"], macros["Range"]), (seed, text)
         checked += 1
