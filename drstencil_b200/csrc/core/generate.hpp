@@ -106,6 +106,14 @@ enum KnobBit { KB_STEP = 0, KB_DIST, KB_STREAMING, KB_BX, KB_BY, KB_SN, KB_UNROL
 
 inline bool factorise_rows(KernelSpec& s);
 
+// A deferred scale eta makes the values of level s carry eta^-s and the store multiply by eta^ts.  Both have to stay
+// far inside the dtype's range: a leading coefficient of 1e-10 at depth 4 in fp32 would give levels of ~1e40 (Inf)
+// and a scale of 1e-40 (subnormal).  2^60 leaves fp32 a factor 2^68 for the values themselves, 2^500 leaves fp64
+// 2^524.  (The shipped stencils need at most 13.3 bits: 2d9pt_cross at depth 4.)
+inline bool scale_in_range(double eta, int ts, int dtype) {
+    return ts * std::fabs(std::log2(std::fabs(eta))) <= (dtype == DRS_F64 ? 500.0 : 60.0);
+}
+
 // Chooses the specialisation.  Returns "" or an error text (-> DRS_E_ARG).
 //
 // How the reference's knobs (main.cpp:12-56) map onto this engine when given explicitly:
@@ -244,7 +252,10 @@ inline std::string choose_spec(const Stencil& base_in, const drs_knobs& k, Kerne
         // by eta^ts.  Tolerance-checked modes only (the bit-exact chain is never scaled).
         for (const Term& t : s.chain) {
             const int lead = s.dim == 3 ? t.dk : t.dj;
-            if (lead == -(s.dim == 3 ? s.rk : s.rj)) { if (t.coef != 0.0 && t.coef != 1.0) s.fscale = t.coef; break; }
+            if (lead == -(s.dim == 3 ? s.rk : s.rj)) {
+                if (t.coef != 0.0 && t.coef != 1.0 && scale_in_range(t.coef, s.ts, s.dtype)) s.fscale = t.coef;
+                break;
+            }
         }
     }
     // --- geometry ---
@@ -419,7 +430,7 @@ inline bool factorise_rows(KernelSpec& s) {
     const int base = hrow_ops(s.fh);
     double best_eta = 1.0; int best = base;
     for (double eta : s.fh) {
-        if (eta == 0.0 || eta == 1.0) continue;
+        if (eta == 0.0 || eta == 1.0 || !scale_in_range(eta, s.ts, s.dtype)) continue;
         std::vector<double> h2 = s.fh;
         for (double& v : h2) v /= eta;
         const int ops = hrow_ops(h2);
