@@ -90,6 +90,9 @@ def lib():
         "drs_plan_source": (ctypes.c_char_p, [vp]),
         "drs_plan_note": (ctypes.c_char_p, [vp]),
         "drs_plan_cache_key": (ctypes.c_char_p, [vp]),
+        "drs_plan_pair_source": (ctypes.c_char_p, [vp]),
+        "drs_plan_pair_cache_key": (ctypes.c_char_p, [vp]),
+        "drs_plan_pair_split": (i32, [vp, i32, P(i32), P(i32)]),
         "drs_sweep": (i32, [vp, vp, vp, vp]),
         "drs_gold_sweep": (i32, [vp, vp, vp, vp]),
         "drs_run": (i32, [vp, vp, vp, i32, vp, P(i32)]),
@@ -399,6 +402,21 @@ class Plan:
     @property
     def cache_key(self) -> str:
         return lib().drs_plan_cache_key(self._h).decode()
+
+    @property
+    def pair_source(self) -> str:
+        """Translation unit of the exact pair kernel run() uses on this plan ("" = none: one launch per sweep)."""
+        return lib().drs_plan_pair_source(self._h).decode()
+
+    @property
+    def pair_cache_key(self) -> str:
+        return lib().drs_plan_pair_cache_key(self._h).decode()
+
+    def pair_split(self, iterations: int):
+        """(pairs, singles): run() performs `pairs` exact pair launches, then `singles` single sweeps."""
+        p, s = ctypes.c_int(), ctypes.c_int()
+        _check(lib().drs_plan_pair_split(self._h, iterations, ctypes.byref(p), ctypes.byref(s)))
+        return p.value, s.value
 
     @property
     def halo(self) -> int:

@@ -31,6 +31,9 @@
 extern const char* const drs_embedded_header_names[];
 extern const char* const drs_embedded_header_texts[];
 extern const int drs_embedded_header_count;
+extern const char* const drs_pair_header_names[];
+extern const char* const drs_pair_header_texts[];
+extern const int drs_pair_header_count;
 
 namespace {
 
@@ -183,10 +186,18 @@ std::string cache_dir() {
 const char* kNvrtcOpts[] = {"--gpu-architecture=sm_100a", "-std=c++17", "-lineinfo", "--fmad=false",
                             "-default-device", "--ptxas-options=-v"};
 
-// source -> cubin, through the on-disk cache
-int compile_cubin(const std::string& src, std::vector<char>& cubin, std::string& key_out) {
+// source -> cubin, through the on-disk cache.  The key covers the source, every header the unit may include and the
+// options.  pair: the unit of the exact pair kernel, which may include the kernels/pair/ headers as well (they are part
+// of its key only: the keys of every other unit do not depend on them).
+int compile_cubin(const std::string& src, std::vector<char>& cubin, std::string& key_out, bool pair = false) {
+    std::vector<const char*> names(drs_embedded_header_names, drs_embedded_header_names + drs_embedded_header_count);
+    std::vector<const char*> texts(drs_embedded_header_texts, drs_embedded_header_texts + drs_embedded_header_count);
+    if (pair) {
+        names.insert(names.end(), drs_pair_header_names, drs_pair_header_names + drs_pair_header_count);
+        texts.insert(texts.end(), drs_pair_header_texts, drs_pair_header_texts + drs_pair_header_count);
+    }
     std::string all = src;
-    for (int i = 0; i < drs_embedded_header_count; ++i) all += drs_embedded_header_texts[i];
+    for (const char* t : texts) all += t;
     for (const char* o : kNvrtcOpts) all += o;
     int maj = 0, min = 0;
     Nvrtc& n = nvrtc();
@@ -205,8 +216,7 @@ int compile_cubin(const std::string& src, std::vector<char>& cubin, std::string&
     }
     if (!n.ok) return fail(DRS_E_COMPILE, "NVRTC unavailable: " + n.why);
     Nvrtc::Prog prog = nullptr;
-    int r = n.CreateProgram(&prog, src.c_str(), "drs_generated.cu", drs_embedded_header_count,
-                            drs_embedded_header_texts, drs_embedded_header_names);
+    int r = n.CreateProgram(&prog, src.c_str(), "drs_generated.cu", (int)names.size(), texts.data(), names.data());
     if (r != 0) return fail(DRS_E_COMPILE, "nvrtcCreateProgram failed");
     r = n.CompileProgram(prog, (int)(sizeof kNvrtcOpts / sizeof kNvrtcOpts[0]), kNvrtcOpts);
     size_t logn = 0;
@@ -275,6 +285,14 @@ struct drs_plan {
     drs::KernelSpec spec;
     std::string source, cache_key;
     std::vector<char> cubin;
+    // exact pair launches of drs_run (generate.hpp: pair_spec): their own unit, cubin, module and tensor maps
+    bool pair = false;
+    drs::KernelSpec pspec;
+    std::string pair_source, pair_key;
+    std::vector<char> pair_cubin;
+    CUmodule pmod = nullptr;
+    CUfunction f_pair = nullptr;
+    std::map<const void*, CUtensorMap> ptmaps;
     // device state (bound at first use)
     bool loaded = false;
     int device = -1;
@@ -376,6 +394,13 @@ int ensure_loaded(drs_plan* p) {
     r = d.ModuleGetFunction(&p->f_signal, p->mod, ("signal_" + nm).c_str());
     if (r == CUDA_SUCCESS) r = d.ModuleGetFunction(&p->f_wait, p->mod, ("wait_" + nm).c_str());
     if (r != CUDA_SUCCESS) return fail(DRS_E_CUDA, "cuModuleGetFunction(signal_/wait_): " + cu_err(r));
+    if (p->pair) {
+        r = d.ModuleLoadData(&p->pmod, p->pair_cubin.data());
+        if (r != CUDA_SUCCESS) return fail(DRS_E_CUDA, "cuModuleLoadData(pair): " + cu_err(r));
+        r = d.ModuleGetFunction(&p->f_pair, p->pmod, ("drpair_" + nm).c_str());
+        if (r == CUDA_SUCCESS) r = d.FuncSetAttribute(p->f_pair, CU_FUNC_ATTRIBUTE_MAX_DYNAMIC_SHARED_SIZE_BYTES, p->pspec.smem_bytes());
+        if (r != CUDA_SUCCESS) return fail(DRS_E_CUDA, "cuModuleGetFunction(drpair_): " + cu_err(r));
+    }
     if (cudaMalloc(&p->d_fault, sizeof(int)) != cudaSuccess) return fail(DRS_E_CUDA, "cudaMalloc(fault flag)");
     cudaMemset(p->d_fault, 0, sizeof(int));
     if (cudaMalloc(&p->d_res, 2 * sizeof(double)) != cudaSuccess) return fail(DRS_E_CUDA, "cudaMalloc(result)");
@@ -383,10 +408,11 @@ int ensure_loaded(drs_plan* p) {
     return DRS_OK;
 }
 
-int tensor_map_for(drs_plan* p, const void* base, CUtensorMap** out) {
-    auto it = p->tmaps.find(base);
-    if (it != p->tmaps.end()) { *out = &it->second; return DRS_OK; }
-    const drs::KernelSpec& s = p->spec;
+int tensor_map_for(drs_plan* p, const void* base, CUtensorMap** out, bool pair = false) {
+    std::map<const void*, CUtensorMap>& tmaps = pair ? p->ptmaps : p->tmaps;
+    auto it = tmaps.find(base);
+    if (it != tmaps.end()) { *out = &it->second; return DRS_OK; }
+    const drs::KernelSpec& s = pair ? p->pspec : p->spec;
     if (s.flat != 2 && (reinterpret_cast<uintptr_t>(base) & 15) != 0) return fail(DRS_E_ARG, "device buffers must be 16-byte aligned");
     CUtensorMap m;
     const CUtensorMapDataType dt = s.dtype == DRS_F64 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT64 : CU_TENSOR_MAP_DATA_TYPE_FLOAT32;
@@ -429,8 +455,8 @@ int tensor_map_for(drs_plan* p, const void* base, CUtensorMap** out) {
                                           promo, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
     }
     if (r != CUDA_SUCCESS) return fail(DRS_E_CUDA, "cuTensorMapEncodeTiled: " + cu_err(r));
-    if (p->tmaps.size() > 64) p->tmaps.clear();
-    auto ins = p->tmaps.emplace(base, m);
+    if (tmaps.size() > 64) tmaps.clear();
+    auto ins = tmaps.emplace(base, m);
     *out = &ins.first->second;
     return DRS_OK;
 }
@@ -440,9 +466,10 @@ struct SlowRange { long long lo, hi; };   // output range along the slow axis, l
 // ring = frozen ring width of this launch (spec.halo, or the sub-step's share of it);
 // sub  = restrict the launch to these slow-axis outputs (time-skewed blocks of drs_run_host)
 // seq_off >= 0: this launch is sweep number seq_off of a drs_run_slab call and handles its own step flags
+// spec: the specialisation the launch runs (default: the plan's main one; the exact pair kernel has its own tile)
 void fill_params(const drs_plan* p, const void* in, void* out, DevParams& q, int ring = -1, const SlowRange* sub = nullptr,
-                 int seq_off = -1) {
-    const drs::KernelSpec& s = p->spec;
+                 int seq_off = -1, const drs::KernelSpec* spec = nullptr) {
+    const drs::KernelSpec& s = spec ? *spec : p->spec;
     std::memset(&q, 0, sizeof q);
     q.in = in; q.out = out;
     q.L = p->st.L; q.M = p->st.M; q.N = p->st.N;
@@ -590,6 +617,48 @@ int launch_one(drs_plan* p, const void* in, void* out, cudaStream_t stream, int 
     return DRS_OK;
 }
 
+// One exact pair launch (kernels/pair/drs_pair3d.cuh): two sweeps of drs_run's ping-pong schedule, from the level in
+// `in` to the level two steps later in the interior of `out`.  a / b are the run's buffers: even levels have a's ring,
+// odd ones b's.
+int launch_pair(drs_plan* p, const void* in, void* out, const void* a, const void* b, cudaStream_t stream) {
+    if (in == out) return fail(DRS_E_ARG, "d_in and d_out must differ");
+    CUtensorMap* tm = nullptr;
+    int rc = tensor_map_for(p, in, &tm, true);
+    if (rc != DRS_OK) return rc;
+    CUtensorMap map_in = *tm;          // (the next lookup may clear the cache)
+    rc = tensor_map_for(p, a, &tm, true);
+    if (rc != DRS_OK) return rc;
+    CUtensorMap map_a = *tm;
+    if ((reinterpret_cast<uintptr_t>(out) & 15) != 0) return fail(DRS_E_ARG, "device buffers must be 16-byte aligned");
+    DevParams q;
+    fill_params(p, in, out, q, -1, nullptr, -1, &p->pspec);
+    const long long tiles = (long long)q.nxs * q.nys * q.nzs;
+    if (tiles <= 0) return DRS_OK;
+    if (tiles > 0x7fffffffLL) return fail(DRS_E_ARG, "grid too large");
+    const void* ring_a = a;
+    const void* ring_b = b;
+    void* args[] = {&map_in, &map_a, &q, &ring_a, &ring_b};
+    CUresult r = driver().LaunchKernel(p->f_pair, (unsigned)tiles, 1, 1, (unsigned)(p->pspec.nw * 32), 1, 1,
+                                       (unsigned)p->pspec.smem_bytes(), (CUstream)stream, args, nullptr);
+    if (r != CUDA_SUCCESS) return fail(DRS_E_CUDA, "launch drpair_: " + cu_err(r));
+    p->launches++;
+    return DRS_OK;
+}
+
+// drs_run's n sweeps over (a, b): sweep s writes the interior of bufs[(s+1)%2] from bufs[s%2].  Plans with exact pair
+// launches run p pairs (pair i: bufs[i%2] -> level 2i+2 in bufs[(i+1)%2]) and then s single sweeps (generate.hpp:
+// pair_split); both buffers end exactly as after n single sweeps.
+int enqueue_run(drs_plan* p, void* a, void* b, int n, cudaStream_t stream) {
+    int pairs = 0, singles = n;
+    if (p->pair) drs::pair_split(n, pairs, singles);
+    int rc = DRS_OK;
+    for (int i = 0; i < pairs && rc == DRS_OK; ++i)
+        rc = (i & 1) ? launch_pair(p, b, a, a, b, stream) : launch_pair(p, a, b, a, b, stream);
+    for (int s = 0; s < singles && rc == DRS_OK; ++s)
+        rc = (s & 1) ? launch_sweep(p, b, a, stream) : launch_sweep(p, a, b, stream);
+    return rc;
+}
+
 int check_sizes(const drs::Stencil& st) {
     if (st.M <= 0 || st.N <= 0 || (st.dim == 3 && st.L <= 0)) return fail(DRS_E_ARG, "grid extents must be positive");
     if (st.M > 0x7fffff00LL || st.N > 0x7fffff00LL || st.L > 0x7fffff00LL) return fail(DRS_E_ARG, "extent too large");
@@ -613,8 +682,11 @@ int make_plan(const drs_stencil* s, const drs_knobs* k, drs_plan** out, bool com
         return fail(DRS_E_ARG, err);
     }
     p->source = drs::generate_tu(p->spec);
+    p->pair = drs::pair_spec(p->st, p->spec, p->pspec);
+    if (p->pair) p->pair_source = drs::generate_pair_tu(p->pspec);
     if (compile) {
         rc = compile_cubin(p->source, p->cubin, p->cache_key);
+        if (rc == DRS_OK && p->pair) rc = compile_cubin(p->pair_source, p->pair_cubin, p->pair_key, true);
         if (rc != DRS_OK) { delete p; return rc; }
     }
     *out = p;
@@ -750,6 +822,7 @@ void drs_plan_destroy(drs_plan* p) {
         for (cudaStream_t st : {p->hs_up, p->hs_run, p->hs_dn, p->cap_stream}) if (st) cudaStreamDestroy(st);
         for (auto& g : p->graphs) cudaGraphExecDestroy(g.second.exec);
         if (p->mod) driver().ModuleUnload(p->mod);
+        if (p->pmod) driver().ModuleUnload(p->pmod);
     }
     delete p;
 }
@@ -790,6 +863,8 @@ int drs_plan_get_info(const drs_plan* p, drs_plan_info* info) {
 const char* drs_plan_source(const drs_plan* p) { return p ? p->source.c_str() : ""; }
 const char* drs_plan_note(const drs_plan* p) { return p ? p->spec.note.c_str() : ""; }
 const char* drs_plan_cache_key(const drs_plan* p) { return p ? p->cache_key.c_str() : ""; }
+const char* drs_plan_pair_source(const drs_plan* p) { return p ? p->pair_source.c_str() : ""; }
+const char* drs_plan_pair_cache_key(const drs_plan* p) { return p ? p->pair_key.c_str() : ""; }
 
 int drs_sweep(drs_plan* p, const void* d_in, void* d_out, void* stream) {
     if (!p || !d_in || !d_out) return fail(DRS_E_ARG, "null argument");
@@ -831,13 +906,12 @@ static bool run_graph(drs_plan* p, void* a, void* b, int n, cudaStream_t stream)
         // tensor maps are encoded outside the capture (host-only, but keeps the captured region to launches)
         CUtensorMap* tm = nullptr;
         if (tensor_map_for(p, a, &tm) != DRS_OK || tensor_map_for(p, b, &tm) != DRS_OK) return false;
+        if (p->pair && (tensor_map_for(p, a, &tm, true) != DRS_OK || tensor_map_for(p, b, &tm, true) != DRS_OK)) return false;
         const long long l0 = p->launches;
         if (cudaStreamBeginCapture(p->cap_stream, cudaStreamCaptureModeThreadLocal) != cudaSuccess) {
             cudaGetLastError(); p->use_graph = false; return false;
         }
-        int rc = DRS_OK;
-        for (int s = 0; s < n && rc == DRS_OK; ++s)
-            rc = (s & 1) ? launch_sweep(p, b, a, p->cap_stream) : launch_sweep(p, a, b, p->cap_stream);
+        const int rc = enqueue_run(p, a, b, n, p->cap_stream);
         cudaGraph_t g = nullptr;
         const cudaError_t ce = cudaStreamEndCapture(p->cap_stream, &g);
         const int kernels = (int)(p->launches - l0);
@@ -869,15 +943,29 @@ static int run_schedule(drs_plan* p, void* a, void* b, int iterations, void* str
         }
         n = 0;
     }
-    for (int t = 0; t < iterations; t += 2 * p->spec.step) {
-        rc = gold ? launch_gold(p, a, b, (cudaStream_t)stream) : launch_sweep(p, a, b, (cudaStream_t)stream);
+    for (int t = 0; t < iterations; t += 2 * p->spec.step) n += 2;
+    if (gold) {
+        for (int s = 0; s < n; ++s) {
+            rc = (s & 1) ? launch_gold(p, b, a, (cudaStream_t)stream) : launch_gold(p, a, b, (cudaStream_t)stream);
+            if (rc != DRS_OK) return rc;
+        }
+    } else {
+        rc = enqueue_run(p, a, b, n, (cudaStream_t)stream);
         if (rc != DRS_OK) return rc;
-        rc = gold ? launch_gold(p, b, a, (cudaStream_t)stream) : launch_sweep(p, b, a, (cudaStream_t)stream);
-        if (rc != DRS_OK) return rc;
-        n += 2;
     }
     if (sweeps) *sweeps = n;
     return DRS_OK;
+}
+
+int drs_plan_pair_split(const drs_plan* p, int iterations, int* pairs, int* singles) {
+    if (!p) return fail(DRS_E_ARG, "null plan");
+    int n = 0;
+    for (int t = 0; t < iterations; t += 2 * p->spec.step) n += 2;
+    int np = 0, ns = n;
+    if (p->pair) drs::pair_split(n, np, ns);
+    if (pairs) *pairs = np;
+    if (singles) *singles = ns;
+    return n;
 }
 
 int drs_run(drs_plan* p, void* d_a, void* d_b, int iterations, void* stream, int* sweeps) {

@@ -106,6 +106,17 @@ enum KnobBit { KB_STEP = 0, KB_DIST, KB_STREAMING, KB_BX, KB_BY, KB_SN, KB_UNROL
 
 inline bool factorise_rows(KernelSpec& s);
 
+// A 3D grid whose arrays are each >= 1 GiB: nothing of one sweep is left in the L2 (126 MB on B200) for the next.
+// Such grids get the L2 evict_last policy on their plane loads (keep_planes) and drs_run's exact pair launches.
+inline bool far_beyond_l2(const Stencil& st, int dtype) {
+    return st.dim == 3 && (long double)st.L * (long double)st.M * (long double)st.N * (dtype == DRS_F64 ? 8 : 4) >= 1073741824.0L;
+}
+
+// The fused 3D temporal kernel's tile keeps useful columns at this depth (and depth <= 4)
+inline bool fused3d_fits(int emax, int vec, int step) {
+    return 32 * vec - 2 * (((step - 1) * emax + vec - 1) / vec * vec) >= vec && step <= 4;
+}
+
 // A deferred scale eta makes the values of level s carry eta^-s and the store multiply by eta^ts.  Both have to stay
 // far inside the dtype's range: a leading coefficient of 1e-10 at depth 4 in fp32 would give levels of ~1e40 (Inf)
 // and a scale of 1e-40 (subnormal).  2^60 leaves fp32 a factor 2^68 for the values themselves, 2^500 leaves fp64
@@ -184,8 +195,7 @@ inline std::string choose_spec(const Stencil& base_in, const drs_knobs& k, Kerne
     }
     // (measured on B200, c5: 388.5 -> 393.0 GStencil/s, depth 2 644.5 -> 649.6; evict_first instead: 321 / 463;
     // DRS_NO_LD_HINT is the A/B switch)
-    s.keep_planes = s.dim == 3 && !s.flat && !std::getenv("DRS_NO_LD_HINT") &&
-                    (long double)st.L * (long double)st.M * (long double)st.N * (s.dtype == DRS_F64 ? 8 : 4) >= 1073741824.0L;
+    s.keep_planes = s.dim == 3 && !s.flat && !std::getenv("DRS_NO_LD_HINT") && far_beyond_l2(st, s.dtype);
     bool temporal = (k.fuse == DRS_FUSE_TEMPORAL) && k.step > 1;
     if (temporal) {
         // The reference multiplies the operator out and prints the result with 6 significant digits
@@ -214,7 +224,7 @@ inline std::string choose_spec(const Stencil& base_in, const drs_knobs& k, Kerne
         temporal = false;
         int emax = 0;
         for (const auto& [p, c] : st.base) emax = std::max(emax, std::abs(std::get<2>(p)));
-        const bool fits = 32 * vec - 2 * (((k.step - 1) * emax + vec - 1) / vec * vec) >= vec && k.step <= 4;
+        const bool fits = fused3d_fits(emax, vec, k.step);
         if (fits && !(k.reserved[6] & 2)) fused3d = true;
         else {
             multi3d = true;
@@ -606,6 +616,86 @@ inline std::string generate_tu(const KernelSpec& s) {
     else if (s.tma_ok)
         o << "#include \"" << (s.fused3d ? "drs_sweep3d_t.cuh" : s.share3d ? "drs_sweep3d_cta.cuh" : s.dim == 3 ? "drs_sweep3d.cuh" : "drs_sweep2d.cuh") << "\"\n";
     o << "#include \"drs_gold.cuh\"\n";
+    return o.str();
+}
+
+// ---- exact pair launches (drs_run on step-1 3D plans far beyond the L2; kernels/pair/drs_pair3d.cuh) ----------------
+
+// The specialisation of the pair kernel for a plan whose main specialisation is `m`, or false where the plan keeps one
+// launch per sweep: 3D, step 1, the single-step TMA sweep with a 16-byte row pitch, arrays of >= 1 GiB, and an operator
+// whose depth-2 tile keeps useful columns.  The geometry is that of the fused temporal kernel at depth 2 (8 warps x 4
+// rows, two CTAs per SM, chunks of 128 planes); the ring is that of one step.
+inline bool pair_spec(const Stencil& st, const KernelSpec& m, KernelSpec& s) {
+    if (m.dim != 3 || m.step != 1 || m.ts != 1 || m.flat || m.reuse || !m.tma_ok || m.sub_launches != 1) return false;
+    if (!far_beyond_l2(st, m.dtype) || !fused3d_fits(m.e, m.vec(), 2)) return false;
+    s = KernelSpec();
+    s.dim = 3; s.dtype = m.dtype; s.step = 1; s.fuse = m.fuse; s.ts = 2;
+    s.halo = m.halo; s.base_order = m.base_order;
+    s.rk = m.rk; s.rj = m.rj; s.e = m.e;
+    s.chain = m.chain; s.gold = m.gold;
+    s.fused3d = true;
+    s.keep_planes = m.keep_planes;
+    s.name = m.name;
+    s.nw = 8; s.ry = 4; s.st = 2; s.chunk = 128; s.minb = 2;
+    // two levels of partial sums stay within what 3d7pt fills at 4 rows (96 of the 128 registers): fewer rows per
+    // thread for deeper k windows, more warps where the tile would then lose all its rows
+    auto live = [&](int ry) { return 2 * (2 * s.rk + 1) * ry * s.vec() * (s.esize() / 4); };
+    while (s.ry > 1 && live(s.ry) > 96) s.ry /= 2;
+    if (s.tile_rows_useful() < 1) { s.nw = 16; s.minb = 1; }
+    const long long slow_out = std::max<long long>(1, st.L - 2 * s.halo);
+    if (s.chunk > slow_out) s.chunk = (int)slow_out;
+    return s.tile_rows_useful() >= 1 && s.smem_bytes() <= 227 * 1024;
+}
+
+// (p, s): drs_run's n sweeps as p pair launches followed by s single sweeps.  p is even, so that A holds an even level
+// again when the single sweeps start, and the last two sweeps are single ones, so that B ends at level n - 1.
+inline void pair_split(int n, int& pairs, int& singles) {
+    singles = n < 2 ? n : (((n - 2) / 2) % 2 == 0 ? 2 : 4);
+    if (singles > n) singles = n;
+    pairs = (n - singles) / 2;
+}
+
+// Exact 3D scatter: every output receives its terms in the order of the single-step chain (emit_chain: MUL(t1),
+// FMA(t0), FMA(t2), ... -- gold order, which ascends in dk, so plane arrival order follows it), with DRS_CHAIN's
+// literals and without a deferred scale.  The one exception to arrival order is the chain's start: when t0 lies on an
+// earlier plane than t1 (it is then alone on that plane; every star operator), t0's operand is parked in the output's
+// own partial-sum slot -- still unused at that point -- until t1's plane arrives, and the output starts there as
+// fma(t0, c0, t1 * c1).  No register beyond the partial sums is needed.
+inline void emit_scatter3_exact(std::ostringstream& o, const KernelSpec& s) {
+    const std::vector<Term>& t = s.chain;
+    auto U = [](const Term& x) { return "U(" + std::to_string(x.dj) + ", " + std::to_string(x.di) + ")"; };
+    auto C = [](const Term& x) { return "(real)(" + coef_literal_text(x.coef) + ")"; };
+    o << "#define DRS_SCATTER3(P, U)";
+    for (int dk = -s.rk; dk <= s.rk; ++dk) {
+        const std::string P = "P(" + std::to_string(dk) + ")";
+        if (t.size() == 1) {
+            if (t[0].dk == dk) o << " \\\n    " << P << " = rmul(" << U(t[0]) << ", " << C(t[0]) << ");";
+            continue;
+        }
+        if (t[0].dk == dk && t[1].dk != dk) o << " \\\n    " << P << " = " << U(t[0]) << ";";
+        if (t[1].dk == dk)
+            o << " \\\n    " << P << " = rfma(" << (t[0].dk == dk ? U(t[0]) : P) << ", " << C(t[0]) << ", rmul(" << U(t[1]) << ", "
+              << C(t[1]) << "));";
+        for (size_t q = 2; q < t.size(); ++q)
+            if (t[q].dk == dk) o << " \\\n    " << P << " = rfma(" << U(t[q]) << ", " << C(t[q]) << ", " << P << ");";
+    }
+    o << "\n";
+}
+
+// The pair kernel's translation unit (includes kernels/pair/drs_pair3d.cuh, nothing of the plan's main unit)
+inline std::string generate_pair_tu(const KernelSpec& s) {
+    std::ostringstream o;
+    o << "// generated by drstencil-b200 for sm_100a -- stencil '" << s.name << "', 3D, " << (s.dtype == DRS_F64 ? "fp64" : "fp32")
+      << ", two exact single steps per launch\n";
+    o << "#define DRS_DIM 3\n";
+    o << "#define DRS_T " << (s.dtype == DRS_F64 ? "double" : "float") << "\n";
+    o << "#define DRS_PAIR_NAME drpair_" << s.name << "\n";
+    o << "#define DRS_HALO " << s.halo << "\n";
+    o << "#define DRS_RK " << s.rk << "\n#define DRS_RJ " << s.rj << "\n#define DRS_E " << s.e << "\n";
+    o << "#define DRS_NW " << s.nw << "\n#define DRS_ST " << s.st << "\n#define DRS_RY " << s.ry << "\n#define DRS_MINB " << s.minb << "\n";
+    if (s.keep_planes) o << "#ifndef DRS_LD_HINT\n#define DRS_LD_HINT 1\n#endif\n";
+    emit_scatter3_exact(o, s);
+    o << "#include \"drs_pair3d.cuh\"\n";
     return o.str();
 }
 

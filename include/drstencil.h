@@ -130,6 +130,9 @@ const char *drs_plan_source(const drs_plan *p);
 const char *drs_plan_note(const drs_plan *p);
 /* key of the compiled cubin in the on-disk cache (<cache dir>/<key>.cubin) */
 const char *drs_plan_cache_key(const drs_plan *p);
+/* the translation unit / cache key of the exact pair kernel drs_run uses on this plan, "" if it uses none */
+const char *drs_plan_pair_source(const drs_plan *p);
+const char *drs_plan_pair_cache_key(const drs_plan *p);
 
 /* one `dr_<name><<<grid, block>>>(d_in, d_out)` (codegen_2d.hpp:606): advances the interior
  * [Halo, dim-Halo) by `step` timesteps; the Halo ring of d_out is not written.  d_in != d_out.
@@ -139,8 +142,15 @@ int drs_sweep(drs_plan *p, const void *d_in, void *d_out, void *stream);
  * one-thread-per-point evaluation of the composed operator, for on-device self-checks */
 int drs_gold_sweep(drs_plan *p, const void *d_in, void *d_out, void *stream);
 /* the emitted host loop (codegen_2d.hpp:610-613): for (t = 0; t < iterations; t += 2*step)
- * { sweep(A,B); sweep(B,A); } -- result is in A.  Writes the number of sweeps to *sweeps. */
+ * { sweep(A,B); sweep(B,A); } -- result is in A.  Writes the number of sweeps to *sweeps.
+ * On 3D step-1 plans whose arrays are >= 1 GiB each (16-byte row pitch, an operator the depth-2 tile fits) the
+ * sweeps run as exact pair launches -- one kernel computes two sweeps, bit for bit, with each level's ring taken from
+ * the buffer that level lives in -- followed by two or four single sweeps; A and B end exactly as after the plain
+ * loop (drs_plan_pair_split). */
 int drs_run(drs_plan *p, void *d_a, void *d_b, int iterations, void *stream, int *sweeps);
+/* how drs_run splits the sweeps of `iterations` timesteps: *pairs pair launches, then *singles single sweeps
+ * (*pairs = 0 on plans without pair launches); returns the number of sweeps.  Needs no GPU. */
+int drs_plan_pair_split(const drs_plan *p, int iterations, int *pairs, int *singles);
 /* drs_run replays its launches as one CUDA graph per (d_a, d_b, sweep count) -- same kernels, same
  * order, without the gap between dependent launches (matters for grids as small as 4096^2).  On
  * by default; a stream that is itself being captured always gets plain launches.  0 switches it off. */
