@@ -15,6 +15,7 @@
 #include <cstdlib>
 #include <cstring>
 #include <fstream>
+#include <functional>
 #include <map>
 #include <mutex>
 #include <sstream>
@@ -305,14 +306,15 @@ struct drs_plan {
     void* h_dev[2] = {nullptr, nullptr};  // buffers owned by drs_run_host
     bool h_dev_b_ring_zero = false;       // h_dev[1]'s frozen ring still holds the zeros it was cleared to
     long long host_block = 0;             // drs_plan_set_host_block: 0 = auto, < 0 = no streaming
-    cudaStream_t hs_up = nullptr, hs_run = nullptr, hs_dn = nullptr;   // streams of the streamed drs_run_host
+    cudaStream_t hs_up = nullptr, hs_run = nullptr, hs_dn = nullptr;   // streams of the streamed host runs
     void* scratch[2] = {nullptr, nullptr};  // intermediate time levels of multi-launch 3D temporal sweeps
     long long launches = 0;
-    // drs_run replays its launch sequence as a CUDA graph (one per buffer pair and sweep count)
+    // drs_run and drs_run_slab replay their launch sequences as CUDA graphs (run_graph), one per A, B, sweep
+    // count and sequence (true: drs_run_slab's; a slab plan may run either on the same buffers)
     bool use_graph = true;
     cudaStream_t cap_stream = nullptr;
     struct RunGraph { cudaGraphExec_t exec; int kernels; };
-    std::map<std::tuple<const void*, const void*, int>, RunGraph> graphs;
+    std::map<std::tuple<const void*, const void*, int, bool>, RunGraph> graphs;
     // slab mode
     bool slab = false;
     long long g_slow = 0, lo = 0, hi = 0;
@@ -327,7 +329,6 @@ struct drs_plan {
     void* upper_flag = nullptr;
     void* d_sync = nullptr;               // { long long seq_base; unsigned face_cnt[2]; }
     long long slab_seq = 0;
-    std::map<int, RunGraph> slab_graphs;  // launch sequence of drs_run_slab per sweep count
 
     long long local_slow() const { return spec.dim == 3 ? st.L : st.M; }
 };
@@ -415,46 +416,34 @@ int tensor_map_for(drs_plan* p, const void* base, CUtensorMap** out, bool pair =
     const drs::KernelSpec& s = pair ? p->pspec : p->spec;
     if (s.flat != 2 && (reinterpret_cast<uintptr_t>(base) & 15) != 0) return fail(DRS_E_ARG, "device buffers must be 16-byte aligned");
     CUtensorMap m;
-    const CUtensorMapDataType dt = s.dtype == DRS_F64 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT64 : CU_TENSOR_MAP_DATA_TYPE_FLOAT32;
-    const cuuint64_t es = (cuuint64_t)s.esize();
-    CUresult r;
-    // L2 promotion of the TMA fetches: 256 B for plane boxes (c5 1536^3: 9.54 -> 9.40 ms, c4 +0.5 %; none / 64 B /
-    // 128 B are equal), 128 B for row boxes (2D: no difference).  DRS_TMA_L2PROMO=0..3 overrides (development aid).
-    CUtensorMapL2promotion promo = s.dim == 3 ? CU_TENSOR_MAP_L2_PROMOTION_L2_256B : CU_TENSOR_MAP_L2_PROMOTION_L2_128B;
-    if (const char* e = getenv("DRS_TMA_L2PROMO")) promo = (CUtensorMapL2promotion)atoi(e);
     if (s.flat == 2) {
         // the kernel fills its stages with cp.async and uses no tensor map: the parameter slot carries zeros
         std::memset(&m, 0, sizeof m);
-        r = CUDA_SUCCESS;
-    } else if (s.flat == 1) {
-        // the whole array as one row of a {total, 1} tensor; a tile arrives as one box of wb() + vec() elements per row,
-        // each starting on a 16-byte boundary (a rank-1 map is not an option: the encoder wants a stride array)
-        const cuuint64_t total = (cuuint64_t)p->st.L * (cuuint64_t)p->st.M * (cuuint64_t)p->st.N;
-        cuuint64_t dims[2] = {total, 1};
-        cuuint64_t strides[1] = {(total * es + 15) / 16 * 16};
-        cuuint32_t box[2] = {(cuuint32_t)(s.wb() + s.vec()), 1};
-        cuuint32_t estr[2] = {1, 1};
-        r = driver().TensorMapEncodeTiled(&m, dt, 2, const_cast<void*>(base), dims, strides, box, estr,
-                                          CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE,
-                                          promo, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    } else if (s.dim == 2) {
-        cuuint64_t dims[2] = {(cuuint64_t)p->st.N, (cuuint64_t)p->st.M};
-        cuuint64_t strides[1] = {(cuuint64_t)p->st.N * es};
-        cuuint32_t box[2] = {(cuuint32_t)s.wb(), (cuuint32_t)s.rb};
-        cuuint32_t estr[2] = {1, 1};
-        r = driver().TensorMapEncodeTiled(&m, dt, 2, const_cast<void*>(base), dims, strides, box, estr,
-                                          CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE,
-                                          promo, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
     } else {
-        cuuint64_t dims[3] = {(cuuint64_t)p->st.N, (cuuint64_t)p->st.M, (cuuint64_t)p->st.L};
-        cuuint64_t strides[2] = {(cuuint64_t)p->st.N * es, (cuuint64_t)p->st.N * (cuuint64_t)p->st.M * es};
-        cuuint32_t box[3] = {(cuuint32_t)s.wb(), (cuuint32_t)s.box_rows(), 1};
-        cuuint32_t estr[3] = {1, 1, 1};
-        r = driver().TensorMapEncodeTiled(&m, dt, 3, const_cast<void*>(base), dims, strides, box, estr,
-                                          CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE,
-                                          promo, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+        const CUtensorMapDataType dt = s.dtype == DRS_F64 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT64 : CU_TENSOR_MAP_DATA_TYPE_FLOAT32;
+        const cuuint64_t es = (cuuint64_t)s.esize(), L = p->st.L, M = p->st.M, N = p->st.N;
+        // L2 promotion of the TMA fetches: 256 B for plane boxes (c5 1536^3: 9.54 -> 9.40 ms, c4 +0.5 %; none / 64 B /
+        // 128 B are equal), 128 B for row boxes (2D: no difference).  DRS_TMA_L2PROMO=0..3 overrides (development aid).
+        CUtensorMapL2promotion promo = s.dim == 3 ? CU_TENSOR_MAP_L2_PROMOTION_L2_256B : CU_TENSOR_MAP_L2_PROMOTION_L2_128B;
+        if (const char* e = getenv("DRS_TMA_L2PROMO")) promo = (CUtensorMapL2promotion)atoi(e);
+        // 2D: rows of N elements, boxes of wb() x rb; 3D: planes of M rows, boxes of wb() x box_rows() x 1
+        cuuint32_t rank = s.dim;
+        cuuint64_t dims[3] = {N, M, L}, strides[2] = {N * es, N * M * es};
+        cuuint32_t box[3] = {(cuuint32_t)s.wb(), (cuuint32_t)(s.dim == 3 ? s.box_rows() : s.rb), 1};
+        const cuuint32_t estr[3] = {1, 1, 1};
+        if (s.flat == 1) {
+            // the whole array as one row of a {total, 1} tensor; a tile arrives as one box of wb() + vec() elements per
+            // row, each starting on a 16-byte boundary (a rank-1 map is not an option: the encoder wants a stride array)
+            rank = 2;
+            dims[0] = L * M * N; dims[1] = 1;
+            strides[0] = (dims[0] * es + 15) / 16 * 16;
+            box[0] = (cuuint32_t)(s.wb() + s.vec()); box[1] = 1;
+        }
+        const CUresult r = driver().TensorMapEncodeTiled(&m, dt, rank, const_cast<void*>(base), dims, strides, box, estr,
+                                                         CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE,
+                                                         promo, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+        if (r != CUDA_SUCCESS) return fail(DRS_E_CUDA, "cuTensorMapEncodeTiled: " + cu_err(r));
     }
-    if (r != CUDA_SUCCESS) return fail(DRS_E_CUDA, "cuTensorMapEncodeTiled: " + cu_err(r));
     if (tmaps.size() > 64) tmaps.clear();
     auto ins = tmaps.emplace(base, m);
     *out = &ins.first->second;
@@ -645,6 +634,24 @@ int launch_pair(drs_plan* p, const void* in, void* out, const void* a, const voi
     return DRS_OK;
 }
 
+// The slab step-flag kernels (drs_gold.cuh): signal_ release-stores `value` into the non-null remote flag words;
+// wait_ waits until the selected words of `flags` (lower, upper) hold >= value, or sets the fault flag after 5 s.
+int launch_signal(drs_plan* p, cudaStream_t stream, void* lower, void* upper, long long value) {
+    void* args[] = {&lower, &upper, &value};
+    CUresult r = driver().LaunchKernel(p->f_signal, 1, 1, 1, 32, 1, 1, 0, (CUstream)stream, args, nullptr);
+    if (r != CUDA_SUCCESS) return fail(DRS_E_CUDA, "launch signal_: " + cu_err(r));
+    p->launches++;
+    return DRS_OK;
+}
+
+int launch_wait(drs_plan* p, cudaStream_t stream, const void* flags, int lo, int hi, long long value) {
+    void* args[] = {(void*)&flags, &lo, &hi, &value, &p->d_fault};
+    CUresult r = driver().LaunchKernel(p->f_wait, 1, 1, 1, 32, 1, 1, 0, (CUstream)stream, args, nullptr);
+    if (r != CUDA_SUCCESS) return fail(DRS_E_CUDA, "launch wait_: " + cu_err(r));
+    p->launches++;
+    return DRS_OK;
+}
+
 // drs_run's n sweeps over (a, b): sweep s writes the interior of bufs[(s+1)%2] from bufs[s%2].  Plans with exact pair
 // launches run p pairs (pair i: bufs[i%2] -> level 2i+2 in bufs[(i+1)%2]) and then s single sweeps (generate.hpp:
 // pair_split); both buffers end exactly as after n single sweeps.
@@ -818,7 +825,6 @@ void drs_plan_destroy(drs_plan* p) {
         for (void* b : p->h_dev) if (b) cudaFree(b);
         for (void* b : p->scratch) if (b) cudaFree(b);
         if (p->d_sync) cudaFree(p->d_sync);
-        for (auto& g : p->slab_graphs) cudaGraphExecDestroy(g.second.exec);
         for (cudaStream_t st : {p->hs_up, p->hs_run, p->hs_dn, p->cap_stream}) if (st) cudaStreamDestroy(st);
         for (auto& g : p->graphs) cudaGraphExecDestroy(g.second.exec);
         if (p->mod) driver().ModuleUnload(p->mod);
@@ -883,35 +889,36 @@ int drs_gold_sweep(drs_plan* p, const void* d_in, void* d_out, void* stream) {
 static void drop_graphs(drs_plan* p) {
     for (auto& g : p->graphs) cudaGraphExecDestroy(g.second.exec);
     p->graphs.clear();
-    for (auto& g : p->slab_graphs) cudaGraphExecDestroy(g.second.exec);
-    p->slab_graphs.clear();
 }
 
-// The launch sequence of drs_run as an instantiated CUDA graph: built once per (A, B, sweep count) by
-// capturing the very same cuLaunchKernel calls on a private stream, replayed with one
-// cudaGraphLaunch.  Saves the per-launch gap between dependent kernels, which is what separates a
-// 45 us sweep (c1: 4096^2) from the roofline (47.2 -> 45.4 us per sweep on B200).  Returns false
-// (and switches graphs off for the plan) if anything about the capture fails; the caller then
-// launches directly.
-static bool run_graph(drs_plan* p, void* a, void* b, int n, cudaStream_t stream) {
+// A launch sequence as an instantiated CUDA graph: built once per key by capturing the very same
+// cuLaunchKernel calls (enqueue(stream)) on a private stream, replayed with one cudaGraphLaunch.  Saves the
+// per-launch gap between dependent kernels, which is what separates a 45 us sweep (c1: 4096^2) from the
+// roofline (47.2 -> 45.4 us per sweep on B200).  Returns false when the caller must launch directly: graphs
+// are off, the caller is capturing `stream` itself, a tensor map cannot be encoded, or anything about the
+// capture fails (which switches graphs off for the plan).
+static bool run_graph(drs_plan* p, void* a, void* b, int n, bool slab, cudaStream_t stream,
+                      const std::function<int(cudaStream_t)>& enqueue) {
+    if (!p->use_graph) return false;
     cudaStreamCaptureStatus cs = cudaStreamCaptureStatusNone;
     if (cudaStreamIsCapturing(stream, &cs) != cudaSuccess) { cudaGetLastError(); return false; }
-    if (cs != cudaStreamCaptureStatusNone) return false;      // the caller is capturing us: launch directly
-    const auto key = std::make_tuple((const void*)a, (const void*)b, n);
+    if (cs != cudaStreamCaptureStatusNone) return false;
+    const auto key = std::make_tuple((const void*)a, (const void*)b, n, slab);
     auto it = p->graphs.find(key);
     if (it == p->graphs.end()) {
         if (!p->cap_stream && cudaStreamCreateWithFlags(&p->cap_stream, cudaStreamNonBlocking) != cudaSuccess) {
             cudaGetLastError(); p->use_graph = false; return false;
         }
-        // tensor maps are encoded outside the capture (host-only, but keeps the captured region to launches)
+        // tensor maps are encoded outside the capture (host-only, but keeps the captured region to launches);
+        // only drs_run's sequence has pair launches
         CUtensorMap* tm = nullptr;
         if (tensor_map_for(p, a, &tm) != DRS_OK || tensor_map_for(p, b, &tm) != DRS_OK) return false;
-        if (p->pair && (tensor_map_for(p, a, &tm, true) != DRS_OK || tensor_map_for(p, b, &tm, true) != DRS_OK)) return false;
+        if (p->pair && !slab && (tensor_map_for(p, a, &tm, true) != DRS_OK || tensor_map_for(p, b, &tm, true) != DRS_OK)) return false;
         const long long l0 = p->launches;
         if (cudaStreamBeginCapture(p->cap_stream, cudaStreamCaptureModeThreadLocal) != cudaSuccess) {
             cudaGetLastError(); p->use_graph = false; return false;
         }
-        const int rc = enqueue_run(p, a, b, n, p->cap_stream);
+        const int rc = enqueue(p->cap_stream);
         cudaGraph_t g = nullptr;
         const cudaError_t ce = cudaStreamEndCapture(p->cap_stream, &g);
         const int kernels = (int)(p->launches - l0);
@@ -930,28 +937,28 @@ static bool run_graph(drs_plan* p, void* a, void* b, int n, cudaStream_t stream)
     return true;
 }
 
+// Sweeps of a run of `iterations` timesteps: the ping-pong loop always runs whole pairs, so A ends with the result.
+static int sweeps_for(const drs_plan* p, int iterations) {
+    int n = 0;
+    for (int t = 0; t < iterations; t += 2 * p->spec.step) n += 2;
+    return n;
+}
+
 static int run_schedule(drs_plan* p, void* a, void* b, int iterations, void* stream, int* sweeps, bool gold) {
     if (!p || !a || !b) return fail(DRS_E_ARG, "null argument");
     int rc = ensure_loaded(p);
     if (rc != DRS_OK) return rc;
-    int n = 0;
-    if (!gold && p->use_graph && p->spec.tma_ok && p->spec.sub_launches <= 1 && a != b) {
-        for (int t = 0; t < iterations; t += 2 * p->spec.step) n += 2;
-        if (n >= 2 && run_graph(p, a, b, n, (cudaStream_t)stream)) {
-            if (sweeps) *sweeps = n;
-            return DRS_OK;
-        }
-        n = 0;
-    }
-    for (int t = 0; t < iterations; t += 2 * p->spec.step) n += 2;
+    const int n = sweeps_for(p, iterations);
     if (gold) {
         for (int s = 0; s < n; ++s) {
             rc = (s & 1) ? launch_gold(p, b, a, (cudaStream_t)stream) : launch_gold(p, a, b, (cudaStream_t)stream);
             if (rc != DRS_OK) return rc;
         }
     } else {
-        rc = enqueue_run(p, a, b, n, (cudaStream_t)stream);
-        if (rc != DRS_OK) return rc;
+        const bool graph = p->spec.tma_ok && p->spec.sub_launches <= 1 && a != b && n >= 2;
+        auto enqueue = [&](cudaStream_t st) { return enqueue_run(p, a, b, n, st); };
+        if (!(graph && run_graph(p, a, b, n, false, (cudaStream_t)stream, enqueue)) && (rc = enqueue((cudaStream_t)stream)) != DRS_OK)
+            return rc;
     }
     if (sweeps) *sweeps = n;
     return DRS_OK;
@@ -959,8 +966,7 @@ static int run_schedule(drs_plan* p, void* a, void* b, int iterations, void* str
 
 int drs_plan_pair_split(const drs_plan* p, int iterations, int* pairs, int* singles) {
     if (!p) return fail(DRS_E_ARG, "null plan");
-    int n = 0;
-    for (int t = 0; t < iterations; t += 2 * p->spec.step) n += 2;
+    const int n = sweeps_for(p, iterations);
     int np = 0, ns = n;
     if (p->pair) drs::pair_split(n, np, ns);
     if (pairs) *pairs = np;
@@ -1011,18 +1017,20 @@ static long long host_block_units(const drs_plan* p, int sweeps, bool allow_slab
 
 // The emitted main()'s data path (H2D, the ping-pong schedule, D2H) in the time-skewed block order of
 // core/host_schedule.hpp: uploads on one stream, sweeps on a second, downloads on a third, chained
-// by events -- the wall time tends to max(H2D, sweeps, D2H) instead of their sum.
-static int run_host_streamed(drs_plan* p, void* h_a, int n, long long S, size_t bytes, float* device_ms) {
-    const long long slow = p->local_slow();
-    const size_t unit = bytes / (size_t)slow;
-    const drs::HostSchedule hs = drs::plan_host_schedule(slow, p->spec.halo, S, n);
-    const int B = hs.blocks();
+// by events -- the wall time tends to max(H2D, sweeps, D2H) instead of their sum.  Odd sweeps run
+// dA -> dB, even ones dB -> dA; local plane i is host[i - h0].  clear_b: clear dB before the first sweep.
+// Face steps (slab runs) use the flag values flag_base + 1 ...: launches that touch a face are bracketed by
+// the flag kernels, and the upload that brings a face's level-0 planes is followed by a peer copy of them into
+// the neighbour's ghosts.  `what` prefixes the message of a CUDA error found at the end.
+static int run_blocks(drs_plan* p, const std::vector<drs::HostStep>& steps, char* dA, char* dB, char* host, long long h0,
+                      bool clear_b, long long flag_base, const char* what, float* device_ms) {
+    const long long H = p->spec.halo, local = p->local_slow(), org = p->lo - H;
+    const size_t unit = (size_t)(p->spec.dim == 3 ? p->st.M * p->st.N : p->st.N) * p->spec.esize();
     for (cudaStream_t* st : {&p->hs_up, &p->hs_run, &p->hs_dn})
         if (!*st && cudaStreamCreateWithFlags(st, cudaStreamNonBlocking) != cudaSuccess)
             return fail(DRS_E_CUDA, "cudaStreamCreate failed");
-    char* dA = (char*)p->h_dev[0];
-    char* dB = (char*)p->h_dev[1];
-    char* hA = (char*)h_a;
+    int B = 0;
+    for (const drs::HostStep& st : steps) B = std::max(B, st.block + 1);
     std::vector<cudaEvent_t> up(B), done(B);
     cudaEvent_t e0, e1, fin;
     cudaEventCreate(&e0); cudaEventCreate(&e1);
@@ -1034,28 +1042,48 @@ static int run_host_streamed(drs_plan* p, void* h_a, int n, long long S, size_t 
     cudaEventRecord(e0, 0);
     for (cudaStream_t st : {p->hs_up, p->hs_run, p->hs_dn}) cudaStreamWaitEvent(st, e0, 0);
     // every upload is queued first: the copy engine runs ahead of the sweeps as far as it can
-    for (const drs::HostStep& st : hs.steps) {
-        if (st.kind != drs::HostStep::UPLOAD) continue;
-        cudaMemcpyAsync(dA + st.lo * unit, hA + st.lo * unit, (size_t)(st.hi - st.lo) * unit, cudaMemcpyHostToDevice, p->hs_up);
+    int rc = DRS_OK;
+    for (const drs::HostStep& st : steps) {
+        if (st.kind != drs::HostStep::UPLOAD || rc != DRS_OK) continue;
+        cudaMemcpyAsync(dA + st.lo * unit, host + (st.lo - h0) * unit, (size_t)(st.hi - st.lo) * unit, cudaMemcpyHostToDevice, p->hs_up);
+        if ((st.faces & drs::INIT_LOWER) && p->lower_bases[0]) {
+            // my planes [H, 2H) are the lower neighbour's upper ghost: same plane shift as the kernel's push
+            const long long shift = org - (p->lower_lo - H);
+            cudaMemcpyAsync((char*)p->lower_bases[0] + (H + shift) * unit, dA + H * unit, (size_t)H * unit, cudaMemcpyDefault, p->hs_up);
+            rc = launch_signal(p, p->hs_up, p->lower_flag, nullptr, flag_base + 1);
+        }
+        if ((st.faces & drs::INIT_UPPER) && p->upper_bases[0] && rc == DRS_OK) {
+            const long long shift = org - (p->upper_lo - H);
+            cudaMemcpyAsync((char*)p->upper_bases[0] + (local - 2 * H + shift) * unit, dA + (local - 2 * H) * unit, (size_t)H * unit,
+                            cudaMemcpyDefault, p->hs_up);
+            rc = launch_signal(p, p->hs_up, nullptr, p->upper_flag, flag_base + 1);
+        }
         cudaEventRecord(up[st.block], p->hs_up);
     }
     // the reference's h_out is all zeros (getZero2DArray); only its frozen ring is ever read before
     // it is written, and no sweep writes the ring, so one clear serves every later call
-    if (!p->h_dev_b_ring_zero) cudaMemsetAsync(dB, 0, bytes, p->hs_run);
-    p->h_dev_b_ring_zero = true;
-    int rc = DRS_OK;
-    for (const drs::HostStep& st : hs.steps) {
+    if (clear_b) {
+        cudaMemsetAsync(dB, 0, unit * (size_t)local, p->hs_run);
+        p->h_dev_b_ring_zero = true;
+    }
+    for (const drs::HostStep& st : steps) {
         if (rc != DRS_OK) break;
         if (st.kind == drs::HostStep::UPLOAD) {
             cudaStreamWaitEvent(p->hs_run, up[st.block], 0);
         } else if (st.kind == drs::HostStep::SWEEP) {
+            if (st.faces & (drs::WAIT_LOWER | drs::WAIT_UPPER))
+                rc = launch_wait(p, p->hs_run, p->my_flags, (st.faces & drs::WAIT_LOWER) != 0, (st.faces & drs::WAIT_UPPER) != 0,
+                                 flag_base + st.sweep);
             const SlowRange r = {st.lo, st.hi};
-            rc = (st.sweep & 1) ? launch_one(p, dA, dB, p->hs_run, -1, &r) : launch_one(p, dB, dA, p->hs_run, -1, &r);
+            if (rc == DRS_OK) rc = (st.sweep & 1) ? launch_one(p, dA, dB, p->hs_run, -1, &r) : launch_one(p, dB, dA, p->hs_run, -1, &r);
+            if (rc == DRS_OK && (st.faces & (drs::SIGNAL_LOWER | drs::SIGNAL_UPPER)))
+                rc = launch_signal(p, p->hs_run, (st.faces & drs::SIGNAL_LOWER) ? p->lower_flag : nullptr,
+                                   (st.faces & drs::SIGNAL_UPPER) ? p->upper_flag : nullptr, flag_base + st.sweep + 1);
         } else {
             cudaEventRecord(done[st.block], p->hs_run);
             cudaStreamWaitEvent(p->hs_dn, done[st.block], 0);
             if (st.hi > st.lo)
-                cudaMemcpyAsync(hA + st.lo * unit, dA + st.lo * unit, (size_t)(st.hi - st.lo) * unit, cudaMemcpyDeviceToHost, p->hs_dn);
+                cudaMemcpyAsync(host + (st.lo - h0) * unit, dA + st.lo * unit, (size_t)(st.hi - st.lo) * unit, cudaMemcpyDeviceToHost, p->hs_dn);
         }
     }
     cudaEventRecord(fin, p->hs_dn);
@@ -1069,27 +1097,50 @@ static int run_host_streamed(drs_plan* p, void* h_a, int n, long long S, size_t 
     for (int b = 0; b < B; ++b) { cudaEventDestroy(up[b]); cudaEventDestroy(done[b]); }
     if (device_ms) *device_ms = ms;
     const cudaError_t ce = cudaGetLastError();
-    if (rc == DRS_OK && rc2 == DRS_OK && ce != cudaSuccess)
-        return fail(DRS_E_CUDA, std::string("streamed host run: ") + cudaGetErrorString(ce));
+    if (rc == DRS_OK && rc2 == DRS_OK && ce != cudaSuccess) return fail(DRS_E_CUDA, std::string(what) + cudaGetErrorString(ce));
     return rc != DRS_OK ? rc : rc2;
+}
+
+// Step list of a streamed drs_run_host; empty when the plain copy-sweep-copy sequence applies.
+static std::vector<drs::HostStep> host_steps(const drs_plan* p, int n) {
+    const long long S = host_block_units(p, n);
+    if (S <= 0) return {};
+    return drs::plan_block_schedule(drs::whole_grid(p->local_slow(), p->spec.halo), p->spec.halo, S, n);
+}
+
+// Step list of this rank for a slab host run; empty when the plain sequence applies.
+static std::vector<drs::HostStep> slab_steps(const drs_plan* p, int n, bool up_skew) {
+    const long long S = host_block_units(p, n, true);
+    if (S <= 0) return {};
+    const long long H = p->spec.halo, org = p->lo - H;
+    drs::SlabSide g;
+    g.local = p->local_slow();
+    g.own_lo = H; g.own_hi = g.local - H;
+    g.out_lo = std::max<long long>(p->lo, H) - org;
+    g.out_hi = std::min<long long>(p->hi, p->g_slow - H) - org;
+    g.has_lower = p->lo > 0; g.has_upper = p->hi < p->g_slow;
+    g.up_skew = up_skew;
+    if (g.out_hi - g.out_lo < 2 * H || g.own_hi - g.own_lo <= S) return {};
+    return drs::plan_block_schedule(g, H, S, n);
+}
+
+// A step list as records of `width` fields: kind, block, sweep, lo, hi (, faces).  Returns the number of steps.
+static int step_records(const std::vector<drs::HostStep>& steps, long long* records, int width, int capacity) {
+    if (records) {
+        if (capacity < (int)steps.size()) return fail(DRS_E_ARG, "buffer too small");
+        for (size_t i = 0; i < steps.size(); ++i) {
+            const drs::HostStep& st = steps[i];
+            long long* r = records + width * i;
+            r[0] = st.kind; r[1] = st.block; r[2] = st.sweep; r[3] = st.lo; r[4] = st.hi;
+            if (width > 5) r[5] = st.faces;
+        }
+    }
+    return (int)steps.size();
 }
 
 int drs_plan_host_schedule(const drs_plan* p, int iterations, long long* records5, int capacity) {
     if (!p) return fail(DRS_E_ARG, "null plan");
-    int n = 0;
-    for (int t = 0; t < iterations; t += 2 * p->spec.step) n += 2;
-    const long long S = host_block_units(p, n);
-    if (S <= 0) return 0;
-    const drs::HostSchedule hs = drs::plan_host_schedule(p->local_slow(), p->spec.halo, S, n);
-    if (records5) {
-        if (capacity < (int)hs.steps.size()) return fail(DRS_E_ARG, "buffer too small");
-        for (size_t i = 0; i < hs.steps.size(); ++i) {
-            const drs::HostStep& st = hs.steps[i];
-            long long* r = records5 + 5 * i;
-            r[0] = st.kind; r[1] = st.block; r[2] = st.sweep; r[3] = st.lo; r[4] = st.hi;
-        }
-    }
-    return (int)hs.steps.size();
+    return step_records(host_steps(p, sweeps_for(p, iterations)), records5, 5, capacity);
 }
 
 int drs_run_host(drs_plan* p, void* h_a, void* h_b, int iterations, float* device_ms) {
@@ -1100,10 +1151,10 @@ int drs_run_host(drs_plan* p, void* h_a, void* h_b, int iterations, float* devic
     for (int i = 0; i < 2; ++i)
         if (!p->h_dev[i] && cudaMalloc(&p->h_dev[i], bytes) != cudaSuccess)
             return fail(DRS_E_CUDA, "cudaMalloc of the sweep buffers failed");
-    int n = 0;
-    for (int t = 0; t < iterations; t += 2 * p->spec.step) n += 2;
-    const long long S = h_b ? 0 : host_block_units(p, n);
-    if (S > 0) return run_host_streamed(p, h_a, n, S, bytes, device_ms);
+    const std::vector<drs::HostStep> steps = h_b ? std::vector<drs::HostStep>() : host_steps(p, sweeps_for(p, iterations));
+    if (!steps.empty())
+        return run_blocks(p, steps, (char*)p->h_dev[0], (char*)p->h_dev[1], (char*)h_a, 0, !p->h_dev_b_ring_zero, 0,
+                          "streamed host run: ", device_ms);
     cudaEvent_t e0, e1;
     cudaEventCreate(&e0); cudaEventCreate(&e1);
     cudaEventRecord(e0, 0);
@@ -1122,38 +1173,10 @@ int drs_run_host(drs_plan* p, void* h_a, void* h_b, int iterations, float* devic
     return rc != DRS_OK ? rc : rc2;
 }
 
-// Step list of this rank for a slab host run; empty when the plain sequence applies.
-static std::vector<drs::SlabStep> slab_steps(const drs_plan* p, int n, bool up_skew) {
-    const long long S = host_block_units(p, n, true);
-    if (S <= 0) return {};
-    const long long H = p->spec.halo, org = p->lo - H;
-    drs::SlabSide g;
-    g.local = p->local_slow();
-    g.own_lo = H; g.own_hi = g.local - H;
-    g.out_lo = std::max<long long>(p->lo, H) - org;
-    g.out_hi = std::min<long long>(p->hi, p->g_slow - H) - org;
-    g.has_lower = p->lo > 0; g.has_upper = p->hi < p->g_slow;
-    g.up_skew = up_skew;
-    if (g.out_hi - g.out_lo < 2 * H || g.own_hi - g.own_lo <= S) return {};
-    return drs::plan_slab_schedule(g, H, S, n);
-}
-
 int drs_plan_slab_schedule(const drs_plan* p, int iterations, int up_skew, long long* records6, int capacity) {
     if (!p) return fail(DRS_E_ARG, "null plan");
     if (!p->slab) return fail(DRS_E_ARG, "call drs_plan_set_slab first");
-    int n = 0;
-    for (int t = 0; t < iterations; t += 2 * p->spec.step) n += 2;
-    const std::vector<drs::SlabStep> steps = slab_steps(p, n, up_skew != 0);
-    if (steps.empty()) return 0;
-    if (records6) {
-        if (capacity < (int)steps.size()) return fail(DRS_E_ARG, "buffer too small");
-        for (size_t i = 0; i < steps.size(); ++i) {
-            const drs::SlabStep& st = steps[i];
-            long long* r = records6 + 6 * i;
-            r[0] = st.kind; r[1] = st.block; r[2] = st.sweep; r[3] = st.lo; r[4] = st.hi; r[5] = st.faces;
-        }
-    }
-    return (int)steps.size();
+    return step_records(slab_steps(p, sweeps_for(p, iterations), up_skew != 0), records6, 6, capacity);
 }
 
 int drs_plan_set_graph(drs_plan* p, int enable) {
@@ -1231,22 +1254,14 @@ int drs_signal_peers(drs_plan* p, void* lower_flag, void* upper_flag, long long 
     if (!p) return fail(DRS_E_ARG, "null plan");
     int rc = ensure_loaded(p);
     if (rc != DRS_OK) return rc;
-    void* args[] = {&lower_flag, &upper_flag, &value};
-    CUresult r = driver().LaunchKernel(p->f_signal, 1, 1, 1, 32, 1, 1, 0, (CUstream)stream, args, nullptr);
-    if (r != CUDA_SUCCESS) return fail(DRS_E_CUDA, "launch signal_: " + cu_err(r));
-    p->launches++;
-    return DRS_OK;
+    return launch_signal(p, (cudaStream_t)stream, lower_flag, upper_flag, value);
 }
 
 int drs_wait_flags(drs_plan* p, const void* my_flags, int wait_lower, int wait_upper, long long value, void* stream) {
     if (!p || !my_flags) return fail(DRS_E_ARG, "null argument");
     int rc = ensure_loaded(p);
     if (rc != DRS_OK) return rc;
-    void* args[] = {(void*)&my_flags, &wait_lower, &wait_upper, &value, &p->d_fault};
-    CUresult r = driver().LaunchKernel(p->f_wait, 1, 1, 1, 32, 1, 1, 0, (CUstream)stream, args, nullptr);
-    if (r != CUDA_SUCCESS) return fail(DRS_E_CUDA, "launch wait_: " + cu_err(r));
-    p->launches++;
-    return DRS_OK;
+    return launch_wait(p, (cudaStream_t)stream, my_flags, wait_lower, wait_upper, value);
 }
 
 int drs_plan_set_flags(drs_plan* p, const void* my_flags, void* lower_flag, void* upper_flag) {
@@ -1276,8 +1291,7 @@ int drs_run_slab(drs_plan* p, int iterations, void* stream_, int* sweeps) {
         if (cudaMalloc(&p->d_sync, 16) != cudaSuccess) return fail(DRS_E_CUDA, "cudaMalloc(slab sync words)");
         cudaMemset(p->d_sync, 0, 16);
     }
-    int n = 0;
-    for (int t = 0; t < iterations; t += 2 * p->spec.step) n += 2;
+    const int n = sweeps_for(p, iterations);
     if (sweeps) *sweeps = n;
     if (n == 0) return DRS_OK;
     // flag value of this call's sweep 0, in stream order (no kernel)
@@ -1296,159 +1310,29 @@ int drs_run_slab(drs_plan* p, int iterations, void* stream_, int* sweeps) {
             r = (s & 1) ? launch_one(p, b, a, st, -1, nullptr, s) : launch_one(p, a, b, st, -1, nullptr, s);
         return r;
     };
-    cudaStreamCaptureStatus cs = cudaStreamCaptureStatusNone;
-    const bool capturing = cudaStreamIsCapturing(stream, &cs) != cudaSuccess || cs != cudaStreamCaptureStatusNone;
-    cudaGetLastError();
-    bool done = false;
-    if (p->use_graph && !capturing) {
-        auto it = p->slab_graphs.find(n);
-        if (it == p->slab_graphs.end()) {
-            CUtensorMap* tm = nullptr;
-            if ((rc = tensor_map_for(p, a, &tm)) != DRS_OK || (rc = tensor_map_for(p, b, &tm)) != DRS_OK) return rc;
-            if (!p->cap_stream && cudaStreamCreateWithFlags(&p->cap_stream, cudaStreamNonBlocking) != cudaSuccess) {
-                cudaGetLastError(); p->use_graph = false;
-            } else if (cudaStreamBeginCapture(p->cap_stream, cudaStreamCaptureModeThreadLocal) != cudaSuccess) {
-                cudaGetLastError(); p->use_graph = false;
-            } else {
-                const long long l0 = p->launches;
-                rc = enqueue(p->cap_stream);
-                cudaGraph_t g = nullptr;
-                const cudaError_t ce = cudaStreamEndCapture(p->cap_stream, &g);
-                const int kernels = (int)(p->launches - l0);
-                p->launches = l0;
-                cudaGraphExec_t exec = nullptr;
-                if (rc != DRS_OK || ce != cudaSuccess || !g || cudaGraphInstantiate(&exec, g, 0) != cudaSuccess) {
-                    if (g) cudaGraphDestroy(g);
-                    cudaGetLastError(); p->use_graph = false;
-                    if (rc != DRS_OK) return rc;
-                } else {
-                    cudaGraphDestroy(g);
-                    if (p->slab_graphs.size() >= 8) {
-                        for (auto& x : p->slab_graphs) cudaGraphExecDestroy(x.second.exec);
-                        p->slab_graphs.clear();
-                    }
-                    it = p->slab_graphs.emplace(n, drs_plan::RunGraph{exec, kernels}).first;
-                }
-            }
-        }
-        if (p->use_graph && it != p->slab_graphs.end()) {
-            if (cudaGraphLaunch(it->second.exec, stream) == cudaSuccess) { p->launches += it->second.kernels; done = true; }
-            else { cudaGetLastError(); p->use_graph = false; }
-        }
-    }
-    if (!done && (rc = enqueue(stream)) != DRS_OK) return rc;
+    if (!run_graph(p, a, b, n, true, stream, enqueue) && (rc = enqueue(stream)) != DRS_OK) return rc;
     p->slab_seq += n;
     return DRS_OK;
 }
 
 // Executor of drs_plan_slab_schedule (validated on 2, 4 and 8 GPUs: bit-exact against the single-GPU run,
-// tools/slab_check.py and bench.py's in-run parity).  One rank's share of a slab-decomposed host-buffer run: h_own
-// holds the rank's own planes; uploads, sweeps and downloads run on three streams chained by events as in
-// run_host_streamed; launches that touch a face are bracketed by the slab flag kernels, and the upload that brings a
-// face's level-0 planes is followed by a peer copy of them into the neighbour's ghosts.  Flags are monotone: this call
-// uses the values slab_seq + 1 ... slab_seq + sweeps + 1 and leaves slab_seq at the largest one; the caller separates
-// calls by a barrier.
+// tools/slab_check.py and bench.py's in-run parity): one rank's share of a slab-decomposed host-buffer run, on
+// the block executor of drs_run_host.  h_own holds the rank's own planes, local planes [H, local - H).  Flags are
+// monotone: this call uses the values slab_seq + 1 ... slab_seq + sweeps + 1 and leaves slab_seq at the largest
+// one; the caller separates calls by a barrier.
 int drs_run_host_slab(drs_plan* p, void* h_own, int iterations, int up_skew, float* device_ms) {
     if (!p || !h_own) return fail(DRS_E_ARG, "null argument");
     if (!p->slab || !p->my_bases[0] || !p->my_bases[1]) return fail(DRS_E_ARG, "call drs_plan_set_slab and drs_plan_set_peers first");
     if (!p->my_flags) return fail(DRS_E_ARG, "call drs_plan_set_flags first");
     int rc = ensure_loaded(p);
     if (rc != DRS_OK) return rc;
-    const void* my_flags = p->my_flags;
-    void* lower_flag = p->lower_flag;
-    void* upper_flag = p->upper_flag;
-    const long long flag_base = p->slab_seq;
-    int n = 0;
-    for (int t = 0; t < iterations; t += 2 * p->spec.step) n += 2;
-    const std::vector<drs::SlabStep> steps = slab_steps(p, n, up_skew != 0);
+    const int n = sweeps_for(p, iterations);
+    const std::vector<drs::HostStep> steps = slab_steps(p, n, up_skew != 0);
     if (steps.empty()) return fail(DRS_E_ARG, "no streamed schedule for this slab (too thin, or switched off): use the plain sequence");
-    const long long H = p->spec.halo, local = p->local_slow(), org = p->lo - H;
-    const size_t unit = (size_t)(p->spec.dim == 3 ? p->st.M * p->st.N : p->st.N) * p->spec.esize();
-    for (cudaStream_t* st : {&p->hs_up, &p->hs_run, &p->hs_dn})
-        if (!*st && cudaStreamCreateWithFlags(st, cudaStreamNonBlocking) != cudaSuccess)
-            return fail(DRS_E_CUDA, "cudaStreamCreate failed");
-    char* dA = (char*)p->my_bases[0];
-    char* dB = (char*)p->my_bases[1];
-    char* hA = (char*)h_own;
-    int B = 0;
-    for (const drs::SlabStep& st : steps) B = std::max(B, st.block + 1);
-    std::vector<cudaEvent_t> up(B), done(B);
-    cudaEvent_t e0, e1, fin;
-    cudaEventCreate(&e0); cudaEventCreate(&e1);
-    cudaEventCreateWithFlags(&fin, cudaEventDisableTiming);
-    for (int b = 0; b < B; ++b) {
-        cudaEventCreateWithFlags(&up[b], cudaEventDisableTiming);
-        cudaEventCreateWithFlags(&done[b], cudaEventDisableTiming);
-    }
-    auto signal = [&](cudaStream_t st, bool lo, bool hi, long long value) -> int {
-        void* lf = lo ? lower_flag : nullptr;
-        void* uf = hi ? upper_flag : nullptr;
-        void* args[] = {&lf, &uf, &value};
-        CUresult r = driver().LaunchKernel(p->f_signal, 1, 1, 1, 32, 1, 1, 0, (CUstream)st, args, nullptr);
-        if (r != CUDA_SUCCESS) return fail(DRS_E_CUDA, "launch signal_: " + cu_err(r));
-        p->launches++;
-        return DRS_OK;
-    };
-    cudaEventRecord(e0, 0);
-    for (cudaStream_t st : {p->hs_up, p->hs_run, p->hs_dn}) cudaStreamWaitEvent(st, e0, 0);
-    // uploads (own planes: host index = local index - H), each followed by the level-0 ghost push it enables
-    for (const drs::SlabStep& st : steps) {
-        if (st.kind != drs::HostStep::UPLOAD || rc != DRS_OK) continue;
-        cudaMemcpyAsync(dA + st.lo * unit, hA + (st.lo - H) * unit, (size_t)(st.hi - st.lo) * unit, cudaMemcpyHostToDevice, p->hs_up);
-        if ((st.faces & drs::INIT_LOWER) && p->lower_bases[0]) {
-            // my planes [H, 2H) are the lower neighbour's upper ghost: same plane shift as the kernel's push
-            const long long shift = org - (p->lower_lo - H);
-            cudaMemcpyAsync((char*)p->lower_bases[0] + (H + shift) * unit, dA + H * unit, (size_t)H * unit, cudaMemcpyDefault, p->hs_up);
-            rc = signal(p->hs_up, true, false, flag_base + 1);
-        }
-        if ((st.faces & drs::INIT_UPPER) && p->upper_bases[0] && rc == DRS_OK) {
-            const long long shift = org - (p->upper_lo - H);
-            cudaMemcpyAsync((char*)p->upper_bases[0] + (local - 2 * H + shift) * unit, dA + (local - 2 * H) * unit, (size_t)H * unit,
-                            cudaMemcpyDefault, p->hs_up);
-            rc = signal(p->hs_up, false, true, flag_base + 1);
-        }
-        cudaEventRecord(up[st.block], p->hs_up);
-    }
-    for (const drs::SlabStep& st : steps) {
-        if (rc != DRS_OK) break;
-        if (st.kind == drs::HostStep::UPLOAD) {
-            cudaStreamWaitEvent(p->hs_run, up[st.block], 0);
-        } else if (st.kind == drs::HostStep::SWEEP) {
-            const bool wl = st.faces & drs::WAIT_LOWER, wu = st.faces & drs::WAIT_UPPER;
-            if (wl || wu) {
-                int a = wl, b = wu;
-                long long value = flag_base + st.sweep;
-                void* args[] = {(void*)&my_flags, &a, &b, &value, &p->d_fault};
-                CUresult r = driver().LaunchKernel(p->f_wait, 1, 1, 1, 32, 1, 1, 0, (CUstream)p->hs_run, args, nullptr);
-                if (r != CUDA_SUCCESS) { rc = fail(DRS_E_CUDA, "launch wait_: " + cu_err(r)); break; }
-                p->launches++;
-            }
-            const SlowRange r = {st.lo, st.hi};
-            rc = (st.sweep & 1) ? launch_one(p, dA, dB, p->hs_run, -1, &r) : launch_one(p, dB, dA, p->hs_run, -1, &r);
-            if (rc == DRS_OK && (st.faces & (drs::SIGNAL_LOWER | drs::SIGNAL_UPPER)))
-                rc = signal(p->hs_run, st.faces & drs::SIGNAL_LOWER, st.faces & drs::SIGNAL_UPPER, flag_base + st.sweep + 1);
-        } else {
-            cudaEventRecord(done[st.block], p->hs_run);
-            cudaStreamWaitEvent(p->hs_dn, done[st.block], 0);
-            if (st.hi > st.lo)
-                cudaMemcpyAsync(hA + (st.lo - H) * unit, dA + st.lo * unit, (size_t)(st.hi - st.lo) * unit, cudaMemcpyDeviceToHost, p->hs_dn);
-        }
-    }
-    cudaEventRecord(fin, p->hs_dn);
-    cudaStreamWaitEvent(0, fin, 0);
-    cudaEventRecord(e1, 0);
-    int rc2 = drs_plan_sync_check(p, nullptr);
-    for (cudaStream_t st : {p->hs_up, p->hs_run, p->hs_dn}) cudaStreamSynchronize(st);
-    float ms = 0.f;
-    cudaEventElapsedTime(&ms, e0, e1);
-    cudaEventDestroy(e0); cudaEventDestroy(e1); cudaEventDestroy(fin);
-    for (int b = 0; b < B; ++b) { cudaEventDestroy(up[b]); cudaEventDestroy(done[b]); }
-    if (device_ms) *device_ms = ms;
-    const cudaError_t ce = cudaGetLastError();
-    if (rc == DRS_OK && rc2 == DRS_OK && ce != cudaSuccess)
-        return fail(DRS_E_CUDA, std::string("streamed slab run: ") + cudaGetErrorString(ce));
-    if (rc == DRS_OK && rc2 == DRS_OK) p->slab_seq = flag_base + n + 1;    // the largest flag value this call wrote
-    return rc != DRS_OK ? rc : rc2;
+    rc = run_blocks(p, steps, (char*)p->my_bases[0], (char*)p->my_bases[1], (char*)h_own, p->spec.halo, false, p->slab_seq,
+                    "streamed slab run: ", device_ms);
+    if (rc == DRS_OK) p->slab_seq += n + 1;    // the largest flag value this call wrote
+    return rc;
 }
 
 int drs_ipc_export(void* d_ptr, unsigned char handle[64]) {

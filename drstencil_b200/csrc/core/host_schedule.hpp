@@ -1,13 +1,13 @@
-// Time-skewed block schedule of the host-buffer run (drs_run_host): pure host logic, no CUDA.
+// Time-skewed block schedule of the host-buffer runs (drs_run_host, drs_run_host_slab): pure host logic, no CUDA.
 //
 // The emitted main() of the reference copies the grid in, runs the ping-pong loop, copies it out
 // (/root/reference/codegen_2d.hpp:572-583,604-619,647).  This planner orders the same work so that
-// the three phases can overlap.  The grid is cut into blocks along the slow axis; block b runs ALL
-// n sweeps before block b+1 starts, its output range sliding down one halo per sweep:
+// the three phases can overlap.  The planes a device holds along the slow axis are cut into blocks;
+// block b runs ALL n sweeps before block b+1 starts, its output range sliding down one halo per sweep:
 //
-//     sweep s (1-based) of block b produces  [edge[b] - s*H, edge[b+1] - s*H)  clamped to [H, slow-H)
+//     sweep s (1-based) of block b produces  [edge[b] - s*H, edge[b+1] - s*H)  clamped to [out_lo, out_hi)
 //
-// (the first block is pinned to H at the bottom, the last one to slow-H at the top).  With every
+// (the first block is pinned to out_lo at the bottom, the last one to out_hi at the top).  With every
 // block at least 2*H thick this order honours each dependency of the plain schedule in place, on the
 // same two buffers:
 //   * what sweep s reads -- [edge[b] - s*H - H, edge[b+1] - s*H + H) of level s-1 -- was produced by
@@ -17,73 +17,15 @@
 // A sweep is a pure function of its input array, so the result equals the plain schedule bit for bit.
 // Block b needs nothing above edge[b+1] on the device, and its final planes never change afterwards:
 // the upload of later blocks and the download of earlier ones can run under the sweeps.
-// tests/test_host_schedule.py replays the step list on the CPU (not-yet-uploaded planes poisoned)
-// for both extreme interleavings of the copies and compares with the plain schedule.
-#pragma once
-#include <algorithm>
-#include <vector>
-
-namespace drs {
-
-struct HostStep {
-    enum Kind { UPLOAD = 0, SWEEP = 1, DOWNLOAD = 2 };
-    int kind, block, sweep;     // sweep: 1..n for SWEEP (odd: A -> B, even: B -> A), else 0
-    long long lo, hi;           // slow-axis range [lo, hi): planes copied / output planes of the launch
-};
-
-struct HostSchedule {
-    std::vector<long long> edge;     // blocks + 1 increasing values, edge[0] = 0, edge[blocks] = slow
-    std::vector<HostStep> steps;     // per block: UPLOAD, its non-empty SWEEPs in order, DOWNLOAD
-    int blocks() const { return (int)edge.size() - 1; }
-};
-
-// slow = slow-axis extent, H = halo of one sweep, S = nominal block thickness (>= 2*H), n = sweeps (even).
-// The first and the last block are thin (a quarter of S, at least 2*H): the first one's upload and the
-// last one's download (its thickness + n*H planes) are the only copies that nothing overlaps.
-inline HostSchedule plan_host_schedule(long long slow, long long H, long long S, int n) {
-    HostSchedule hs;
-    S = std::max<long long>(S, std::max<long long>(2 * H, 1));
-    const long long thin = std::max<long long>(2 * H, std::max<long long>(S / 4, 1));
-    hs.edge.push_back(0);
-    long long at = std::min(thin, slow);
-    while (at < slow) {
-        hs.edge.push_back(at);
-        at += (slow - at - thin > S) ? S : ((slow - at > 2 * thin) ? slow - at - thin : slow - at);
-    }
-    hs.edge.push_back(slow);
-    // every block must be at least 2*H thick (see above): a thinner remainder joins its predecessor
-    while (hs.edge.size() > 2 && hs.edge.back() - hs.edge[hs.edge.size() - 2] < 2 * H) hs.edge.erase(hs.edge.end() - 2);
-    const int B = hs.blocks();
-    auto cut = [&](int b, int s) -> long long {   // first output plane of block b at sweep s
-        if (b <= 0) return H;
-        if (b >= B) return slow - H;
-        return std::min(std::max(hs.edge[b] - (long long)s * H, H), slow - H);
-    };
-    for (int b = 0; b < B; ++b) {
-        hs.steps.push_back({HostStep::UPLOAD, b, 0, hs.edge[b], hs.edge[b + 1]});
-        for (int s = 1; s <= n; ++s) {
-            const long long lo = cut(b, s), hi = cut(b + 1, s);
-            if (hi > lo) hs.steps.push_back({HostStep::SWEEP, b, s, lo, hi});
-        }
-        const long long lo = b == 0 ? 0 : cut(b, n), hi = b == B - 1 ? slow : cut(b + 1, n);
-        hs.steps.push_back({HostStep::DOWNLOAD, b, 0, lo, std::max(lo, hi)});
-    }
-    return hs;
-}
-
-// ---------------------------------------------------------------------------------------------
-// The same block order for ONE RANK of a slab-decomposed run (executor: drs_run_host_slab;
-// tests/test_slab_schedule.py runs the step lists of all ranks against each other on the CPU, with
-// random interleavings, ghost planes and flags).
 //
-// Local plane indices: the rank's array holds `local` planes, of which [own_lo, own_hi) are its own
-// (host slab, uploaded / downloaded) and [out_lo, out_hi) are swept (out_lo > own_lo only where the
-// global frozen ring lies inside the slab); the rest are ghost planes a neighbour fills.
-//
-// A face to a neighbour is fixed in space, so the blocks cannot slide past it: neighbouring ranks
-// skew in OPPOSITE directions (even ranks down, odd ranks up, processing their blocks top-down).
-// Then the two blocks that meet at a face are both processed first, or both processed last, and run
-// their sweeps in lockstep through the existing step flags:
+// A single-device run (whole_grid) owns every plane and has no neighbours.  One rank of a slab-decomposed
+// run may have a face to a neighbour below and one above.  Its array holds `local` planes, of which
+// [own_lo, own_hi) are its own (host slab, uploaded / downloaded) and [out_lo, out_hi) are swept (out_lo >
+// own_lo only where the global frozen ring lies inside the slab); the rest are ghost planes a neighbour fills.
+// A face is fixed in space, so the blocks cannot slide past it: neighbouring ranks skew in OPPOSITE
+// directions (even ranks down, odd ranks up, processing their blocks top-down).  Then the two blocks that
+// meet at a face are both processed first, or both processed last, and run their sweeps in lockstep through
+// the step flags:
 //   wait   before a launch that reads ghost planes of a face: flag of that face >= sweep
 //          (the neighbour has produced -- and pushed -- level sweep-1, and has finished reading what
 //          this launch's own push will overwrite);
@@ -92,20 +34,43 @@ inline HostSchedule plan_host_schedule(long long slow, long long H, long long S,
 //          ghost, flag := 1.
 // When a block's range has slid off a face the next block inherits the lockstep at the same sweep on
 // both sides (mirror symmetry), so no rank ever waits for a level its neighbour produces later than
-// it needs it itself.
+// it needs it itself.  Without neighbours every step's `faces` is 0.
+//
+// tests/test_host_schedule.py replays the single-device step list on the CPU (not-yet-uploaded planes
+// poisoned) for both extreme interleavings of the copies and compares with the plain schedule;
+// tests/test_slab_schedule.py runs the step lists of all ranks against each other, with random
+// interleavings, ghost planes and flags.
+#pragma once
+#include <algorithm>
+#include <vector>
+
+namespace drs {
+
+enum HostFace {
+    WAIT_LOWER = 1, WAIT_UPPER = 2, SIGNAL_LOWER = 4, SIGNAL_UPPER = 8, INIT_LOWER = 16, INIT_UPPER = 32
+};
+
+struct HostStep {
+    enum Kind { UPLOAD = 0, SWEEP = 1, DOWNLOAD = 2 };
+    int kind, block, sweep;     // sweep: 1..n for SWEEP (odd: A -> B, even: B -> A), else 0
+    long long lo, hi;           // slow-axis range [lo, hi): planes copied / output planes of the launch
+    int faces;                  // HostFace bits
+};
+
 struct SlabSide {
     long long local, own_lo, own_hi, out_lo, out_hi;
     bool has_lower, has_upper;   // neighbours below / above
     bool up_skew;                // mirror image: blocks processed top-down, ranges slide up
 };
 
-enum HostFace {
-    WAIT_LOWER = 1, WAIT_UPPER = 2, SIGNAL_LOWER = 4, SIGNAL_UPPER = 8, INIT_LOWER = 16, INIT_UPPER = 32
-};
+// A grid of `slow` planes on one device: every plane is owned, the outer H on each side are the frozen ring.
+inline SlabSide whole_grid(long long slow, long long H) { return {slow, 0, slow, H, slow - H, false, false, false}; }
 
-struct SlabStep : HostStep { int faces; };
-
-inline std::vector<SlabStep> plan_slab_schedule(SlabSide g, long long H, long long S, int n) {
+// H = halo of one sweep, S = nominal block thickness (>= 2*H), n = sweeps (even).  Per block: UPLOAD, its
+// non-empty SWEEPs in order, DOWNLOAD.  The first and the last block are thin (a quarter of S, at least 2*H):
+// the first one's upload and the last one's download (its thickness + n*H planes) are the only copies that
+// nothing overlaps.
+inline std::vector<HostStep> plan_block_schedule(SlabSide g, long long H, long long S, int n) {
     const long long L = g.local;
     if (g.up_skew) {            // plan the mirror image, reflect the result
         SlabSide m = g;
@@ -113,8 +78,8 @@ inline std::vector<SlabStep> plan_slab_schedule(SlabSide g, long long H, long lo
         m.own_lo = L - g.own_hi; m.own_hi = L - g.own_lo;
         m.out_lo = L - g.out_hi; m.out_hi = L - g.out_lo;
         m.has_lower = g.has_upper; m.has_upper = g.has_lower;
-        std::vector<SlabStep> r = plan_slab_schedule(m, H, S, n);
-        for (SlabStep& st : r) {
+        std::vector<HostStep> r = plan_block_schedule(m, H, S, n);
+        for (HostStep& st : r) {
             const long long lo = L - st.hi, hi = L - st.lo;
             st.lo = lo; st.hi = hi;
             const int f = st.faces;
@@ -135,23 +100,24 @@ inline std::vector<SlabStep> plan_slab_schedule(SlabSide g, long long H, long lo
         at += (left - thin > S) ? S : ((left > 2 * thin) ? left - thin : left);
     }
     edge.push_back(g.own_hi);
+    // every block must be at least 2*H thick (see above): a thinner remainder joins its predecessor
     while (edge.size() > 2 && edge.back() - edge[edge.size() - 2] < 2 * H) edge.erase(edge.end() - 2);
     const int B = (int)edge.size() - 1;
-    auto cut = [&](int b, int s) -> long long {
+    auto cut = [&](int b, int s) -> long long {   // first output plane of block b at sweep s
         if (b <= 0) return g.out_lo;
         if (b >= B) return g.out_hi;
         return std::min(std::max(edge[b] - (long long)s * H, g.out_lo), g.out_hi);
     };
-    std::vector<SlabStep> steps;
+    std::vector<HostStep> steps;
     for (int b = 0; b < B; ++b) {
-        SlabStep up{};
+        HostStep up{};
         up.kind = HostStep::UPLOAD; up.block = b; up.sweep = 0; up.lo = edge[b]; up.hi = edge[b + 1];
         up.faces = (g.has_lower && b == 0 ? INIT_LOWER : 0) | (g.has_upper && b == B - 1 ? INIT_UPPER : 0);
         steps.push_back(up);
         for (int s = 1; s <= n; ++s) {
             const long long lo = cut(b, s), hi = cut(b + 1, s);
             if (hi <= lo) continue;
-            SlabStep sw{};
+            HostStep sw{};
             sw.kind = HostStep::SWEEP; sw.block = b; sw.sweep = s; sw.lo = lo; sw.hi = hi;
             if (g.has_lower && lo < g.own_lo + H) {
                 sw.faces |= WAIT_LOWER;
@@ -163,7 +129,7 @@ inline std::vector<SlabStep> plan_slab_schedule(SlabSide g, long long H, long lo
             }
             steps.push_back(sw);
         }
-        SlabStep dn{};
+        HostStep dn{};
         dn.kind = HostStep::DOWNLOAD; dn.block = b; dn.sweep = 0;
         dn.lo = b == 0 ? g.own_lo : cut(b, n);
         dn.hi = std::max(dn.lo, b == B - 1 ? g.own_hi : cut(b + 1, n));

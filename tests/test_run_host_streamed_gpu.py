@@ -1,5 +1,5 @@
 """drs_run_host with the copy/sweep/copy phases overlapped by time skewing (capi.cpp:
-run_host_streamed) must return exactly what the plain sequence returns: a sweep is a pure function
+run_blocks) must return exactly what the plain sequence returns: a sweep is a pure function
 of its input array, so any block order that honours the dependencies is bit-identical."""
 import numpy as np
 import pytest

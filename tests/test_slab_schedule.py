@@ -1,4 +1,4 @@
-"""Planner for the slab-decomposed host-buffer run (csrc/core/host_schedule.hpp: plan_slab_schedule,
+"""Planner for the slab-decomposed host-buffer run (csrc/core/host_schedule.hpp: plan_block_schedule,
 reported by drs_plan_slab_schedule) checked on the CPU: the step lists of ALL ranks are executed against
 each other -- the CPU oracle stands in for the sweep kernel, ghost planes are pushed into the neighbour's
 array exactly where the kernel's fused halo push would store them, flags gate the launches as the slab
