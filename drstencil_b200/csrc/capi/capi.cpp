@@ -652,12 +652,16 @@ int launch_wait(drs_plan* p, cudaStream_t stream, const void* flags, int lo, int
     return DRS_OK;
 }
 
+// Whether drs_run runs pair launches on this plan.  Not on a slab: the pair kernel takes its ring from the local
+// array's edges instead of the global faces, and it makes no peer stores.
+bool uses_pairs(const drs_plan* p) { return p->pair && !p->slab; }
+
 // drs_run's n sweeps over (a, b): sweep s writes the interior of bufs[(s+1)%2] from bufs[s%2].  Plans with exact pair
 // launches run p pairs (pair i: bufs[i%2] -> level 2i+2 in bufs[(i+1)%2]) and then s single sweeps (generate.hpp:
 // pair_split); both buffers end exactly as after n single sweeps.
 int enqueue_run(drs_plan* p, void* a, void* b, int n, cudaStream_t stream) {
     int pairs = 0, singles = n;
-    if (p->pair) drs::pair_split(n, pairs, singles);
+    if (uses_pairs(p)) drs::pair_split(n, pairs, singles);
     int rc = DRS_OK;
     for (int i = 0; i < pairs && rc == DRS_OK; ++i)
         rc = (i & 1) ? launch_pair(p, b, a, a, b, stream) : launch_pair(p, a, b, a, b, stream);
@@ -913,7 +917,7 @@ static bool run_graph(drs_plan* p, void* a, void* b, int n, bool slab, cudaStrea
         // only drs_run's sequence has pair launches
         CUtensorMap* tm = nullptr;
         if (tensor_map_for(p, a, &tm) != DRS_OK || tensor_map_for(p, b, &tm) != DRS_OK) return false;
-        if (p->pair && !slab && (tensor_map_for(p, a, &tm, true) != DRS_OK || tensor_map_for(p, b, &tm, true) != DRS_OK)) return false;
+        if (uses_pairs(p) && !slab && (tensor_map_for(p, a, &tm, true) != DRS_OK || tensor_map_for(p, b, &tm, true) != DRS_OK)) return false;
         const long long l0 = p->launches;
         if (cudaStreamBeginCapture(p->cap_stream, cudaStreamCaptureModeThreadLocal) != cudaSuccess) {
             cudaGetLastError(); p->use_graph = false; return false;
@@ -968,7 +972,7 @@ int drs_plan_pair_split(const drs_plan* p, int iterations, int* pairs, int* sing
     if (!p) return fail(DRS_E_ARG, "null plan");
     const int n = sweeps_for(p, iterations);
     int np = 0, ns = n;
-    if (p->pair) drs::pair_split(n, np, ns);
+    if (uses_pairs(p)) drs::pair_split(n, np, ns);
     if (pairs) *pairs = np;
     if (singles) *singles = ns;
     return n;

@@ -146,10 +146,11 @@ int drs_gold_sweep(drs_plan *p, const void *d_in, void *d_out, void *stream);
  * On 3D step-1 plans whose arrays are >= 1 GiB each (16-byte row pitch, an operator the depth-2 tile fits) the
  * sweeps run as exact pair launches -- one kernel computes two sweeps, bit for bit, with each level's ring taken from
  * the buffer that level lives in -- followed by two or four single sweeps; A and B end exactly as after the plain
- * loop (drs_plan_pair_split). */
+ * loop (drs_plan_pair_split).  A slab plan (drs_plan_set_slab) never gets pair launches: its drs_run is the loop of
+ * drs_sweep, boundary planes pushed to the neighbours' ghost planes and no step flags. */
 int drs_run(drs_plan *p, void *d_a, void *d_b, int iterations, void *stream, int *sweeps);
 /* how drs_run splits the sweeps of `iterations` timesteps: *pairs pair launches, then *singles single sweeps
- * (*pairs = 0 on plans without pair launches); returns the number of sweeps.  Needs no GPU. */
+ * (*pairs = 0 on plans without pair launches, slab plans included); returns the number of sweeps.  Needs no GPU. */
 int drs_plan_pair_split(const drs_plan *p, int iterations, int *pairs, int *singles);
 /* drs_run replays its launches as one CUDA graph per (d_a, d_b, sweep count) -- same kernels, same
  * order, without the gap between dependent launches (matters for grids as small as 4096^2).  On

@@ -57,6 +57,9 @@ OPS = {
     # fp32 over six sweeps
     "star7asym": {(0, 0, 0): -1 / 4, (-1, 0, 0): 1 / 8, (1, 0, 0): -1 / 8, (0, -1, 0): -1 / 8, (0, 1, 0): 1 / 8,
                   (0, 0, -1): 1 / 8, (0, 0, 1): -1 / 8},
+    # two terms of +-1/2 on a diagonal through k, j and i: sum |K| = 1 with f = 1, so values stay multiples of 2^-d
+    # below 3 -- exact over the 16 to 24 levels of the deep fused slab runs (test_exact_slab*.py), fp32 included
+    "diag2k": {(-1, 0, 0): 1 / 2, (1, 1, -1): -1 / 2},
     # shaped like the shipped 2D stencils (same offsets, same classes of equal coefficients, hence the same kernel
     # path as the preset: test_exact_sizes.py compares the generated units).  Composed coefficients must print
     # exactly with 6 digits (generate.hpp), which rules out deep dyadic fractions: c2 and c3 use small integers with a
@@ -282,15 +285,22 @@ def interior(shape, H):
     return tuple(slice(H, n - H) for n in shape)
 
 
-def exact_run(op, step, A, B, sweeps):
+def _f64(u):
+    return u.astype(np.float64) if _is_np(u) else u.to(_torch().float64).clone()
+
+
+def exact_run(op, step, A, B, sweeps, slow=None):
     """The ping-pong schedule of Plan.run: sweep s writes interior(Halo) of buffer (s + 1) % 2 from buffer s % 2,
-    every sweep applying the operator `step` times; the destination's ring keeps its contents.  float64 copies."""
-    bufs = [A.astype(np.float64), B.astype(np.float64)]
+    every sweep applying the operator `step` times; the destination's ring keeps its contents.  float64 copies (numpy
+    or torch, like the inputs).  slow = (lo, hi): the sweeps write slow-axis planes / rows [lo, hi) instead of
+    [Halo, n - Halo) -- a slab's output range, everything outside it (its ghost planes) frozen."""
+    bufs = [_f64(A), _f64(B)]
     H = halo_of(op, step)
-    inner = interior(A.shape, H)
+    lo, hi = (H, A.shape[0] - H) if slow is None else slow
+    inner = (slice(lo, hi),) + interior(A.shape[1:], H)
     for s in range(sweeps):
         src, dst = bufs[s & 1], bufs[(s & 1) ^ 1]
-        if all(n > 2 * H for n in A.shape):
+        if hi > lo and all(n > 2 * H for n in A.shape[1:]):
             dst[inner] = apply_levels(src, op, step)[inner]
     return bufs
 
@@ -516,16 +526,17 @@ def source_window(op, step, sweeps, n_slow, z0, z1):
     return max(0, z0 - sweeps * step * rm), min(n_slow, z1 + sweeps * step * rp)
 
 
-def window_run(op, step, sweeps, shape, z0, z1, source):
+def window_run(op, step, sweeps, shape, z0, z1, source, slow=None):
     """exact_run restricted to slow-axis planes / rows [z0, z1) of both buffers: `source(s0, s1)` gives (A, B) over
-    source_window(), float64 (numpy or torch); sweeps write the interior of the global grid, the frozen ring keeps its
-    contents.  Planes the window's cut edges make wrong after sweep s lie within s * step * r of the cut, outside
-    [z0, z1).  Returns the float64 windows (A, B)."""
+    source_window(), float64 (numpy or torch); sweeps write the interior of the global grid (slow: exact_run's
+    slow-axis output range instead), the frozen ring keeps its contents.  Planes the window's cut edges make wrong
+    after sweep s lie within s * step * r of the cut, outside [z0, z1).  Returns the float64 windows (A, B)."""
     s0, s1 = source_window(op, step, sweeps, shape[0], z0, z1)
     bufs = list(source(s0, s1))
     H = halo_of(op, step)
-    if all(n > 2 * H for n in shape):
-        lo, hi = max(H, s0) - s0, min(shape[0] - H, s1) - s0
+    olo, ohi = (H, shape[0] - H) if slow is None else slow
+    if ohi > olo and all(n > 2 * H for n in shape[1:]):
+        lo, hi = max(olo, s0) - s0, min(ohi, s1) - s0
         inner = (slice(lo, max(lo, hi)),) + interior(shape[1:], H)
         for s in range(sweeps):
             src, dst = bufs[s & 1], bufs[(s & 1) ^ 1]
