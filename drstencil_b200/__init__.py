@@ -92,6 +92,8 @@ def lib():
         "drs_plan_cache_key": (ctypes.c_char_p, [vp]),
         "drs_plan_pair_source": (ctypes.c_char_p, [vp]),
         "drs_plan_pair_cache_key": (ctypes.c_char_p, [vp]),
+        "drs_plan_slab_source": (ctypes.c_char_p, [vp]),
+        "drs_plan_slab_cache_key": (ctypes.c_char_p, [vp]),
         "drs_plan_pair_split": (i32, [vp, i32, P(i32), P(i32)]),
         "drs_sweep": (i32, [vp, vp, vp, vp]),
         "drs_gold_sweep": (i32, [vp, vp, vp, vp]),
@@ -411,6 +413,16 @@ class Plan:
     @property
     def pair_cache_key(self) -> str:
         return lib().drs_plan_pair_cache_key(self._h).decode()
+
+    @property
+    def slab_source(self) -> str:
+        """Translation unit of the 2D slab entry drslab_<name>, made by set_slab ("" on 3D plans, whose main unit has
+        it, and on plans without a slab kernel)."""
+        return lib().drs_plan_slab_source(self._h).decode()
+
+    @property
+    def slab_cache_key(self) -> str:
+        return lib().drs_plan_slab_cache_key(self._h).decode()
 
     def pair_split(self, iterations: int):
         """(pairs, singles): run() performs `pairs` exact pair launches, then `singles` single sweeps."""

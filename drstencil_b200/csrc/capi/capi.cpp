@@ -35,6 +35,9 @@ extern const int drs_embedded_header_count;
 extern const char* const drs_pair_header_names[];
 extern const char* const drs_pair_header_texts[];
 extern const int drs_pair_header_count;
+extern const char* const drs_slab2d_header_names[];
+extern const char* const drs_slab2d_header_texts[];
+extern const int drs_slab2d_header_count;
 
 namespace {
 
@@ -187,15 +190,22 @@ std::string cache_dir() {
 const char* kNvrtcOpts[] = {"--gpu-architecture=sm_100a", "-std=c++17", "-lineinfo", "--fmad=false",
                             "-default-device", "--ptxas-options=-v"};
 
+// Which unit compile_cubin builds: the plan's main unit, the exact pair kernel's (kernels/pair/ headers) or the 2D slab
+// entry's (kernels/slab2d/ headers).
+enum class Unit { MAIN, PAIR, SLAB2D };
+
 // source -> cubin, through the on-disk cache.  The key covers the source, every header the unit may include and the
-// options.  pair: the unit of the exact pair kernel, which may include the kernels/pair/ headers as well (they are part
-// of its key only: the keys of every other unit do not depend on them).
-int compile_cubin(const std::string& src, std::vector<char>& cubin, std::string& key_out, bool pair = false) {
+// options.  The pair and 2D slab units may include their own subdirectory's headers as well; those are part of their
+// keys only: the keys of every other unit do not depend on them.
+int compile_cubin(const std::string& src, std::vector<char>& cubin, std::string& key_out, Unit unit = Unit::MAIN) {
     std::vector<const char*> names(drs_embedded_header_names, drs_embedded_header_names + drs_embedded_header_count);
     std::vector<const char*> texts(drs_embedded_header_texts, drs_embedded_header_texts + drs_embedded_header_count);
-    if (pair) {
+    if (unit == Unit::PAIR) {
         names.insert(names.end(), drs_pair_header_names, drs_pair_header_names + drs_pair_header_count);
         texts.insert(texts.end(), drs_pair_header_texts, drs_pair_header_texts + drs_pair_header_count);
+    } else if (unit == Unit::SLAB2D) {
+        names.insert(names.end(), drs_slab2d_header_names, drs_slab2d_header_names + drs_slab2d_header_count);
+        texts.insert(texts.end(), drs_slab2d_header_texts, drs_slab2d_header_texts + drs_slab2d_header_count);
     }
     std::string all = src;
     for (const char* t : texts) all += t;
@@ -294,10 +304,16 @@ struct drs_plan {
     CUmodule pmod = nullptr;
     CUfunction f_pair = nullptr;
     std::map<const void*, CUtensorMap> ptmaps;
+    // 2D slab plans (generate.hpp: has_slab2d_unit): the unit of drslab_, generated and compiled by drs_plan_set_slab, its
+    // module loaded with the plan's device state.  The tensor maps are the main kernel's.
+    std::string slab_source, slab_key;
+    std::vector<char> slab_cubin;
+    CUmodule smod = nullptr;
     // device state (bound at first use)
     bool loaded = false;
     int device = -1;
     CUmodule mod = nullptr;
+    // f_slab: drslab_, from the main module (3D) or from smod (2D)
     CUfunction f_sweep = nullptr, f_slab = nullptr, f_gold = nullptr, f_check = nullptr, f_signal = nullptr, f_wait = nullptr;
     int regs = 0, spill = 0;
     int* d_fault = nullptr;
@@ -335,6 +351,25 @@ struct drs_plan {
 
 namespace {
 
+// The 2D slab unit's module and drslab_, with f_sweep's dynamic shared memory and carve-out (once the plan is loaded and
+// has a compiled slab unit; drs_plan_set_slab may come after the first use of the plan)
+int load_slab2d(drs_plan* p) {
+    if (p->slab_cubin.empty() || p->smod) return DRS_OK;
+    Driver& d = driver();
+    CUresult r = d.ModuleLoadData(&p->smod, p->slab_cubin.data());
+    if (r != CUDA_SUCCESS) { p->smod = nullptr; return fail(DRS_E_CUDA, "cuModuleLoadData(slab): " + cu_err(r)); }
+    r = d.ModuleGetFunction(&p->f_slab, p->smod, ("drslab_" + p->spec.name).c_str());
+    if (r == CUDA_SUCCESS) r = d.FuncSetAttribute(p->f_slab, CU_FUNC_ATTRIBUTE_MAX_DYNAMIC_SHARED_SIZE_BYTES, p->spec.smem_bytes());
+    if (r != CUDA_SUCCESS) {
+        d.ModuleUnload(p->smod);
+        p->smod = nullptr;
+        p->f_slab = nullptr;
+        return fail(DRS_E_CUDA, "cuModuleGetFunction(drslab_): " + cu_err(r));
+    }
+    if (const char* co = std::getenv("DRS_CARVEOUT")) d.FuncSetAttribute(p->f_slab, CU_FUNC_ATTRIBUTE_PREFERRED_SHARED_MEMORY_CARVEOUT, std::atoi(co));
+    return DRS_OK;
+}
+
 int ensure_loaded(drs_plan* p) {
     if (p->loaded) {
         // the module, tensor maps and scratch memory belong to the device that was current at first use
@@ -342,7 +377,7 @@ int ensure_loaded(drs_plan* p) {
         if (cudaGetDevice(&cur) != cudaSuccess || cur != p->device)
             return fail(DRS_E_ARG, "plan is bound to CUDA device " + std::to_string(p->device) + " but device " +
                                        std::to_string(cur) + " is current");
-        return DRS_OK;
+        return load_slab2d(p);
     }
     Driver& d = driver();
     if (!d.ok) return fail(DRS_E_NOGPU, "drstencil needs a CUDA device (no CPU fallback): " + d.why);
@@ -406,7 +441,7 @@ int ensure_loaded(drs_plan* p) {
     cudaMemset(p->d_fault, 0, sizeof(int));
     if (cudaMalloc(&p->d_res, 2 * sizeof(double)) != cudaSuccess) return fail(DRS_E_CUDA, "cudaMalloc(result)");
     p->loaded = true;
-    return DRS_OK;
+    return load_slab2d(p);
 }
 
 int tensor_map_for(drs_plan* p, const void* base, CUtensorMap** out, bool pair = false) {
@@ -496,22 +531,25 @@ void fill_params(const drs_plan* p, const void* in, void* out, DevParams& q, int
     }
     q.chunk = s.chunk;
     q.fault = p->d_fault;
-    if (seq_off >= 0 && p->slab && p->my_flags && p->d_sync && s.dim == 3 && !sub && (q.peer_lo || q.peer_hi)) {
+    if (seq_off >= 0 && p->slab && p->my_flags && p->d_sync && !sub && (q.peer_lo || q.peer_hi)) {
         q.my_flags = (const long long*)p->my_flags;
         q.lower_flag = q.peer_lo ? (long long*)p->lower_flag : nullptr;
         q.upper_flag = q.peer_hi ? (long long*)p->upper_flag : nullptr;
         q.seq_base = (const long long*)p->d_sync;
         q.face_cnt = (unsigned int*)((char*)p->d_sync + sizeof(long long));
         q.seq_off = seq_off;
-        // a chunk [za, zb) belongs to a face when it reads that neighbour's ghost planes or produces planes
-        // that are pushed to it; its input reaches Halo planes beyond its outputs on both sides
+        // a chunk [za, zb) belongs to a face when it reads that neighbour's ghost planes (rows in 2D) or produces
+        // planes that are pushed to it; its input reaches Halo planes beyond its outputs on both sides.  The chunks are
+        // the nzs plane chunks in 3D, the nys row chunks in 2D (one unit = one warp, nxs of them per row chunk).
         const long long ghost = s.halo, local = p->local_slow();
         q.face_lo_end = 2 * ghost;
         q.face_hi_begin = local - 2 * ghost;
-        const long long units_per_chunk = s.share3d ? (long long)s.nw * ((q.nxs + s.sx - 1) / s.sx) * ((q.nys + s.sy - 1) / s.sy)
-                                                    : (long long)q.nxs * q.nys;
+        const long long units_per_chunk = s.dim == 2 ? (long long)q.nxs
+                                          : s.share3d ? (long long)s.nw * ((q.nxs + s.sx - 1) / s.sx) * ((q.nys + s.sy - 1) / s.sy)
+                                                      : (long long)q.nxs * q.nys;
+        const long long nchunks = s.dim == 2 ? q.nys : q.nzs;
         int nlo = 0, nhi = 0;
-        for (long long zc = 0; zc < q.nzs; ++zc) {
+        for (long long zc = 0; zc < nchunks; ++zc) {
             const long long za = q.slow_lo + zc * s.chunk, zb = std::min(za + s.chunk, q.slow_hi);
             if (q.lower_flag && za < q.face_lo_end) ++nlo;
             if (q.upper_flag && zb > q.face_hi_begin) ++nhi;
@@ -519,7 +557,7 @@ void fill_params(const drs_plan* p, const void* in, void* out, DevParams& q, int
         // the kernel lists the lower-face chunks first, then the upper-face ones; a chunk that touches both
         // faces (thin slabs) is counted on both and keeps its place in the prefix
         q.face_lo_chunks = nlo;
-        q.face_hi_chunks = std::min<long long>(nhi, q.nzs - nlo);
+        q.face_hi_chunks = std::min<long long>(nhi, nchunks - nlo);
         q.face_lo_units = (unsigned int)(nlo * units_per_chunk);
         q.face_hi_units = (unsigned int)(nhi * units_per_chunk);
     }
@@ -599,9 +637,13 @@ int launch_one(drs_plan* p, const void* in, void* out, cudaStream_t stream, int 
     const long long ctas = p->spec.ctas(q.nxs, q.nys, q.nzs);
     if (ctas > 0x7fffffffLL) return fail(DRS_E_ARG, "grid too large");
     void* args[] = {tm, &q};
-    CUresult r = driver().LaunchKernel(q.my_flags && p->f_slab ? p->f_slab : p->f_sweep, (unsigned)ctas, 1, 1, (unsigned)(p->spec.nw * 32), 1, 1,
+    // 3D: drslab_ runs the flagged sweeps of drs_run_slab (dr_ makes the peer stores itself).  2D: dr_ makes none, so
+    // every launch of a slab plan with peers runs drslab_ (flags or not); without peers the ghost rows stay frozen.
+    const bool slab_fn = p->spec.dim == 2 ? p->slab && p->my_bases[0] != nullptr : q.my_flags != nullptr;
+    if (slab_fn && !p->f_slab) return fail(DRS_E_ARG, "this plan has no slab kernel");
+    CUresult r = driver().LaunchKernel(slab_fn ? p->f_slab : p->f_sweep, (unsigned)ctas, 1, 1, (unsigned)(p->spec.nw * 32), 1, 1,
                                        (unsigned)p->spec.smem_bytes(), (CUstream)stream, args, nullptr);
-    if (r != CUDA_SUCCESS) return fail(DRS_E_CUDA, "launch dr_: " + cu_err(r));
+    if (r != CUDA_SUCCESS) return fail(DRS_E_CUDA, std::string(slab_fn ? "launch drslab_: " : "launch dr_: ") + cu_err(r));
     p->launches++;
     return DRS_OK;
 }
@@ -697,7 +739,7 @@ int make_plan(const drs_stencil* s, const drs_knobs* k, drs_plan** out, bool com
     if (p->pair) p->pair_source = drs::generate_pair_tu(p->pspec);
     if (compile) {
         rc = compile_cubin(p->source, p->cubin, p->cache_key);
-        if (rc == DRS_OK && p->pair) rc = compile_cubin(p->pair_source, p->pair_cubin, p->pair_key, true);
+        if (rc == DRS_OK && p->pair) rc = compile_cubin(p->pair_source, p->pair_cubin, p->pair_key, Unit::PAIR);
         if (rc != DRS_OK) { delete p; return rc; }
     }
     *out = p;
@@ -833,6 +875,7 @@ void drs_plan_destroy(drs_plan* p) {
         for (auto& g : p->graphs) cudaGraphExecDestroy(g.second.exec);
         if (p->mod) driver().ModuleUnload(p->mod);
         if (p->pmod) driver().ModuleUnload(p->pmod);
+        if (p->smod) driver().ModuleUnload(p->smod);
     }
     delete p;
 }
@@ -875,6 +918,8 @@ const char* drs_plan_note(const drs_plan* p) { return p ? p->spec.note.c_str() :
 const char* drs_plan_cache_key(const drs_plan* p) { return p ? p->cache_key.c_str() : ""; }
 const char* drs_plan_pair_source(const drs_plan* p) { return p ? p->pair_source.c_str() : ""; }
 const char* drs_plan_pair_cache_key(const drs_plan* p) { return p ? p->pair_key.c_str() : ""; }
+const char* drs_plan_slab_source(const drs_plan* p) { return p ? p->slab_source.c_str() : ""; }
+const char* drs_plan_slab_cache_key(const drs_plan* p) { return p ? p->slab_key.c_str() : ""; }
 
 int drs_sweep(drs_plan* p, const void* d_in, void* d_out, void* stream) {
     if (!p || !d_in || !d_out) return fail(DRS_E_ARG, "null argument");
@@ -1230,6 +1275,13 @@ int drs_plan_set_slab(drs_plan* p, long long global_slow, long long lo, long lon
         return fail(DRS_E_ARG, "slab runs cannot use per-sub-step launches: use the fused temporal kernel or --fuse algebraic");
     if (hi - lo + 2 * ghost != p->local_slow())
         return fail(DRS_E_ARG, "slab arrays must hold hi - lo + 2*Halo planes along the slow axis");
+    if (drs::has_slab2d_unit(p->spec) && p->slab_cubin.empty()) {
+        std::string src = drs::generate_tu(p->spec, true), key;
+        std::vector<char> cubin;
+        const int rc = compile_cubin(src, cubin, key, Unit::SLAB2D);
+        if (rc != DRS_OK) return rc;
+        p->slab_source = std::move(src); p->slab_key = std::move(key); p->slab_cubin = std::move(cubin);
+    }
     p->slab = true; p->g_slow = global_slow; p->lo = lo; p->hi = hi;
     drop_graphs(p);      // launch parameters changed
     return DRS_OK;
@@ -1239,7 +1291,9 @@ int drs_plan_set_peers(drs_plan* p, void* const my_bases[2], void* const lower_b
                        long long lower_lo, long long upper_lo) {
     if (!p || !my_bases) return fail(DRS_E_ARG, "null argument");
     if (!p->slab) return fail(DRS_E_ARG, "call drs_plan_set_slab first");
-    if (p->spec.dim != 3 || !p->spec.tma_ok) return fail(DRS_E_ARG, "fused halo push is implemented for the 3D TMA sweep");
+    if (p->spec.reuse) return fail(DRS_E_ARG, "--fuse reuse has no fused halo push: use --fuse temporal or algebraic on a slab");
+    if (!p->spec.tma_ok)
+        return fail(DRS_E_ARG, "this plan runs the naive kernel (operator too deep for the TMA ring), which has no fused halo push");
     for (int b = 0; b < 2; ++b)
         for (const void* q : {(const void*)my_bases[b], lower_bases ? (const void*)lower_bases[b] : nullptr,
                               upper_bases ? (const void*)upper_bases[b] : nullptr})

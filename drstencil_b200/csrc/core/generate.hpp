@@ -565,14 +565,18 @@ inline void emit_chain(std::ostringstream& o, const char* macro, const std::vect
 
 // The specialised translation unit (kernel templates are #included by name and resolved from
 // the headers embedded in libdrstencil.so, or from -I .../csrc/kernels for emitted programs).
-inline std::string generate_tu(const KernelSpec& s) {
+// slab2d: the 2D slab unit instead (has_slab2d_unit): every macro of the main unit -- same geometry, chain and tensor
+// maps -- with kernels/slab2d/drs_slab2d.cuh in place of the sweep and gold kernels.
+inline std::string generate_tu(const KernelSpec& s, bool slab2d = false) {
     std::ostringstream o;
     o << "// generated by drstencil-b200 for sm_100a -- stencil '" << s.name << "', " << (s.dim == 3 ? "3D" : "2D")
       << ", " << (s.dtype == DRS_F64 ? "fp64" : "fp32") << ", step " << s.step << " ("
-      << (s.reuse ? "forward/backward data reuse" : s.ts > 1 ? "temporal" : (s.step > 1 ? "algebraic" : "single")) << ")\n";
+      << (s.reuse ? "forward/backward data reuse" : s.ts > 1 ? "temporal" : (s.step > 1 ? "algebraic" : "single")) << ")"
+      << (slab2d ? ", slab entry" : "") << "\n";
     o << "#define DRS_DIM " << s.dim << "\n";
     o << "#define DRS_T " << (s.dtype == DRS_F64 ? "double" : "float") << "\n";
-    o << "#define DRS_NAME dr_" << s.name << "\n";
+    // (the slab unit's copy of the plain kernel is never launched; the plan's main unit has the real dr_)
+    o << "#define DRS_NAME " << (slab2d ? "unused_dr_" : "dr_") << s.name << "\n";
     o << "#define DRS_SLAB_NAME drslab_" << s.name << "\n";
     o << "#define DRS_GOLD_NAME gold_" << s.name << "\n";
     o << "#define DRS_CHECK_NAME check_" << s.name << "\n";
@@ -612,6 +616,10 @@ inline std::string generate_tu(const KernelSpec& s) {
     if (s.fused3d) emit_scatter3(o, s);
     if (s.ts > 1 && s.fscale != 1.0) o << "#define DRS_OUT_SCALE (" << lit17(std::pow(s.fscale, s.ts)) << ")\n";
     emit_chain(o, "DRS_GOLD_CHAIN", s.gold);
+    if (slab2d) {
+        o << "#include \"drs_slab2d.cuh\"\n";
+        return o.str();
+    }
     if (s.reuse) o << "#include \"drs_reuse.cuh\"\n";
     else if (s.tma_ok)
         o << "#include \"" << (s.fused3d ? "drs_sweep3d_t.cuh" : s.share3d ? "drs_sweep3d_cta.cuh" : s.dim == 3 ? "drs_sweep3d.cuh" : "drs_sweep2d.cuh") << "\"\n";
@@ -698,6 +706,13 @@ inline std::string generate_pair_tu(const KernelSpec& s) {
     o << "#include \"drs_pair3d.cuh\"\n";
     return o.str();
 }
+
+// ---- 2D slab entry (drs_run_slab and the peer stores on 2D slab plans; kernels/slab2d/drs_slab2d.cuh) -------------
+
+// Whether a plan whose main specialisation is `s` gets a 2D slab unit (generate_tu(s, true)) when it becomes a slab: the
+// 2D TMA sweep (not the naive kernel of a too-deep operator, not `--fuse reuse`).  3D plans carry drslab_ in their main
+// unit.
+inline bool has_slab2d_unit(const KernelSpec& s) { return s.dim == 2 && s.tma_ok && !s.reuse; }
 
 inline uint64_t fnv1a(const std::string& s, uint64_t h = 1469598103934665603ull) {
     for (unsigned char c : s) { h ^= c; h *= 1099511628211ull; }

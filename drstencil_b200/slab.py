@@ -1,10 +1,10 @@
-"""Slab decomposition of a 3D grid along k (the slowest axis) over the GPUs of one box, one process
-per GPU (torchrun), with nearest-neighbour halo exchange after every sweep.
+"""Slab decomposition of a grid along its slowest axis (planes, k, of a 3D grid; rows, j, of a 2D one) over the GPUs
+of one box, one process per GPU (torchrun), with nearest-neighbour halo exchange after every sweep.
 
 The reference is single-GPU (SURVEY.md F5); this is the engine's extension for BASELINE.json
-config c5.  Semantics are those of ONE global grid swept by the reference's schedule: the global
-Halo-wide ring stays frozen, every rank owns planes [lo, hi) and keeps `ghost` = Halo copies of
-its neighbours' boundary planes on each side.
+config c5 and the 2D configs.  Semantics are those of ONE global grid swept by the reference's schedule: the global
+Halo-wide ring stays frozen, every rank owns planes (rows) [lo, hi) and keeps `ghost` = Halo copies of
+its neighbours' boundary planes (rows) on each side.  Below, "plane" stands for a row of a 2D grid.
 
 Exchange paths (`halo=`):
   "p2p"        drs_run_slab: ONE launch per sweep.  The sweep kernel stores its boundary planes a second
@@ -70,8 +70,8 @@ class SlabGeometry:
 
 
 def halo_exchange(buf, geom: SlabGeometry, group=None) -> None:
-    """Refreshes the ghost planes of `buf` (a [local_planes, M, N] tensor) from the neighbours'
-    boundary planes with point-to-point sends/receives."""
+    """Refreshes the ghost planes of `buf` (a [local_planes, M, N] or [local_planes, N] tensor) from the
+    neighbours' boundary planes with point-to-point sends/receives."""
     import torch.distributed as dist
     ops = []
     if geom.lower is not None:
@@ -169,22 +169,20 @@ class GpuSlab:
         from . import Plan, Stencil, F32
         self.rank, self.world, self.mode, self.group = rank, world, halo, group
         st = Stencil.from_file(stc_path)
-        if st.dim != 3:
-            raise ValueError("slab decomposition is implemented for 3D grids")
         if global_shape is not None:
             st.set_size(global_shape)
         self.global_shape = tuple(st.shape)
-        L, M, N = self.global_shape
+        slow, rest = self.global_shape[0], self.global_shape[1:]     # (L, (M, N)) or (M, (N,))
         probe = Plan(st, knobs)                      # halo of the (possibly multi-step) sweep
         ghost = probe.halo
         self.step = knobs.step
-        self.geom = SlabGeometry(L, world, rank, ghost)
-        st.set_size((self.geom.local_planes, M, N))
+        self.geom = SlabGeometry(slow, world, rank, ghost)
+        shape = (self.geom.local_planes,) + rest
+        st.set_size(shape)
         self.plan = Plan(st, knobs)
-        self.plan.set_slab(L, self.geom.lo, self.geom.hi)
+        self.plan.set_slab(slow, self.geom.lo, self.geom.hi)
         self.dtype = torch.float32 if knobs.dtype == F32 else torch.float64
         typestr, isz = ("<f4", 4) if knobs.dtype == F32 else ("<f8", 8)
-        shape = (self.geom.local_planes, M, N)
         self._raw = [_DevArray(shape, typestr, isz), _DevArray(shape, typestr, isz)]
         self.bufs = [r.tensor() for r in self._raw]
         for b in self.bufs:
@@ -240,8 +238,8 @@ class GpuSlab:
 
     # -- data --
     def fill(self, plane_fn: Callable) -> None:
-        """A[local plane] = plane_fn(global plane index) for every in-grid plane this rank holds
-        (owned and ghost); B = 0.  Restarts the schedule at sweep(A, B).  Collective: every rank calls it."""
+        """A[local plane] = plane_fn(global plane index) for every in-grid plane (row of a 2D grid) this rank
+        holds (owned and ghost); B = 0.  Restarts the schedule at sweep(A, B).  Collective: every rank calls it."""
         import torch
         import torch.distributed as dist
         g = self.geom

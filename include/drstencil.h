@@ -133,6 +133,10 @@ const char *drs_plan_cache_key(const drs_plan *p);
 /* the translation unit / cache key of the exact pair kernel drs_run uses on this plan, "" if it uses none */
 const char *drs_plan_pair_source(const drs_plan *p);
 const char *drs_plan_pair_cache_key(const drs_plan *p);
+/* the translation unit / cache key of the slab entry drslab_<name> of a 2D plan, generated and compiled (NVRTC, no GPU
+ * needed) by drs_plan_set_slab; "" for every other plan (3D plans carry drslab_ in their main unit) */
+const char *drs_plan_slab_source(const drs_plan *p);
+const char *drs_plan_slab_cache_key(const drs_plan *p);
 
 /* one `dr_<name><<<grid, block>>>(d_in, d_out)` (codegen_2d.hpp:606): advances the interior
  * [Halo, dim-Halo) by `step` timesteps; the Halo ring of d_out is not written.  d_in != d_out.
@@ -196,15 +200,18 @@ long long drs_plan_launch_count(const drs_plan *p);
 /* ---- slab decomposition along the slowest axis (extension; the reference is single-GPU) -- */
 
 /* Declares that this plan's arrays are a slab: planes (3D) / rows (2D) [lo, hi) of a global grid
- * with `global_slow` planes, stored with `ghost` = step*radius extra planes on each side, i.e.
- * the local array holds (hi - lo + 2*ghost) planes.  The global frozen ring applies only at the
- * global faces.  Must be called before the first sweep. */
+ * with `global_slow` planes (rows), stored with `ghost` = step*radius extra planes (rows) on each side, i.e.
+ * the local array holds (hi - lo + 2*ghost) planes (rows).  The global frozen ring applies only at the
+ * global faces.  Must be called before the first sweep.  On a 2D plan with the TMA sweep this generates and
+ * compiles the slab unit (drs_plan_slab_source). */
 int drs_plan_set_slab(drs_plan *p, long long global_slow, long long lo, long long hi);
-/* Fused halo push (3D): while sweeping into my_bases[b], the kernel stores its boundary planes a
- * second time, straight into the neighbours' ghost planes over NVLink.  lower_bases / upper_bases
+/* Fused halo push: while sweeping into my_bases[b], the kernel stores its boundary planes (3D) / rows (2D) a
+ * second time, straight into the neighbours' ghost planes / rows over NVLink.  lower_bases / upper_bases
  * are the *neighbours' array bases* (same ping-pong order, mapped into this process with
  * drs_ipc_import), NULL where there is no neighbour; lower_lo / upper_lo are the neighbours' first
- * owned global planes (their `lo`). */
+ * owned global planes / rows (their `lo`).  On a 2D plan every sweep then runs the slab entry drslab_<name>; a 2D
+ * slab plan without peers keeps the plain kernel and frozen ghost rows.  DRS_E_ARG for plans without a slab kernel:
+ * `--fuse reuse` and the naive kernel of operators too deep for the TMA ring. */
 int drs_plan_set_peers(drs_plan *p, void *const my_bases[2], void *const lower_bases[2],
                        void *const upper_bases[2], long long lower_lo, long long upper_lo);
 /* Cross-GPU step flags.  Each rank owns a device array of two 64-bit slots (slot 0 written by its lower
@@ -213,18 +220,18 @@ int drs_plan_set_peers(drs_plan *p, void *const my_bases[2], void *const lower_b
  * lower_flag = the lower neighbour's slot 1, upper_flag = the upper neighbour's slot 0 (NULL where there is no
  * neighbour).  Flag values are monotone over the life of the plan (sweeps run so far), never reset. */
 int drs_plan_set_flags(drs_plan *p, const void *my_flags, void *lower_flag, void *upper_flag);
-/* This rank's share of the emitted host loop (codegen.hpp:575-589) on a slab-decomposed grid: `for (t = 0; t <
- * iterations; t += 2*step) { sweep(A,B); sweep(B,A); }` over the arrays given to drs_plan_set_peers, ONE kernel
- * launch per sweep, replayed as a CUDA graph.  The sweep kernel does the whole exchange itself: tiles next to a
- * neighbour's slab wait (ld.acquire.sys) until that neighbour's boundary tiles of the previous sweep are done,
- * boundary planes are stored a second time into the neighbour's ghost planes over NVLink, and the last boundary
+/* This rank's share of the emitted host loop (codegen.hpp:575-589, codegen_2d.hpp:610-613) on a slab-decomposed grid:
+ * `for (t = 0; t < iterations; t += 2*step) { sweep(A,B); sweep(B,A); }` over the arrays given to drs_plan_set_peers,
+ * ONE kernel launch per sweep, replayed as a CUDA graph.  The sweep kernel does the whole exchange itself: tiles next
+ * to a neighbour's slab wait (ld.acquire.sys) until that neighbour's boundary tiles of the previous sweep are done,
+ * boundary planes (rows in 2D) are stored a second time into the neighbour's ghost planes over NVLink, and the last boundary
  * tile of a face releases the next flag value (st.release.sys); boundary tiles are scheduled first, so the
  * signal leaves early and the next sweep does not wait.  Every rank must call it with the same `iterations`;
  * after new data was written into the arrays (ghost planes included) the ranks must pass a barrier of the
  * caller's before the next call.  Writes the number of sweeps to *sweeps. */
 int drs_run_slab(drs_plan *p, int iterations, void *stream, int *sweeps);
 /* This rank's share of a slab-decomposed HOST-buffer run (the executor of drs_plan_slab_schedule): h_own = the
- * rank's own planes (pinned for overlap), result written back in place; uploads, sweeps and downloads overlap
+ * rank's own planes (rows in 2D; pinned for overlap), result written back in place; uploads, sweeps and downloads overlap
  * by time-skewed blocks, the faces run in lockstep with the neighbours through the plan's flags.  The device
  * arrays are the ones given to drs_plan_set_peers (second one zero-initialised by the caller).  Ranks pass a
  * barrier of the caller's between calls.  up_skew as for drs_plan_slab_schedule.  *device_ms as drs_run_host. */
