@@ -94,6 +94,11 @@ def lib():
         "drs_plan_pair_cache_key": (ctypes.c_char_p, [vp]),
         "drs_plan_slab_source": (ctypes.c_char_p, [vp]),
         "drs_plan_slab_cache_key": (ctypes.c_char_p, [vp]),
+        "drs_plan_slab_pair_source": (ctypes.c_char_p, [vp]),
+        "drs_plan_slab_pair_cache_key": (ctypes.c_char_p, [vp]),
+        "drs_plan_slab_split": (i32, [vp, i32, P(i32), P(i32)]),
+        "drs_sweep_pair": (i32, [vp, vp, vp, vp]),
+        "drs_plan_set_slab_pairs": (i32, [vp, ll, ll, ll]),
         "drs_plan_pair_split": (i32, [vp, i32, P(i32), P(i32)]),
         "drs_sweep": (i32, [vp, vp, vp, vp]),
         "drs_gold_sweep": (i32, [vp, vp, vp, vp]),
@@ -424,6 +429,22 @@ class Plan:
     def slab_cache_key(self) -> str:
         return lib().drs_plan_slab_cache_key(self._h).decode()
 
+    @property
+    def slab_pair_source(self) -> str:
+        """Translation unit of the slab pair entry drslabpair_<name>, made by set_slab_pairs ("" on every other plan)."""
+        return lib().drs_plan_slab_pair_source(self._h).decode()
+
+    @property
+    def slab_pair_cache_key(self) -> str:
+        return lib().drs_plan_slab_pair_cache_key(self._h).decode()
+
+    def slab_split(self, iterations: int):
+        """(pairs, singles): run_slab() performs `pairs` pair launches, then `singles` single sweeps (pairs = 0
+        except after set_slab_pairs)."""
+        p, s = ctypes.c_int(), ctypes.c_int()
+        _check(lib().drs_plan_slab_split(self._h, iterations, ctypes.byref(p), ctypes.byref(s)))
+        return p.value, s.value
+
     def pair_split(self, iterations: int):
         """(pairs, singles): run() performs `pairs` exact pair launches, then `singles` single sweeps."""
         p, s = ctypes.c_int(), ctypes.c_int()
@@ -436,6 +457,10 @@ class Plan:
 
     def sweep(self, d_in, d_out, stream=None) -> None:
         _check(lib().drs_sweep(self._h, _ptr(d_in), _ptr(d_out), _stream(stream)))
+
+    def sweep_pair(self, d_in, d_out, stream=None) -> None:
+        """One pair launch on a pair slab with peers set (two sweeps, pushes, no flags): the counterpart of sweep()."""
+        _check(lib().drs_sweep_pair(self._h, _ptr(d_in), _ptr(d_out), _stream(stream)))
 
     def gold_sweep(self, d_in, d_out, stream=None) -> None:
         _check(lib().drs_gold_sweep(self._h, _ptr(d_in), _ptr(d_out), _stream(stream)))
@@ -512,6 +537,10 @@ class Plan:
 
     def set_slab(self, global_slow: int, lo: int, hi: int) -> None:
         _check(lib().drs_plan_set_slab(self._h, global_slow, lo, hi))
+
+    def set_slab_pairs(self, global_slow: int, lo: int, hi: int) -> None:
+        """set_slab with ghost regions of 2 * Halo planes: run_slab() then runs exact pair launches (see drstencil.h)."""
+        _check(lib().drs_plan_set_slab_pairs(self._h, global_slow, lo, hi))
 
     def set_peers(self, my_bases, lower_bases, upper_bases, lower_lo: int, upper_lo: int) -> None:
         arr = lambda xs: (ctypes.c_void_p * 2)(*[_ptr(x) or None for x in xs])

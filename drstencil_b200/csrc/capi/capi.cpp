@@ -38,6 +38,9 @@ extern const int drs_pair_header_count;
 extern const char* const drs_slab2d_header_names[];
 extern const char* const drs_slab2d_header_texts[];
 extern const int drs_slab2d_header_count;
+extern const char* const drs_slabpair_header_names[];
+extern const char* const drs_slabpair_header_texts[];
+extern const int drs_slabpair_header_count;
 
 namespace {
 
@@ -190,12 +193,12 @@ std::string cache_dir() {
 const char* kNvrtcOpts[] = {"--gpu-architecture=sm_100a", "-std=c++17", "-lineinfo", "--fmad=false",
                             "-default-device", "--ptxas-options=-v"};
 
-// Which unit compile_cubin builds: the plan's main unit, the exact pair kernel's (kernels/pair/ headers) or the 2D slab
-// entry's (kernels/slab2d/ headers).
-enum class Unit { MAIN, PAIR, SLAB2D };
+// Which unit compile_cubin builds: the plan's main unit, the exact pair kernel's (kernels/pair/ headers), the 2D slab
+// entry's (kernels/slab2d/ headers) or the slab entry of the pair kernel (kernels/slabpair/ headers).
+enum class Unit { MAIN, PAIR, SLAB2D, SLABPAIR };
 
 // source -> cubin, through the on-disk cache.  The key covers the source, every header the unit may include and the
-// options.  The pair and 2D slab units may include their own subdirectory's headers as well; those are part of their
+// options.  The pair and slab units may include their own subdirectory's headers as well; those are part of their
 // keys only: the keys of every other unit do not depend on them.
 int compile_cubin(const std::string& src, std::vector<char>& cubin, std::string& key_out, Unit unit = Unit::MAIN) {
     std::vector<const char*> names(drs_embedded_header_names, drs_embedded_header_names + drs_embedded_header_count);
@@ -206,6 +209,9 @@ int compile_cubin(const std::string& src, std::vector<char>& cubin, std::string&
     } else if (unit == Unit::SLAB2D) {
         names.insert(names.end(), drs_slab2d_header_names, drs_slab2d_header_names + drs_slab2d_header_count);
         texts.insert(texts.end(), drs_slab2d_header_texts, drs_slab2d_header_texts + drs_slab2d_header_count);
+    } else if (unit == Unit::SLABPAIR) {
+        names.insert(names.end(), drs_slabpair_header_names, drs_slabpair_header_names + drs_slabpair_header_count);
+        texts.insert(texts.end(), drs_slabpair_header_texts, drs_slabpair_header_texts + drs_slabpair_header_count);
     }
     std::string all = src;
     for (const char* t : texts) all += t;
@@ -309,6 +315,14 @@ struct drs_plan {
     std::string slab_source, slab_key;
     std::vector<char> slab_cubin;
     CUmodule smod = nullptr;
+    // pair slabs (drs_plan_set_slab_pairs): ghost regions of 2 * Halo planes, and drs_run_slab runs pair launches of
+    // drslabpair_ (geometry pspec, tensor maps ptmaps); its unit is compiled by drs_plan_set_slab_pairs, its module
+    // loaded with the plan's device state
+    bool slab_pairs = false;
+    std::string slabpair_source, slabpair_key;
+    std::vector<char> slabpair_cubin;
+    CUmodule spmod = nullptr;
+    CUfunction f_slabpair = nullptr;
     // device state (bound at first use)
     bool loaded = false;
     int device = -1;
@@ -347,13 +361,33 @@ struct drs_plan {
     long long slab_seq = 0;
 
     long long local_slow() const { return spec.dim == 3 ? st.L : st.M; }
+    long long ghost() const { return slab_pairs ? 2LL * spec.halo : spec.halo; }   // ghost planes per side of a slab
 };
 
 namespace {
 
+// The slab pair unit's module and drslabpair_ (once the plan is loaded and has a compiled slab pair unit)
+int load_slabpair(drs_plan* p) {
+    if (p->slabpair_cubin.empty() || p->spmod) return DRS_OK;
+    Driver& d = driver();
+    CUresult r = d.ModuleLoadData(&p->spmod, p->slabpair_cubin.data());
+    if (r != CUDA_SUCCESS) { p->spmod = nullptr; return fail(DRS_E_CUDA, "cuModuleLoadData(slab pair): " + cu_err(r)); }
+    r = d.ModuleGetFunction(&p->f_slabpair, p->spmod, ("drslabpair_" + p->spec.name).c_str());
+    if (r == CUDA_SUCCESS) r = d.FuncSetAttribute(p->f_slabpair, CU_FUNC_ATTRIBUTE_MAX_DYNAMIC_SHARED_SIZE_BYTES, p->pspec.smem_bytes());
+    if (r != CUDA_SUCCESS) {
+        d.ModuleUnload(p->spmod);
+        p->spmod = nullptr;
+        p->f_slabpair = nullptr;
+        return fail(DRS_E_CUDA, "cuModuleGetFunction(drslabpair_): " + cu_err(r));
+    }
+    return DRS_OK;
+}
+
 // The 2D slab unit's module and drslab_, with f_sweep's dynamic shared memory and carve-out (once the plan is loaded and
 // has a compiled slab unit; drs_plan_set_slab may come after the first use of the plan)
 int load_slab2d(drs_plan* p) {
+    const int rc = load_slabpair(p);
+    if (rc != DRS_OK) return rc;
     if (p->slab_cubin.empty() || p->smod) return DRS_OK;
     Driver& d = driver();
     CUresult r = d.ModuleLoadData(&p->smod, p->slab_cubin.data());
@@ -501,7 +535,7 @@ void fill_params(const drs_plan* p, const void* in, void* out, DevParams& q, int
     const long long slow = p->local_slow();
     if (!p->slab) { q.slow_lo = q.halo; q.slow_hi = slow - q.halo; }
     else {
-        const long long ghost = s.halo, org = p->lo - ghost;  // global index of local plane 0
+        const long long ghost = p->ghost(), org = p->lo - ghost;  // global index of local plane 0
         const long long glo = std::max<long long>(p->lo, s.halo), ghi = std::min<long long>(p->hi, p->g_slow - s.halo);
         q.slow_lo = glo - org; q.slow_hi = ghi - org;
         int b = -1;
@@ -539,9 +573,11 @@ void fill_params(const drs_plan* p, const void* in, void* out, DevParams& q, int
         q.face_cnt = (unsigned int*)((char*)p->d_sync + sizeof(long long));
         q.seq_off = seq_off;
         // a chunk [za, zb) belongs to a face when it reads that neighbour's ghost planes (rows in 2D) or produces
-        // planes that are pushed to it; its input reaches Halo planes beyond its outputs on both sides.  The chunks are
-        // the nzs plane chunks in 3D, the nys row chunks in 2D (one unit = one warp, nxs of them per row chunk).
-        const long long ghost = s.halo, local = p->local_slow();
+        // planes that are pushed to it.  The pushed planes are the `ghost` owned planes next to the face, and the input
+        // reaches at most `ghost` planes beyond the outputs (Halo for a single sweep; 2 * Halo for a pair launch, which
+        // only runs on slabs with ghost = 2 * Halo), so both fall below 2 * ghost.  The chunks are the nzs plane chunks
+        // in 3D, the nys row chunks in 2D (one unit = one warp, nxs of them per row chunk).
+        const long long ghost = p->ghost(), local = p->local_slow();
         q.face_lo_end = 2 * ghost;
         q.face_hi_begin = local - 2 * ghost;
         const long long units_per_chunk = s.dim == 2 ? (long long)q.nxs
@@ -672,6 +708,40 @@ int launch_pair(drs_plan* p, const void* in, void* out, const void* a, const voi
     CUresult r = driver().LaunchKernel(p->f_pair, (unsigned)tiles, 1, 1, (unsigned)(p->pspec.nw * 32), 1, 1,
                                        (unsigned)p->pspec.smem_bytes(), (CUstream)stream, args, nullptr);
     if (r != CUDA_SUCCESS) return fail(DRS_E_CUDA, "launch drpair_: " + cu_err(r));
+    p->launches++;
+    return DRS_OK;
+}
+
+// One pair launch of a pair slab (kernels/slabpair/drs_slabpair3d.cuh): the pair of sweeps of drs_run_slab's launch
+// `seq_off` (< 0: no step flags), from the level in `in` to the level two steps later on the owned output planes of
+// `out`, pushed to the neighbours' deep ghost planes.  Level 0's global ring is A's (my_bases[0]), level 1's is B's.
+int launch_slabpair(drs_plan* p, const void* in, void* out, cudaStream_t stream, int seq_off) {
+    if (in == out) return fail(DRS_E_ARG, "d_in and d_out must differ");
+    if (!p->f_slabpair) return fail(DRS_E_ARG, "this plan has no slab pair kernel");
+    const void* a = p->my_bases[0];
+    CUtensorMap* tm = nullptr;
+    int rc = tensor_map_for(p, in, &tm, true);
+    if (rc != DRS_OK) return rc;
+    CUtensorMap map_in = *tm;          // (the next lookup may clear the cache)
+    rc = tensor_map_for(p, a, &tm, true);
+    if (rc != DRS_OK) return rc;
+    CUtensorMap map_a = *tm;
+    if ((reinterpret_cast<uintptr_t>(out) & 15) != 0) return fail(DRS_E_ARG, "device buffers must be 16-byte aligned");
+    DevParams q;
+    fill_params(p, in, out, q, -1, nullptr, seq_off, &p->pspec);
+    const long long tiles = (long long)q.nxs * q.nys * q.nzs;
+    if (tiles <= 0) return DRS_OK;
+    if (tiles > 0x7fffffffLL) return fail(DRS_E_ARG, "grid too large");
+    const void* ring_a = a;
+    const void* ring_b = p->my_bases[1];
+    // the global ring planes [0, Halo) and [G - Halo, G) in local coordinates, clamped to the array
+    const long long org = p->lo - p->ghost(), H = p->spec.halo, L = p->st.L;
+    int ring_lo = (int)std::min(L, std::max(0LL, H - org));
+    int ring_hi = (int)std::min(L, std::max(0LL, p->g_slow - H - org));
+    void* args[] = {&map_in, &map_a, &q, &ring_a, &ring_b, &ring_lo, &ring_hi};
+    CUresult r = driver().LaunchKernel(p->f_slabpair, (unsigned)tiles, 1, 1, (unsigned)(p->pspec.nw * 32), 1, 1,
+                                       (unsigned)p->pspec.smem_bytes(), (CUstream)stream, args, nullptr);
+    if (r != CUDA_SUCCESS) return fail(DRS_E_CUDA, "launch drslabpair_: " + cu_err(r));
     p->launches++;
     return DRS_OK;
 }
@@ -876,6 +946,7 @@ void drs_plan_destroy(drs_plan* p) {
         if (p->mod) driver().ModuleUnload(p->mod);
         if (p->pmod) driver().ModuleUnload(p->pmod);
         if (p->smod) driver().ModuleUnload(p->smod);
+        if (p->spmod) driver().ModuleUnload(p->spmod);
     }
     delete p;
 }
@@ -920,6 +991,8 @@ const char* drs_plan_pair_source(const drs_plan* p) { return p ? p->pair_source.
 const char* drs_plan_pair_cache_key(const drs_plan* p) { return p ? p->pair_key.c_str() : ""; }
 const char* drs_plan_slab_source(const drs_plan* p) { return p ? p->slab_source.c_str() : ""; }
 const char* drs_plan_slab_cache_key(const drs_plan* p) { return p ? p->slab_key.c_str() : ""; }
+const char* drs_plan_slab_pair_source(const drs_plan* p) { return p ? p->slabpair_source.c_str() : ""; }
+const char* drs_plan_slab_pair_cache_key(const drs_plan* p) { return p ? p->slabpair_key.c_str() : ""; }
 
 int drs_sweep(drs_plan* p, const void* d_in, void* d_out, void* stream) {
     if (!p || !d_in || !d_out) return fail(DRS_E_ARG, "null argument");
@@ -959,10 +1032,11 @@ static bool run_graph(drs_plan* p, void* a, void* b, int n, bool slab, cudaStrea
             cudaGetLastError(); p->use_graph = false; return false;
         }
         // tensor maps are encoded outside the capture (host-only, but keeps the captured region to launches);
-        // only drs_run's sequence has pair launches
+        // pair launches run in drs_run's sequence on plain plans and in drs_run_slab's on pair slabs
         CUtensorMap* tm = nullptr;
         if (tensor_map_for(p, a, &tm) != DRS_OK || tensor_map_for(p, b, &tm) != DRS_OK) return false;
-        if (uses_pairs(p) && !slab && (tensor_map_for(p, a, &tm, true) != DRS_OK || tensor_map_for(p, b, &tm, true) != DRS_OK)) return false;
+        if ((slab ? p->slab_pairs : uses_pairs(p)) &&
+            (tensor_map_for(p, a, &tm, true) != DRS_OK || tensor_map_for(p, b, &tm, true) != DRS_OK)) return false;
         const long long l0 = p->launches;
         if (cudaStreamBeginCapture(p->cap_stream, cudaStreamCaptureModeThreadLocal) != cudaSuccess) {
             cudaGetLastError(); p->use_graph = false; return false;
@@ -1225,6 +1299,7 @@ int drs_run_host(drs_plan* p, void* h_a, void* h_b, int iterations, float* devic
 int drs_plan_slab_schedule(const drs_plan* p, int iterations, int up_skew, long long* records6, int capacity) {
     if (!p) return fail(DRS_E_ARG, "null plan");
     if (!p->slab) return fail(DRS_E_ARG, "call drs_plan_set_slab first");
+    if (p->slab_pairs) return fail(DRS_E_ARG, "a pair slab (deep ghost planes) has no streamed host schedule");
     return step_records(slab_steps(p, sweeps_for(p, iterations), up_skew != 0), records6, 6, capacity);
 }
 
@@ -1282,9 +1357,58 @@ int drs_plan_set_slab(drs_plan* p, long long global_slow, long long lo, long lon
         if (rc != DRS_OK) return rc;
         p->slab_source = std::move(src); p->slab_key = std::move(key); p->slab_cubin = std::move(cubin);
     }
-    p->slab = true; p->g_slow = global_slow; p->lo = lo; p->hi = hi;
+    p->slab = true; p->slab_pairs = false; p->g_slow = global_slow; p->lo = lo; p->hi = hi;
     drop_graphs(p);      // launch parameters changed
     return DRS_OK;
+}
+
+int drs_plan_set_slab_pairs(drs_plan* p, long long global_slow, long long lo, long long hi) {
+    if (!p) return fail(DRS_E_ARG, "null plan");
+    const drs::KernelSpec& s = p->spec;
+    if (p->slab) return fail(DRS_E_ARG, "this plan is already a slab");
+    if (s.dim != 3) return fail(DRS_E_ARG, "pair slabs are 3D only");
+    if (s.step != 1 || s.ts != 1 || s.sub_launches > 1) return fail(DRS_E_ARG, "pair slabs need a step-1 plan (two single steps per launch)");
+    if (s.reuse) return fail(DRS_E_ARG, "--fuse reuse has no fused halo push: use --fuse temporal or algebraic on a slab");
+    if (!drs::fused3d_fits(s.e, s.vec(), 2)) return fail(DRS_E_ARG, "the operator's depth-2 tile keeps no useful columns");
+    if (!s.tma_ok)
+        return fail(DRS_E_ARG, "this plan runs the naive kernel (operator too deep for the TMA ring), which has no fused halo push");
+    if (s.flat) return fail(DRS_E_ARG, "the pair kernel needs a 16-byte row pitch (N a multiple of 2 in fp64, 4 in fp32)");
+    if (lo < 0 || hi <= lo || hi > global_slow) return fail(DRS_E_ARG, "bad slab range");
+    if (hi - lo + 4LL * s.halo != p->local_slow())
+        return fail(DRS_E_ARG, "pair slab arrays must hold hi - lo + 4*Halo planes along the slow axis");
+    drs::KernelSpec ps;
+    if (!drs::pair_spec(p->st, s, ps, false)) return fail(DRS_E_ARG, "no pair kernel for this operator's tile");
+    std::string src = drs::generate_slabpair_tu(ps), key;
+    std::vector<char> cubin;
+    const int rc = compile_cubin(src, cubin, key, Unit::SLABPAIR);
+    if (rc != DRS_OK) return rc;
+    p->pspec = ps;       // the same specialisation as drs_run's pair unit where the plan has one
+    p->ptmaps.clear();
+    p->slabpair_source = std::move(src); p->slabpair_key = std::move(key); p->slabpair_cubin = std::move(cubin);
+    p->slab = true; p->slab_pairs = true; p->g_slow = global_slow; p->lo = lo; p->hi = hi;
+    drop_graphs(p);
+    return p->loaded ? load_slabpair(p) : DRS_OK;
+}
+
+int drs_plan_slab_split(const drs_plan* p, int iterations, int* pairs, int* singles) {
+    if (!p) return fail(DRS_E_ARG, "null plan");
+    const int n = sweeps_for(p, iterations);
+    int np = 0, ns = n;
+    if (p->slab_pairs) drs::pair_split(n, np, ns);
+    if (pairs) *pairs = np;
+    if (singles) *singles = ns;
+    return n;
+}
+
+int drs_sweep_pair(drs_plan* p, const void* d_in, void* d_out, void* stream) {
+    if (!p || !d_in || !d_out) return fail(DRS_E_ARG, "null argument");
+    if (!p->slab_pairs || !p->my_bases[0] || !p->my_bases[1])
+        return fail(DRS_E_ARG, "call drs_plan_set_slab_pairs and drs_plan_set_peers first");
+    if (!((d_in == p->my_bases[0] && d_out == p->my_bases[1]) || (d_in == p->my_bases[1] && d_out == p->my_bases[0])))
+        return fail(DRS_E_ARG, "a pair launch runs between the two arrays given to drs_plan_set_peers");
+    int rc = ensure_loaded(p);
+    if (rc != DRS_OK) return rc;
+    return launch_slabpair(p, d_in, d_out, (cudaStream_t)stream, -1);
 }
 
 int drs_plan_set_peers(drs_plan* p, void* const my_bases[2], void* const lower_bases[2], void* const upper_bases[2],
@@ -1352,7 +1476,10 @@ int drs_run_slab(drs_plan* p, int iterations, void* stream_, int* sweeps) {
     const int n = sweeps_for(p, iterations);
     if (sweeps) *sweeps = n;
     if (n == 0) return DRS_OK;
-    // flag value of this call's sweep 0, in stream order (no kernel)
+    // pair slabs: `pairs` pair launches, then `singles` single sweeps; flag values count launches
+    int pairs = 0, singles = n;
+    if (p->slab_pairs) drs::pair_split(n, pairs, singles);
+    // flag value of this call's launch 0, in stream order (no kernel)
     const long long base = p->slab_seq;
     if (driver().StreamWriteValue64) {
         CUresult r = driver().StreamWriteValue64((CUstream)stream, (CUdeviceptr)p->d_sync, (cuuint64_t)base, 0);
@@ -1364,12 +1491,14 @@ int drs_run_slab(drs_plan* p, int iterations, void* stream_, int* sweeps) {
     void* b = p->my_bases[1];
     auto enqueue = [&](cudaStream_t st) -> int {
         int r = DRS_OK;
-        for (int s = 0; s < n && r == DRS_OK; ++s)
-            r = (s & 1) ? launch_one(p, b, a, st, -1, nullptr, s) : launch_one(p, a, b, st, -1, nullptr, s);
+        for (int i = 0; i < pairs && r == DRS_OK; ++i)
+            r = (i & 1) ? launch_slabpair(p, b, a, st, i) : launch_slabpair(p, a, b, st, i);
+        for (int s = 0; s < singles && r == DRS_OK; ++s)
+            r = (s & 1) ? launch_one(p, b, a, st, -1, nullptr, pairs + s) : launch_one(p, a, b, st, -1, nullptr, pairs + s);
         return r;
     };
     if (!run_graph(p, a, b, n, true, stream, enqueue) && (rc = enqueue(stream)) != DRS_OK) return rc;
-    p->slab_seq += n;
+    p->slab_seq += pairs + singles;
     return DRS_OK;
 }
 
@@ -1382,6 +1511,7 @@ int drs_run_host_slab(drs_plan* p, void* h_own, int iterations, int up_skew, flo
     if (!p || !h_own) return fail(DRS_E_ARG, "null argument");
     if (!p->slab || !p->my_bases[0] || !p->my_bases[1]) return fail(DRS_E_ARG, "call drs_plan_set_slab and drs_plan_set_peers first");
     if (!p->my_flags) return fail(DRS_E_ARG, "call drs_plan_set_flags first");
+    if (p->slab_pairs) return fail(DRS_E_ARG, "a pair slab (deep ghost planes) has no streamed host run");
     int rc = ensure_loaded(p);
     if (rc != DRS_OK) return rc;
     const int n = sweeps_for(p, iterations);

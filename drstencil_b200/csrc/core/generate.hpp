@@ -632,10 +632,12 @@ inline std::string generate_tu(const KernelSpec& s, bool slab2d = false) {
 // The specialisation of the pair kernel for a plan whose main specialisation is `m`, or false where the plan keeps one
 // launch per sweep: 3D, step 1, the single-step TMA sweep with a 16-byte row pitch, arrays of >= 1 GiB, and an operator
 // whose depth-2 tile keeps useful columns.  The geometry is that of the fused temporal kernel at depth 2 (8 warps x 4
-// rows, two CTAs per SM, chunks of 128 planes); the ring is that of one step.
-inline bool pair_spec(const Stencil& st, const KernelSpec& m, KernelSpec& s) {
+// rows, two CTAs per SM, chunks of 128 planes); the ring is that of one step.  size_gate = false drops the 1 GiB rule:
+// the slab pair launches (drs_plan_set_slab_pairs) must not depend on a rank's local size, or uneven splits would give
+// the ranks different launch sequences.
+inline bool pair_spec(const Stencil& st, const KernelSpec& m, KernelSpec& s, bool size_gate = true) {
     if (m.dim != 3 || m.step != 1 || m.ts != 1 || m.flat || m.reuse || !m.tma_ok || m.sub_launches != 1) return false;
-    if (!far_beyond_l2(st, m.dtype) || !fused3d_fits(m.e, m.vec(), 2)) return false;
+    if ((size_gate && !far_beyond_l2(st, m.dtype)) || !fused3d_fits(m.e, m.vec(), 2)) return false;
     s = KernelSpec();
     s.dim = 3; s.dtype = m.dtype; s.step = 1; s.fuse = m.fuse; s.ts = 2;
     s.halo = m.halo; s.base_order = m.base_order;
@@ -704,6 +706,25 @@ inline std::string generate_pair_tu(const KernelSpec& s) {
     if (s.keep_planes) o << "#ifndef DRS_LD_HINT\n#define DRS_LD_HINT 1\n#endif\n";
     emit_scatter3_exact(o, s);
     o << "#include \"drs_pair3d.cuh\"\n";
+    return o.str();
+}
+
+// ---- slab pair launches (drs_run_slab on slabs with deep ghost regions; kernels/slabpair/drs_slabpair3d.cuh) ---------
+
+// The slab entry of the pair kernel: the pair unit's specialisation (pair_spec), its own name and header.
+inline std::string generate_slabpair_tu(const KernelSpec& s) {
+    std::ostringstream o;
+    o << "// generated by drstencil-b200 for sm_100a -- stencil '" << s.name << "', 3D, " << (s.dtype == DRS_F64 ? "fp64" : "fp32")
+      << ", two exact single steps per launch, slab entry\n";
+    o << "#define DRS_DIM 3\n";
+    o << "#define DRS_T " << (s.dtype == DRS_F64 ? "double" : "float") << "\n";
+    o << "#define DRS_SLABPAIR_NAME drslabpair_" << s.name << "\n";
+    o << "#define DRS_HALO " << s.halo << "\n";
+    o << "#define DRS_RK " << s.rk << "\n#define DRS_RJ " << s.rj << "\n#define DRS_E " << s.e << "\n";
+    o << "#define DRS_NW " << s.nw << "\n#define DRS_ST " << s.st << "\n#define DRS_RY " << s.ry << "\n#define DRS_MINB " << s.minb << "\n";
+    if (s.keep_planes) o << "#ifndef DRS_LD_HINT\n#define DRS_LD_HINT 1\n#endif\n";
+    emit_scatter3_exact(o, s);
+    o << "#include \"drs_slabpair3d.cuh\"\n";
     return o.str();
 }
 

@@ -16,6 +16,10 @@ Exchange paths (`halo=`):
                per sweep, driven from Python) -- round 1's protocol, kept for A/B measurements.
   "nccl"       plain torch.distributed isend/irecv of the boundary planes after each sweep (NCCL on GPUs,
                gloo on CPU -- the path the CPU tests drive with a stand-in sweep).
+
+Pair slabs (`GpuSlab(..., pairs=True)`, 3D step-1 plans, "p2p" only): the ghost regions are 2 * Halo planes deep and
+drs_run_slab runs the sweeps as exact pair launches (two sweeps per launch, one double-depth halo exchange) plus two or
+four single sweeps (drs_plan_set_slab_pairs).
 """
 from __future__ import annotations
 
@@ -35,9 +39,12 @@ class SlabGeometry:
     g_slow: int      # global planes
     world: int
     rank: int
-    ghost: int       # Halo = step * order: ghost planes per side
+    ghost: int       # Halo = step * order: ghost planes per side (2 * Halo on pair slabs)
+    ring: Optional[int] = None   # width of the global frozen ring (default: ghost)
 
     def __post_init__(self):
+        if self.ring is None:
+            self.ring = self.ghost
         b = split(self.g_slow, self.world)
         self.bounds = b
         self.lo, self.hi = b[self.rank]
@@ -49,8 +56,8 @@ class SlabGeometry:
         self.lower = self.rank - 1 if self.rank > 0 else None
         self.upper = self.rank + 1 if self.rank + 1 < self.world else None
         # output range in local indices (the global ring stays frozen)
-        self.out_lo = max(self.lo, self.ghost) - self.origin
-        self.out_hi = min(self.hi, self.g_slow - self.ghost) - self.origin
+        self.out_lo = max(self.lo, self.ring) - self.origin
+        self.out_hi = min(self.hi, self.g_slow - self.ring) - self.origin
 
     def local(self, g: int) -> int:
         return g - self.origin
@@ -163,11 +170,13 @@ class GpuSlab:
     """One rank's share of a slab-decomposed run on its GPU."""
 
     def __init__(self, stc_path: str, knobs, rank: int, world: int, halo: str = "p2p", group=None,
-                 global_shape=None):
+                 global_shape=None, pairs: bool = False):
         import torch
         import torch.distributed as dist
         from . import Plan, Stencil, F32
-        self.rank, self.world, self.mode, self.group = rank, world, halo, group
+        if pairs and halo != "p2p":
+            raise ValueError("pair slabs need the p2p halo mode (drs_run_slab), not %r" % halo)
+        self.rank, self.world, self.mode, self.group, self.pairs = rank, world, halo, group, pairs
         st = Stencil.from_file(stc_path)
         if global_shape is not None:
             st.set_size(global_shape)
@@ -176,11 +185,14 @@ class GpuSlab:
         probe = Plan(st, knobs)                      # halo of the (possibly multi-step) sweep
         ghost = probe.halo
         self.step = knobs.step
-        self.geom = SlabGeometry(slow, world, rank, ghost)
+        self.geom = SlabGeometry(slow, world, rank, 2 * ghost if pairs else ghost, ring=ghost)
         shape = (self.geom.local_planes,) + rest
         st.set_size(shape)
         self.plan = Plan(st, knobs)
-        self.plan.set_slab(slow, self.geom.lo, self.geom.hi)
+        if pairs:
+            self.plan.set_slab_pairs(slow, self.geom.lo, self.geom.hi)
+        else:
+            self.plan.set_slab(slow, self.geom.lo, self.geom.hi)
         self.dtype = torch.float32 if knobs.dtype == F32 else torch.float64
         typestr, isz = ("<f4", 4) if knobs.dtype == F32 else ("<f8", 8)
         self._raw = [_DevArray(shape, typestr, isz), _DevArray(shape, typestr, isz)]
@@ -273,6 +285,8 @@ class GpuSlab:
         import torch.distributed as dist
         if self.mode != "p2p" or self.world < 2:
             raise ValueError("run_host needs the p2p halo mode and at least two ranks (one GPU: Plan.run_host)")
+        if self.pairs:
+            raise ValueError("run_host has no pair schedule: use a GpuSlab with pairs=False")
         self.plan.sync_check()
         torch.cuda.synchronize()
         dist.barrier(group=self.group)               # nobody still reads ghosts of the previous call

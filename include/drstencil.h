@@ -137,6 +137,10 @@ const char *drs_plan_pair_cache_key(const drs_plan *p);
  * needed) by drs_plan_set_slab; "" for every other plan (3D plans carry drslab_ in their main unit) */
 const char *drs_plan_slab_source(const drs_plan *p);
 const char *drs_plan_slab_cache_key(const drs_plan *p);
+/* the translation unit / cache key of the slab pair entry drslabpair_<name>, generated and compiled (NVRTC, no GPU
+ * needed) by drs_plan_set_slab_pairs; "" for every other plan */
+const char *drs_plan_slab_pair_source(const drs_plan *p);
+const char *drs_plan_slab_pair_cache_key(const drs_plan *p);
 
 /* one `dr_<name><<<grid, block>>>(d_in, d_out)` (codegen_2d.hpp:606): advances the interior
  * [Halo, dim-Halo) by `step` timesteps; the Halo ring of d_out is not written.  d_in != d_out.
@@ -150,8 +154,8 @@ int drs_gold_sweep(drs_plan *p, const void *d_in, void *d_out, void *stream);
  * On 3D step-1 plans whose arrays are >= 1 GiB each (16-byte row pitch, an operator the depth-2 tile fits) the
  * sweeps run as exact pair launches -- one kernel computes two sweeps, bit for bit, with each level's ring taken from
  * the buffer that level lives in -- followed by two or four single sweeps; A and B end exactly as after the plain
- * loop (drs_plan_pair_split).  A slab plan (drs_plan_set_slab) never gets pair launches: its drs_run is the loop of
- * drs_sweep, boundary planes pushed to the neighbours' ghost planes and no step flags. */
+ * loop (drs_plan_pair_split).  drs_run on a slab plan (drs_plan_set_slab, drs_plan_set_slab_pairs) never makes pair
+ * launches: it is the loop of drs_sweep, boundary planes pushed to the neighbours' ghost planes and no step flags. */
 int drs_run(drs_plan *p, void *d_a, void *d_b, int iterations, void *stream, int *sweeps);
 /* how drs_run splits the sweeps of `iterations` timesteps: *pairs pair launches, then *singles single sweeps
  * (*pairs = 0 on plans without pair launches, slab plans included); returns the number of sweeps.  Needs no GPU. */
@@ -205,6 +209,23 @@ long long drs_plan_launch_count(const drs_plan *p);
  * global faces.  Must be called before the first sweep.  On a 2D plan with the TMA sweep this generates and
  * compiles the slab unit (drs_plan_slab_source). */
 int drs_plan_set_slab(drs_plan *p, long long global_slow, long long lo, long long hi);
+/* Like drs_plan_set_slab, for a PAIR slab: the ghost regions are 2*Halo planes deep, i.e. the local array holds
+ * (hi - lo + 4*Halo) planes, and drs_run_slab runs the sweeps as exact pair launches (two sweeps per launch, bit for
+ * bit) followed by two or four single sweeps (drs_plan_slab_split), each pair launch exchanging one double-depth halo.
+ * Every single sweep (drs_sweep, drs_run) pushes 2*Halo planes.  Generates and compiles the slab pair unit
+ * (drs_plan_slab_pair_source).  DRS_E_ARG for 2D plans, step > 1 or per-sub-step launches, an unaligned row pitch,
+ * `--fuse reuse`, the naive kernel, operators whose depth-2 tile keeps no useful columns, a wrong local size and a
+ * plan that is already a slab.  drs_run_host_slab and drs_plan_slab_schedule refuse pair slabs. */
+int drs_plan_set_slab_pairs(drs_plan *p, long long global_slow, long long lo, long long hi);
+/* how drs_run_slab splits the sweeps of `iterations` timesteps: *pairs pair launches, then *singles single sweeps
+ * (*pairs = 0 except on pair slabs); the split depends on the sweep count only, so every rank runs the same launch
+ * sequence.  Returns the number of sweeps.  Needs no GPU. */
+int drs_plan_slab_split(const drs_plan *p, int iterations, int *pairs, int *singles);
+/* One pair launch on a pair slab whose peers are set (the pair counterpart of drs_sweep): the level in d_in advanced
+ * by two sweeps on the owned planes of d_out, the 2*Halo boundary planes pushed to the neighbours' deep ghost planes;
+ * no step flags.  d_in and d_out are the two arrays given to drs_plan_set_peers; level 0's global ring is taken from
+ * the first, level 1's from the second, as in drs_run_slab. */
+int drs_sweep_pair(drs_plan *p, const void *d_in, void *d_out, void *stream);
 /* Fused halo push: while sweeping into my_bases[b], the kernel stores its boundary planes (3D) / rows (2D) a
  * second time, straight into the neighbours' ghost planes / rows over NVLink.  lower_bases / upper_bases
  * are the *neighbours' array bases* (same ping-pong order, mapped into this process with
@@ -228,7 +249,9 @@ int drs_plan_set_flags(drs_plan *p, const void *my_flags, void *lower_flag, void
  * tile of a face releases the next flag value (st.release.sys); boundary tiles are scheduled first, so the
  * signal leaves early and the next sweep does not wait.  Every rank must call it with the same `iterations`;
  * after new data was written into the arrays (ghost planes included) the ranks must pass a barrier of the
- * caller's before the next call.  Writes the number of sweeps to *sweeps. */
+ * caller's before the next call.  Writes the number of sweeps to *sweeps.  On a pair slab (drs_plan_set_slab_pairs)
+ * the sweeps run as drs_plan_slab_split's pair launches and single sweeps, one launch each, and the flag values count
+ * launches instead of sweeps. */
 int drs_run_slab(drs_plan *p, int iterations, void *stream, int *sweeps);
 /* This rank's share of a slab-decomposed HOST-buffer run (the executor of drs_plan_slab_schedule): h_own = the
  * rank's own planes (rows in 2D; pinned for overlap), result written back in place; uploads, sweeps and downloads overlap
