@@ -100,6 +100,7 @@ def lib():
         "drs_sweep_pair": (i32, [vp, vp, vp, vp]),
         "drs_plan_set_slab_pairs": (i32, [vp, ll, ll, ll]),
         "drs_plan_pair_split": (i32, [vp, i32, P(i32), P(i32)]),
+        "drs_plan_set_pairs": (i32, [vp, i32]),
         "drs_sweep": (i32, [vp, vp, vp, vp]),
         "drs_gold_sweep": (i32, [vp, vp, vp, vp]),
         "drs_run": (i32, [vp, vp, vp, i32, vp, P(i32)]),
@@ -450,6 +451,12 @@ class Plan:
         p, s = ctypes.c_int(), ctypes.c_int()
         _check(lib().drs_plan_pair_split(self._h, iterations, ctypes.byref(p), ctypes.byref(s)))
         return p.value, s.value
+
+    def set_pairs(self, enable: bool) -> None:
+        """Opt-in exact pair launches for run() and the plain run_host(): on 2D plans the 2D pair unit, on 3D plans the
+        pair unit without its 1 GiB rule (see drs_plan_set_pairs in drstencil.h).  False restores the default rule.
+        Raises DrsError (E_ARG, with the reason) for plans that have no pair kernel and for slab plans."""
+        _check(lib().drs_plan_set_pairs(self._h, 1 if enable else 0))
 
     @property
     def halo(self) -> int:

@@ -41,6 +41,9 @@ extern const int drs_slab2d_header_count;
 extern const char* const drs_slabpair_header_names[];
 extern const char* const drs_slabpair_header_texts[];
 extern const int drs_slabpair_header_count;
+extern const char* const drs_pair2d_header_names[];
+extern const char* const drs_pair2d_header_texts[];
+extern const int drs_pair2d_header_count;
 
 namespace {
 
@@ -194,8 +197,9 @@ const char* kNvrtcOpts[] = {"--gpu-architecture=sm_100a", "-std=c++17", "-linein
                             "-default-device", "--ptxas-options=-v"};
 
 // Which unit compile_cubin builds: the plan's main unit, the exact pair kernel's (kernels/pair/ headers), the 2D slab
-// entry's (kernels/slab2d/ headers) or the slab entry of the pair kernel (kernels/slabpair/ headers).
-enum class Unit { MAIN, PAIR, SLAB2D, SLABPAIR };
+// entry's (kernels/slab2d/ headers), the slab entry of the pair kernel (kernels/slabpair/ headers) or the 2D pair
+// kernel's (kernels/pair2d/ headers).
+enum class Unit { MAIN, PAIR, SLAB2D, SLABPAIR, PAIR2D };
 
 // source -> cubin, through the on-disk cache.  The key covers the source, every header the unit may include and the
 // options.  The pair and slab units may include their own subdirectory's headers as well; those are part of their
@@ -212,6 +216,9 @@ int compile_cubin(const std::string& src, std::vector<char>& cubin, std::string&
     } else if (unit == Unit::SLABPAIR) {
         names.insert(names.end(), drs_slabpair_header_names, drs_slabpair_header_names + drs_slabpair_header_count);
         texts.insert(texts.end(), drs_slabpair_header_texts, drs_slabpair_header_texts + drs_slabpair_header_count);
+    } else if (unit == Unit::PAIR2D) {
+        names.insert(names.end(), drs_pair2d_header_names, drs_pair2d_header_names + drs_pair2d_header_count);
+        texts.insert(texts.end(), drs_pair2d_header_texts, drs_pair2d_header_texts + drs_pair2d_header_count);
     }
     std::string all = src;
     for (const char* t : texts) all += t;
@@ -302,12 +309,14 @@ struct drs_plan {
     drs::KernelSpec spec;
     std::string source, cache_key;
     std::vector<char> cubin;
-    // exact pair launches of drs_run (generate.hpp: pair_spec): their own unit, cubin, module and tensor maps
+    // exact pair launches of drs_run (generate.hpp: pair_spec, and pair_spec2d after drs_plan_set_pairs): their own
+    // unit, cubin, module and tensor maps.  Every pair module loaded stays loaded, by cache key, until the plan is
+    // destroyed: drs_plan_set_pairs may switch units while launches from the previous one are still queued.
     bool pair = false;
     drs::KernelSpec pspec;
     std::string pair_source, pair_key;
     std::vector<char> pair_cubin;
-    CUmodule pmod = nullptr;
+    std::map<std::string, std::pair<CUmodule, CUfunction>> pmods;
     CUfunction f_pair = nullptr;
     std::map<const void*, CUtensorMap> ptmaps;
     // 2D slab plans (generate.hpp: has_slab2d_unit): the unit of drslab_, generated and compiled by drs_plan_set_slab, its
@@ -404,6 +413,28 @@ int load_slab2d(drs_plan* p) {
     return DRS_OK;
 }
 
+// The current pair unit's module and drpair_ (once the plan is loaded), from pmods when it was loaded before
+int load_pair(drs_plan* p) {
+    if (!p->pair) { p->f_pair = nullptr; return DRS_OK; }
+    auto it = p->pmods.find(p->pair_key);
+    if (it == p->pmods.end()) {
+        Driver& d = driver();
+        CUmodule m = nullptr;
+        CUfunction f = nullptr;
+        CUresult r = d.ModuleLoadData(&m, p->pair_cubin.data());
+        if (r != CUDA_SUCCESS) return fail(DRS_E_CUDA, "cuModuleLoadData(pair): " + cu_err(r));
+        r = d.ModuleGetFunction(&f, m, ("drpair_" + p->spec.name).c_str());
+        if (r == CUDA_SUCCESS) r = d.FuncSetAttribute(f, CU_FUNC_ATTRIBUTE_MAX_DYNAMIC_SHARED_SIZE_BYTES, p->pspec.smem_bytes());
+        if (r != CUDA_SUCCESS) {
+            d.ModuleUnload(m);
+            return fail(DRS_E_CUDA, "cuModuleGetFunction(drpair_): " + cu_err(r));
+        }
+        it = p->pmods.emplace(p->pair_key, std::make_pair(m, f)).first;
+    }
+    p->f_pair = it->second.second;
+    return DRS_OK;
+}
+
 int ensure_loaded(drs_plan* p) {
     if (p->loaded) {
         // the module, tensor maps and scratch memory belong to the device that was current at first use
@@ -464,13 +495,8 @@ int ensure_loaded(drs_plan* p) {
     r = d.ModuleGetFunction(&p->f_signal, p->mod, ("signal_" + nm).c_str());
     if (r == CUDA_SUCCESS) r = d.ModuleGetFunction(&p->f_wait, p->mod, ("wait_" + nm).c_str());
     if (r != CUDA_SUCCESS) return fail(DRS_E_CUDA, "cuModuleGetFunction(signal_/wait_): " + cu_err(r));
-    if (p->pair) {
-        r = d.ModuleLoadData(&p->pmod, p->pair_cubin.data());
-        if (r != CUDA_SUCCESS) return fail(DRS_E_CUDA, "cuModuleLoadData(pair): " + cu_err(r));
-        r = d.ModuleGetFunction(&p->f_pair, p->pmod, ("drpair_" + nm).c_str());
-        if (r == CUDA_SUCCESS) r = d.FuncSetAttribute(p->f_pair, CU_FUNC_ATTRIBUTE_MAX_DYNAMIC_SHARED_SIZE_BYTES, p->pspec.smem_bytes());
-        if (r != CUDA_SUCCESS) return fail(DRS_E_CUDA, "cuModuleGetFunction(drpair_): " + cu_err(r));
-    }
+    const int prc = load_pair(p);
+    if (prc != DRS_OK) return prc;
     if (cudaMalloc(&p->d_fault, sizeof(int)) != cudaSuccess) return fail(DRS_E_CUDA, "cudaMalloc(fault flag)");
     cudaMemset(p->d_fault, 0, sizeof(int));
     if (cudaMalloc(&p->d_res, 2 * sizeof(double)) != cudaSuccess) return fail(DRS_E_CUDA, "cudaMalloc(result)");
@@ -684,9 +710,9 @@ int launch_one(drs_plan* p, const void* in, void* out, cudaStream_t stream, int 
     return DRS_OK;
 }
 
-// One exact pair launch (kernels/pair/drs_pair3d.cuh): two sweeps of drs_run's ping-pong schedule, from the level in
-// `in` to the level two steps later in the interior of `out`.  a / b are the run's buffers: even levels have a's ring,
-// odd ones b's.
+// One exact pair launch (kernels/pair/drs_pair3d.cuh, kernels/pair2d/drs_pair2d.cuh): two sweeps of drs_run's ping-pong
+// schedule, from the level in `in` to the level two steps later in the interior of `out`.  a / b are the run's buffers:
+// even levels have a's ring, odd ones b's.  One CTA per tile in 3D, NW warp tiles per CTA in 2D (pspec.ctas).
 int launch_pair(drs_plan* p, const void* in, void* out, const void* a, const void* b, cudaStream_t stream) {
     if (in == out) return fail(DRS_E_ARG, "d_in and d_out must differ");
     CUtensorMap* tm = nullptr;
@@ -701,11 +727,12 @@ int launch_pair(drs_plan* p, const void* in, void* out, const void* a, const voi
     fill_params(p, in, out, q, -1, nullptr, -1, &p->pspec);
     const long long tiles = (long long)q.nxs * q.nys * q.nzs;
     if (tiles <= 0) return DRS_OK;
-    if (tiles > 0x7fffffffLL) return fail(DRS_E_ARG, "grid too large");
+    const long long ctas = p->pspec.ctas(q.nxs, q.nys, q.nzs);
+    if (ctas > 0x7fffffffLL) return fail(DRS_E_ARG, "grid too large");
     const void* ring_a = a;
     const void* ring_b = b;
     void* args[] = {&map_in, &map_a, &q, &ring_a, &ring_b};
-    CUresult r = driver().LaunchKernel(p->f_pair, (unsigned)tiles, 1, 1, (unsigned)(p->pspec.nw * 32), 1, 1,
+    CUresult r = driver().LaunchKernel(p->f_pair, (unsigned)ctas, 1, 1, (unsigned)(p->pspec.nw * 32), 1, 1,
                                        (unsigned)p->pspec.smem_bytes(), (CUstream)stream, args, nullptr);
     if (r != CUDA_SUCCESS) return fail(DRS_E_CUDA, "launch drpair_: " + cu_err(r));
     p->launches++;
@@ -944,7 +971,7 @@ void drs_plan_destroy(drs_plan* p) {
         for (cudaStream_t st : {p->hs_up, p->hs_run, p->hs_dn, p->cap_stream}) if (st) cudaStreamDestroy(st);
         for (auto& g : p->graphs) cudaGraphExecDestroy(g.second.exec);
         if (p->mod) driver().ModuleUnload(p->mod);
-        if (p->pmod) driver().ModuleUnload(p->pmod);
+        for (auto& m : p->pmods) driver().ModuleUnload(m.second.first);
         if (p->smod) driver().ModuleUnload(p->smod);
         if (p->spmod) driver().ModuleUnload(p->spmod);
     }
@@ -1095,6 +1122,49 @@ int drs_plan_pair_split(const drs_plan* p, int iterations, int* pairs, int* sing
     if (pairs) *pairs = np;
     if (singles) *singles = ns;
     return n;
+}
+
+int drs_plan_set_pairs(drs_plan* p, int enable) {
+    if (!p) return fail(DRS_E_ARG, "null plan");
+    if (p->slab) return fail(DRS_E_ARG, "a slab plan has its own pair launches (drs_plan_set_slab_pairs)");
+    const drs::KernelSpec& s = p->spec;
+    drs::KernelSpec ps;
+    bool has = false;
+    std::string src;
+    if (enable) {
+        if (s.dim == 2) {
+            const std::string why = drs::pair_spec2d(p->st, s, ps);
+            if (!why.empty()) return fail(DRS_E_ARG, "no 2D pair kernel for this plan: " + why);
+            src = drs::generate_pair2d_tu(ps);
+        } else {
+            if (s.step != 1 || s.ts != 1 || s.sub_launches > 1)
+                return fail(DRS_E_ARG, "pair launches need a step-1 plan (two single steps per launch)");
+            if (s.reuse) return fail(DRS_E_ARG, "pair launches are not available with --fuse reuse");
+            if (!s.tma_ok) return fail(DRS_E_ARG, "the plan runs the naive kernel (operator too deep for the TMA sweep)");
+            if (s.flat) return fail(DRS_E_ARG, "the pair kernel needs a 16-byte row pitch (N a multiple of 2 in fp64, 4 in fp32)");
+            if (!drs::pair_spec(p->st, s, ps, false)) return fail(DRS_E_ARG, "no pair kernel for this operator's depth-2 tile");
+            src = drs::generate_pair_tu(ps);
+        }
+        has = true;
+    } else if (drs::pair_spec(p->st, s, ps)) {       // the default rule (make_plan)
+        src = drs::generate_pair_tu(ps);
+        has = true;
+    }
+    if (has == p->pair && src == p->pair_source) return DRS_OK;
+    std::string key;
+    std::vector<char> cubin;
+    if (has) {
+        const int rc = compile_cubin(src, cubin, key, s.dim == 2 ? Unit::PAIR2D : Unit::PAIR);
+        if (rc != DRS_OK) return rc;
+    }
+    drop_graphs(p);          // the graph key (A, B, sweep count, slab) does not include this setting
+    p->ptmaps.clear();       // boxes of the new unit's tile
+    p->pair = has;
+    p->pspec = has ? ps : drs::KernelSpec();
+    p->pair_source = std::move(src);
+    p->pair_key = std::move(key);
+    p->pair_cubin = std::move(cubin);
+    return p->loaded ? load_pair(p) : DRS_OK;
 }
 
 int drs_run(drs_plan* p, void* d_a, void* d_b, int iterations, void* stream, int* sweeps) {

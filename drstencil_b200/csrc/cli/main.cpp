@@ -13,7 +13,7 @@
 //   2*Halo >= bx*mx with forward_i (or, 3D, >= by*my with forward_j)  "Invalid configuration!" rc 255
 //                                                                       (codegen_2d.hpp:52-56, codegen.hpp:50-55)
 // On success it writes a CUDA program to -o (default out.cu) -- see csrc/capi/emit_program.hpp.
-// Extensions (not in the reference): --dtype, --fuse, --run, --info, --allow-no-reuse and the
+// Extensions (not in the reference): --dtype, --fuse, --run, --pairs, --info, --allow-no-reuse and the
 // engine-only tile overrides --stages --warps --min-blocks --vectors --rows-3d --rows-per-stage.
 #include <cmath>
 #include <cstdio>
@@ -59,6 +59,9 @@ Extensions:
                         forward/backward data-reuse evaluation of the composed operator (A/B mode).
 --run                   Do not emit: run the emitted program's host loop on the GPU through
                         libdrstencil.so and print the same lines.
+--pairs                 With --run: the host loop runs as exact pair launches (two bit-exact
+                        single-step sweeps per launch, drs_plan_set_pairs); an error where the plan
+                        has no pair kernel.  No effect on the emitted program.
 --info                  Print the chosen tile geometry and the reference macros (Halo Dist Range).
 --allow-no-reuse        Do not stop where the reference prints "No data to reuse".
 --stages --warps --min-blocks --vectors --rows-3d --rows-per-stage <num>   tile overrides.
@@ -82,7 +85,7 @@ int main(int argc, char** argv) {
     drs_knobs k;
     drs_knobs_default(&k);
     std::string out_name = "out.cu";
-    bool is3d = false, run = false, info = false, allow_no_reuse = false;
+    bool is3d = false, run = false, pairs = false, info = false, allow_no_reuse = false;
     struct Opt { const char* name; int* value; int bit; int reserved; };
     const Opt valued[] = {
         {"--step", &k.step, 0, -1}, {"--dist", &k.dist, 1, -1}, {"--bx", &k.bx, 3, -1}, {"--by", &k.by, 4, -1},
@@ -103,6 +106,7 @@ int main(int argc, char** argv) {
         if (a == "--check") { k.check = 1; k.explicit_mask |= 1 << 13; continue; }
         if (a == "--gold") continue;
         if (a == "--run") { run = true; continue; }
+        if (a == "--pairs") { pairs = true; continue; }
         if (a == "--info") { info = true; continue; }
         if (a == "--allow-no-reuse") { allow_no_reuse = true; continue; }
         if (a == "--share-x" || a == "--share-y") {      // CTA-shared ring (drstencil.h, reserved[6])
@@ -190,6 +194,7 @@ int main(int argc, char** argv) {
         drs_stencil_size(st, dims, &iterations);
         drs_plan* p = nullptr;
         if (drs_plan_create(st, &k, &p) != DRS_OK) { std::cout << drs_last_error() << std::endl; exit(-1); }
+        if (pairs && drs_plan_set_pairs(p, 1) != DRS_OK) { std::cout << drs_last_error() << std::endl; exit(-1); }
         puts("Initiating ...");
         const size_t count = (size_t)dims[0] * dims[1] * dims[2];
         const size_t es = k.dtype == DRS_F64 ? 8 : 4;

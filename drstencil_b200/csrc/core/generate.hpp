@@ -709,6 +709,97 @@ inline std::string generate_pair_tu(const KernelSpec& s) {
     return o.str();
 }
 
+// ---- exact pair launches on 2D plans (drs_run after drs_plan_set_pairs; kernels/pair2d/drs_pair2d.cuh) --------------
+
+// The specialisation of the 2D pair kernel for a plan whose main specialisation is `m`.  Returns "" and fills `s`, or
+// the reason the plan has no 2D pair kernel: 2D, step 1 (no sub-step launches), the TMA sweep (not the naive kernel)
+// and not `--fuse reuse`, a 16-byte row pitch, and an operator whose depth-2 strip keeps useful columns within a
+// 256-element TMA box and whose x extent one lane's shuffle reaches.  The geometry is what choose_spec picks for the
+// same stencil and dtype at step 2 (the c1t2 / c3t2 shapes), with the ring of one step.
+inline std::string pair_spec2d(const Stencil& st, const KernelSpec& m, KernelSpec& s) {
+    if (m.dim != 2) return "not a 2D plan";
+    if (m.step != 1 || m.ts != 1 || m.sub_launches != 1) return "pair launches need a step-1 plan (two single steps per launch)";
+    if (m.reuse) return "pair launches are not available with --fuse reuse";
+    if (!m.tma_ok) return "the plan runs the naive kernel (operator too deep for the TMA sweep)";
+    if (m.flat) return "the pair kernel needs a 16-byte row pitch (N a multiple of 2 in fp64, 4 in fp32)";
+    // default knobs (drs_knobs_default) at step 2; fuse given explicitly: the depth-2 geometry even where the composed
+    // operator's literals would lose digits (the pair kernel evaluates the single-step chain, not the composed one)
+    drs_knobs k = {};
+    k.step = 2; k.dtype = m.dtype; k.fuse = DRS_FUSE_TEMPORAL;
+    k.bx = k.by = k.sn = 16; k.stream_unroll = 4; k.merge_forward = 5;
+    k.block_merge_x = k.block_merge_y = k.cyclic_merge_x = k.cyclic_merge_y = 1;
+    k.explicit_mask = 1u << KB_FUSE;
+    KernelSpec t;
+    t.name = m.name;
+    const std::string err = choose_spec(st, k, t);
+    if (!err.empty()) return err;
+    const char* too_wide = "the operator's x extent is beyond what one lane's shuffle reaches at depth 2";
+    if (t.ts != 2) return t.note.find("x extent") != std::string::npos ? too_wide : "the depth-2 strip keeps no useful columns";
+    if (t.e > t.cols()) return too_wide;
+    if (t.wu() < t.vec() || t.wb() > 256 || t.flat || !t.tma_ok) return "the depth-2 strip keeps no useful columns within a 256-element TMA box";
+    s = KernelSpec();
+    s.dim = 2; s.dtype = m.dtype; s.step = 1; s.fuse = m.fuse; s.ts = 2;
+    s.halo = m.halo; s.base_order = m.base_order;
+    s.rk = 0; s.rj = m.rj; s.e = m.e;
+    s.chain = m.chain; s.gold = m.gold;
+    s.name = m.name;
+    s.nw = t.nw; s.st = t.st; s.rb = t.rb; s.vt = t.vt; s.chunk = t.chunk;
+    // choose_spec's register budget at depth 2 plus the row of ring cells loaded one iteration ahead (drs_pair2d.cuh)
+    const int live = (2 * (2 * s.rj + 1) * s.cols() + 2 * (s.cols() + 2 * s.e) + s.cols()) * (s.esize() / 4);
+    const int est = std::min(255, live + 56);
+    s.minb = std::max(1, std::min(32 / s.nw, 65536 / (est * s.nw * 32)));
+    const long long slow_out = std::max<long long>(1, st.M - 2 * s.halo);
+    if (s.chunk > slow_out) s.chunk = (int)slow_out;
+    return "";
+}
+
+// Exact 2D scatter (drs_pair2d.cuh): emit_scatter3_exact with dj in place of dk.  P(dj) is the partial sum of the output
+// row that sees the source row at offset dj, U(di) the source row at column offset di.  Every output receives its terms
+// in DRS_CHAIN's order (MUL t1, FMA t0, FMA t2, ... -- gold order ascends in dj, so row arrival order follows it) with
+// DRS_CHAIN's literals; when t0 lies on an earlier row than t1 (every star operator), t0's operand is parked in the
+// output's own partial-sum slot until t1's row arrives.
+inline void emit_scatter2_exact(std::ostringstream& o, const KernelSpec& s) {
+    const std::vector<Term>& t = s.chain;
+    auto U = [](const Term& x) { return "U(" + std::to_string(x.di) + ")"; };
+    auto C = [](const Term& x) { return "(real)(" + coef_literal_text(x.coef) + ")"; };
+    o << "#define DRS_SCATTER(P, U)";
+    for (int dj = -s.rj; dj <= s.rj; ++dj) {
+        const std::string P = "P(" + std::to_string(dj) + ")";
+        if (t.size() == 1) {
+            if (t[0].dj == dj) o << " \\\n    " << P << " = rmul(" << U(t[0]) << ", " << C(t[0]) << ");";
+            continue;
+        }
+        if (t[0].dj == dj && t[1].dj != dj) o << " \\\n    " << P << " = " << U(t[0]) << ";";
+        if (t[1].dj == dj)
+            o << " \\\n    " << P << " = rfma(" << (t[0].dj == dj ? U(t[0]) : P) << ", " << C(t[0]) << ", rmul(" << U(t[1]) << ", "
+              << C(t[1]) << "));";
+        for (size_t q = 2; q < t.size(); ++q)
+            if (t[q].dj == dj) o << " \\\n    " << P << " = rfma(" << U(t[q]) << ", " << C(t[q]) << ", " << P << ");";
+    }
+    o << "\n";
+}
+
+// The 2D pair kernel's translation unit (kernels/pair2d/drs_pair2d.cuh, which includes drs_sweep2d.cuh at depth 2 for
+// its ring and constants).  The entry point has the name of the 3D pair unit's.
+inline std::string generate_pair2d_tu(const KernelSpec& s) {
+    std::ostringstream o;
+    o << "// generated by drstencil-b200 for sm_100a -- stencil '" << s.name << "', 2D, " << (s.dtype == DRS_F64 ? "fp64" : "fp32")
+      << ", two exact single steps per launch\n";
+    o << "#define DRS_DIM 2\n";
+    o << "#define DRS_T " << (s.dtype == DRS_F64 ? "double" : "float") << "\n";
+    o << "#define DRS_PAIR_NAME drpair_" << s.name << "\n";
+    // (drs_sweep2d.cuh's own kernel, instantiated along with the shared code, is never launched)
+    o << "#define DRS_NAME unused_dr_" << s.name << "\n";
+    o << "#define DRS_HALO " << s.halo << "\n";
+    o << "#define DRS_TS 2\n";
+    o << "#define DRS_RK 0\n#define DRS_RJ " << s.rj << "\n#define DRS_E " << s.e << "\n";
+    o << "#define DRS_NW " << s.nw << "\n#define DRS_ST " << s.st << "\n#define DRS_RB " << s.rb << "\n";
+    o << "#define DRS_VT " << s.vt << "\n#define DRS_MINB " << s.minb << "\n";
+    emit_scatter2_exact(o, s);
+    o << "#include \"drs_pair2d.cuh\"\n";
+    return o.str();
+}
+
 // ---- slab pair launches (drs_run_slab on slabs with deep ghost regions; kernels/slabpair/drs_slabpair3d.cuh) ---------
 
 // The slab entry of the pair kernel: the pair unit's specialisation (pair_spec), its own name and header.

@@ -154,9 +154,22 @@ int drs_gold_sweep(drs_plan *p, const void *d_in, void *d_out, void *stream);
  * On 3D step-1 plans whose arrays are >= 1 GiB each (16-byte row pitch, an operator the depth-2 tile fits) the
  * sweeps run as exact pair launches -- one kernel computes two sweeps, bit for bit, with each level's ring taken from
  * the buffer that level lives in -- followed by two or four single sweeps; A and B end exactly as after the plain
- * loop (drs_plan_pair_split).  drs_run on a slab plan (drs_plan_set_slab, drs_plan_set_slab_pairs) never makes pair
- * launches: it is the loop of drs_sweep, boundary planes pushed to the neighbours' ghost planes and no step flags. */
+ * loop (drs_plan_pair_split).  After drs_plan_set_pairs(p, 1) the same holds for every step-1 plan that has a pair
+ * kernel, 2D plans and 3D plans below 1 GiB included.  drs_run on a slab plan (drs_plan_set_slab,
+ * drs_plan_set_slab_pairs) never makes pair launches: it is the loop of drs_sweep, boundary planes pushed to the
+ * neighbours' ghost planes and no step flags. */
 int drs_run(drs_plan *p, void *d_a, void *d_b, int iterations, void *stream, int *sweeps);
+/* Opt-in exact pair launches.  enable = 1: drs_run (direct launches and graph replay alike) and the plain
+ * copy-sweep-copy drs_run_host (h_b given, or streaming off) run the sweeps as drs_plan_pair_split's pair launches and
+ * single sweeps wherever the plan has a pair kernel: on 2D plans the 2D pair unit (kernels/pair2d/drs_pair2d.cuh),
+ * generated and compiled here (NVRTC, no GPU needed); on 3D plans the pair unit without its 1 GiB size rule (a no-op
+ * where the plan already pairs).  enable = 0 restores the default rule.  drs_plan_pair_source, drs_plan_pair_cache_key
+ * and drs_plan_pair_split follow the setting; drs_sweep, drs_gold_run, the streamed drs_run_host, the slab calls and
+ * drs_emit_program do not.  DRS_E_ARG, with the reason, for plans without a pair kernel: step > 1 or per-sub-step
+ * launches, `--fuse reuse`, the naive kernel, an unaligned row pitch, an operator whose depth-2 strip or tile keeps no
+ * useful columns or whose x extent one lane's shuffle does not reach (2D); and for slab plans, which have
+ * drs_plan_set_slab_pairs.  Drops the plan's cached drs_run graphs. */
+int drs_plan_set_pairs(drs_plan *p, int enable);
 /* how drs_run splits the sweeps of `iterations` timesteps: *pairs pair launches, then *singles single sweeps
  * (*pairs = 0 on plans without pair launches, slab plans included); returns the number of sweeps.  Needs no GPU. */
 int drs_plan_pair_split(const drs_plan *p, int iterations, int *pairs, int *singles);
