@@ -24,6 +24,7 @@ _LIBPATH = os.path.join(_HERE, "libdrstencil.so")
 F64, F32 = 0, 1
 FUSE_TEMPORAL, FUSE_ALGEBRAIC, FUSE_REUSE = 0, 1, 2
 E_ARG, E_IO, E_NOREUSE, E_CONFIG, E_COMPILE, E_CUDA, E_NOGPU, E_KERNEL = -1, -2, -3, -4, -5, -6, -7, -8
+HOST_UPLOAD, HOST_SWEEP, HOST_DOWNLOAD, HOST_PAIR = 0, 1, 2, 3     # record kinds of Plan.host_schedule
 
 
 class DrsError(RuntimeError):
@@ -453,8 +454,8 @@ class Plan:
         return p.value, s.value
 
     def set_pairs(self, enable: bool) -> None:
-        """Opt-in exact pair launches for run() and the plain run_host(): on 2D plans the 2D pair unit, on 3D plans the
-        pair unit without its 1 GiB rule (see drs_plan_set_pairs in drstencil.h).  False restores the default rule.
+        """Opt-in exact pair launches for run() and run_host(), streamed or plain: on 2D plans the 2D pair unit, on 3D
+        plans the pair unit without its 1 GiB rule (see drs_plan_set_pairs in drstencil.h).  False restores the default rule.
         Raises DrsError (E_ARG, with the reason) for plans that have no pair kernel and for slab plans."""
         _check(lib().drs_plan_set_pairs(self._h, 1 if enable else 0))
 
@@ -493,7 +494,10 @@ class Plan:
         _check(lib().drs_plan_set_graph(self._h, int(bool(enable))))
 
     def host_schedule(self, iterations: int):
-        """[(kind, block, sweep, lo, hi)] the streamed run_host would execute ([] = plain sequence); no GPU needed."""
+        """[(kind, block, launch, lo, hi)] the streamed run_host would execute ([] = plain sequence); no GPU needed.
+        kind: HOST_UPLOAD, HOST_SWEEP (one single sweep), HOST_PAIR (one exact pair launch, on plans where run() pairs)
+        or HOST_DOWNLOAD.  launch: 1-based index in run()'s launch sequence (odd: A -> B; the sweep number on plans
+        without pair launches), 0 for copies.  [lo, hi): the slow-axis planes (rows in 2D) copied or stored."""
         n = _check(lib().drs_plan_host_schedule(self._h, iterations, None, 0))
         if n == 0:
             return []

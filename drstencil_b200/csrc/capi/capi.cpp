@@ -713,7 +713,9 @@ int launch_one(drs_plan* p, const void* in, void* out, cudaStream_t stream, int 
 // One exact pair launch (kernels/pair/drs_pair3d.cuh, kernels/pair2d/drs_pair2d.cuh): two sweeps of drs_run's ping-pong
 // schedule, from the level in `in` to the level two steps later in the interior of `out`.  a / b are the run's buffers:
 // even levels have a's ring, odd ones b's.  One CTA per tile in 3D, NW warp tiles per CTA in 2D (pspec.ctas).
-int launch_pair(drs_plan* p, const void* in, void* out, const void* a, const void* b, cudaStream_t stream) {
+// sub: store only these slow-axis outputs (time-skewed blocks of drs_run_host; DESIGN 3.6 for what the chunks read).
+int launch_pair(drs_plan* p, const void* in, void* out, const void* a, const void* b, cudaStream_t stream,
+                const SlowRange* sub = nullptr) {
     if (in == out) return fail(DRS_E_ARG, "d_in and d_out must differ");
     CUtensorMap* tm = nullptr;
     int rc = tensor_map_for(p, in, &tm, true);
@@ -724,7 +726,7 @@ int launch_pair(drs_plan* p, const void* in, void* out, const void* a, const voi
     CUtensorMap map_a = *tm;
     if ((reinterpret_cast<uintptr_t>(out) & 15) != 0) return fail(DRS_E_ARG, "device buffers must be 16-byte aligned");
     DevParams q;
-    fill_params(p, in, out, q, -1, nullptr, -1, &p->pspec);
+    fill_params(p, in, out, q, -1, sub, -1, &p->pspec);
     const long long tiles = (long long)q.nxs * q.nys * q.nzs;
     if (tiles <= 0) return DRS_OK;
     const long long ctas = p->pspec.ctas(q.nxs, q.nys, q.nzs);
@@ -1190,12 +1192,23 @@ int drs_plan_sync_check(drs_plan* p, void* stream) {
     return DRS_OK;
 }
 
-// Slow-axis units per block of the streamed host run, 0 = run the plain copy-sweep-copy sequence.
-// A block must be at least two halos thick (core/host_schedule.hpp); blocks of >= 32 MiB keep the
-// copy engines efficient, at most ~16 of them keep the number of small launches low.
-static long long host_block_units(const drs_plan* p, int sweeps, bool allow_slab = false) {
+// Levels of each launch of a streamed host run of n sweeps: drs_run's launch sequence (pair_split: 2 for a pair
+// launch, then the single sweeps' 1s) on plans where drs_run pairs, n single sweeps otherwise.
+static std::vector<int> launch_depths(const drs_plan* p, int n) {
+    int pairs = 0, singles = n;
+    if (uses_pairs(p)) drs::pair_split(n, pairs, singles);
+    std::vector<int> depth(pairs, 2);
+    depth.insert(depth.end(), singles, 1);
+    return depth;
+}
+
+// Slow-axis units per block of the streamed host run of launches `depth`, 0 = run the plain copy-sweep-copy
+// sequence.  A block must be at least drs::min_block thick (core/host_schedule.hpp: 2 halos, 4 with pair
+// launches); blocks of >= 32 MiB keep the copy engines efficient, at most ~16 of them keep the number of small
+// launches low.
+static long long host_block_units(const drs_plan* p, const std::vector<int>& depth, bool allow_slab = false) {
     const drs::KernelSpec& s = p->spec;
-    if (p->host_block < 0 || (p->slab && !allow_slab) || !s.tma_ok || s.sub_launches > 1 || sweeps <= 0) return 0;
+    if (p->host_block < 0 || (p->slab && !allow_slab) || !s.tma_ok || s.sub_launches > 1 || depth.empty()) return 0;
     const long long slow = p->local_slow(), H = s.halo;
     const double unit = (double)(s.dim == 3 ? p->st.M * p->st.N : p->st.N) * s.esize();
     long long S = p->host_block;
@@ -1204,14 +1217,15 @@ static long long host_block_units(const drs_plan* p, int sweeps, bool allow_slab
         S = (long long)std::ceil(target / unit);
         S = (S + s.chunk - 1) / s.chunk * s.chunk;     // whole tiles per launch
     }
-    S = std::max<long long>(S, std::max<long long>(2 * H, 1));
+    S = std::max(S, drs::min_block(depth, H));
     return S < slow ? S : 0;
 }
 
 // The emitted main()'s data path (H2D, the ping-pong schedule, D2H) in the time-skewed block order of
-// core/host_schedule.hpp: uploads on one stream, sweeps on a second, downloads on a third, chained
-// by events -- the wall time tends to max(H2D, sweeps, D2H) instead of their sum.  Odd sweeps run
-// dA -> dB, even ones dB -> dA; local plane i is host[i - h0].  clear_b: clear dB before the first sweep.
+// core/host_schedule.hpp: uploads on one stream, launches on a second, downloads on a third, chained
+// by events -- the wall time tends to max(H2D, sweeps, D2H) instead of their sum.  Odd launches run
+// dA -> dB, even ones dB -> dA; a pair launch takes level 0's ring from dA and level 1's from dB, whose ring
+// is the cleared one.  Local plane i is host[i - h0].  clear_b: clear dB before the first launch.
 // Face steps (slab runs) use the flag values flag_base + 1 ...: launches that touch a face are bracketed by
 // the flag kernels, and the upload that brings a face's level-0 planes is followed by a peer copy of them into
 // the neighbour's ghosts.  `what` prefixes the message of a CUDA error found at the end.
@@ -1263,15 +1277,18 @@ static int run_blocks(drs_plan* p, const std::vector<drs::HostStep>& steps, char
         if (rc != DRS_OK) break;
         if (st.kind == drs::HostStep::UPLOAD) {
             cudaStreamWaitEvent(p->hs_run, up[st.block], 0);
+        } else if (st.kind == drs::HostStep::PAIR) {
+            const SlowRange r = {st.lo, st.hi};
+            rc = (st.launch & 1) ? launch_pair(p, dA, dB, dA, dB, p->hs_run, &r) : launch_pair(p, dB, dA, dA, dB, p->hs_run, &r);
         } else if (st.kind == drs::HostStep::SWEEP) {
             if (st.faces & (drs::WAIT_LOWER | drs::WAIT_UPPER))
                 rc = launch_wait(p, p->hs_run, p->my_flags, (st.faces & drs::WAIT_LOWER) != 0, (st.faces & drs::WAIT_UPPER) != 0,
-                                 flag_base + st.sweep);
+                                 flag_base + st.launch);
             const SlowRange r = {st.lo, st.hi};
-            if (rc == DRS_OK) rc = (st.sweep & 1) ? launch_one(p, dA, dB, p->hs_run, -1, &r) : launch_one(p, dB, dA, p->hs_run, -1, &r);
+            if (rc == DRS_OK) rc = (st.launch & 1) ? launch_one(p, dA, dB, p->hs_run, -1, &r) : launch_one(p, dB, dA, p->hs_run, -1, &r);
             if (rc == DRS_OK && (st.faces & (drs::SIGNAL_LOWER | drs::SIGNAL_UPPER)))
                 rc = launch_signal(p, p->hs_run, (st.faces & drs::SIGNAL_LOWER) ? p->lower_flag : nullptr,
-                                   (st.faces & drs::SIGNAL_UPPER) ? p->upper_flag : nullptr, flag_base + st.sweep + 1);
+                                   (st.faces & drs::SIGNAL_UPPER) ? p->upper_flag : nullptr, flag_base + st.launch + 1);
         } else {
             cudaEventRecord(done[st.block], p->hs_run);
             cudaStreamWaitEvent(p->hs_dn, done[st.block], 0);
@@ -1296,14 +1313,16 @@ static int run_blocks(drs_plan* p, const std::vector<drs::HostStep>& steps, char
 
 // Step list of a streamed drs_run_host; empty when the plain copy-sweep-copy sequence applies.
 static std::vector<drs::HostStep> host_steps(const drs_plan* p, int n) {
-    const long long S = host_block_units(p, n);
+    const std::vector<int> depth = launch_depths(p, n);
+    const long long S = host_block_units(p, depth);
     if (S <= 0) return {};
-    return drs::plan_block_schedule(drs::whole_grid(p->local_slow(), p->spec.halo), p->spec.halo, S, n);
+    return drs::plan_block_schedule(drs::whole_grid(p->local_slow(), p->spec.halo), p->spec.halo, S, depth);
 }
 
 // Step list of this rank for a slab host run; empty when the plain sequence applies.
 static std::vector<drs::HostStep> slab_steps(const drs_plan* p, int n, bool up_skew) {
-    const long long S = host_block_units(p, n, true);
+    const std::vector<int> depth(n, 1);         // single sweeps: launch_depths is all 1s on slab plans
+    const long long S = host_block_units(p, depth, true);
     if (S <= 0) return {};
     const long long H = p->spec.halo, org = p->lo - H;
     drs::SlabSide g;
@@ -1314,17 +1333,17 @@ static std::vector<drs::HostStep> slab_steps(const drs_plan* p, int n, bool up_s
     g.has_lower = p->lo > 0; g.has_upper = p->hi < p->g_slow;
     g.up_skew = up_skew;
     if (g.out_hi - g.out_lo < 2 * H || g.own_hi - g.own_lo <= S) return {};
-    return drs::plan_block_schedule(g, H, S, n);
+    return drs::plan_block_schedule(g, H, S, depth);
 }
 
-// A step list as records of `width` fields: kind, block, sweep, lo, hi (, faces).  Returns the number of steps.
+// A step list as records of `width` fields: kind, block, launch, lo, hi (, faces).  Returns the number of steps.
 static int step_records(const std::vector<drs::HostStep>& steps, long long* records, int width, int capacity) {
     if (records) {
         if (capacity < (int)steps.size()) return fail(DRS_E_ARG, "buffer too small");
         for (size_t i = 0; i < steps.size(); ++i) {
             const drs::HostStep& st = steps[i];
             long long* r = records + width * i;
-            r[0] = st.kind; r[1] = st.block; r[2] = st.sweep; r[3] = st.lo; r[4] = st.hi;
+            r[0] = st.kind; r[1] = st.block; r[2] = st.launch; r[3] = st.lo; r[4] = st.hi;
             if (width > 5) r[5] = st.faces;
         }
     }

@@ -164,11 +164,11 @@ int drs_run(drs_plan *p, void *d_a, void *d_b, int iterations, void *stream, int
  * single sweeps wherever the plan has a pair kernel: on 2D plans the 2D pair unit (kernels/pair2d/drs_pair2d.cuh),
  * generated and compiled here (NVRTC, no GPU needed); on 3D plans the pair unit without its 1 GiB size rule (a no-op
  * where the plan already pairs).  enable = 0 restores the default rule.  drs_plan_pair_source, drs_plan_pair_cache_key
- * and drs_plan_pair_split follow the setting; drs_sweep, drs_gold_run, the streamed drs_run_host, the slab calls and
- * drs_emit_program do not.  DRS_E_ARG, with the reason, for plans without a pair kernel: step > 1 or per-sub-step
- * launches, `--fuse reuse`, the naive kernel, an unaligned row pitch, an operator whose depth-2 strip or tile keeps no
- * useful columns or whose x extent one lane's shuffle does not reach (2D); and for slab plans, which have
- * drs_plan_set_slab_pairs.  Drops the plan's cached drs_run graphs. */
+ * and drs_plan_pair_split follow the setting, and so does the streamed drs_run_host (which pairs wherever drs_run
+ * does); drs_sweep, drs_gold_run, the slab calls and drs_emit_program do not.  DRS_E_ARG, with the reason, for
+ * plans without a pair kernel: step > 1 or per-sub-step launches, `--fuse reuse`, the naive kernel, an unaligned
+ * row pitch, an operator whose depth-2 strip or tile keeps no useful columns or whose x extent one lane's shuffle
+ * does not reach (2D); and for slab plans, which have drs_plan_set_slab_pairs.  Drops the plan's cached drs_run graphs. */
 int drs_plan_set_pairs(drs_plan *p, int enable);
 /* how drs_run splits the sweeps of `iterations` timesteps: *pairs pair launches, then *singles single sweeps
  * (*pairs = 0 on plans without pair launches, slab plans included); returns the number of sweeps.  Needs no GPU. */
@@ -187,14 +187,19 @@ int drs_gold_run(drs_plan *p, void *d_a, void *d_b, int iterations, void *stream
  * is cut into blocks of planes (rows in 2D), each block runs the whole schedule with its output
  * range sliding down one Halo per sweep while later blocks upload and earlier ones download
  * (pinned host memory needed for the overlap; results are bit-identical to the plain sequence).
+ * On plans where drs_run makes pair launches the blocks run drs_run's launch sequence -- the pair launches of
+ * drs_plan_pair_split, then the single sweeps -- with the range sliding two Halos per pair launch (and two at the
+ * first single sweep after them), on blocks at least 4*Halo thick.
  * *device_ms = device time from the first copy to the last, CUDA events. */
 int drs_run_host(drs_plan *p, void *h_a, void *h_b, int iterations, float *device_ms);
 /* block thickness of the streamed drs_run_host in slow-axis units: 0 = chosen by the engine
- * (>= 32 MiB, about 16 blocks), < 0 = plain copy-sweep-copy, > 0 = as given (raised to 2*Halo) */
+ * (>= 32 MiB, about 16 blocks), < 0 = plain copy-sweep-copy, > 0 = as given (raised to 2*Halo, or to 4*Halo when
+ * the run makes pair launches) */
 int drs_plan_set_host_block(drs_plan *p, long long units);
 /* the step list the streamed drs_run_host would execute for `iterations` (needs no GPU): records of five
- * values {kind (0 upload, 1 sweep, 2 download), block, sweep (1-based; odd: A -> B), lo, hi} with [lo, hi)
- * the slow-axis range copied / produced; per block: its upload, its sweeps, its download.  Returns the
+ * values {kind (0 upload, 1 sweep, 2 download, 3 pair launch), block, launch (1-based index in drs_run's launch
+ * sequence; odd: A -> B; on plans without pair launches the sweep number), lo, hi} with [lo, hi) the slow-axis
+ * range copied / stored by the launch; per block: its upload, its launches, its download.  Returns the
  * number of records (pass NULL to query), 0 when the plain sequence would run. */
 int drs_plan_host_schedule(const drs_plan *p, int iterations, long long *records5, int capacity);
 /* The step list one rank of a slab-decomposed host-buffer run executes so that its copies overlap its sweeps
